@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the descriptor-matching hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[4], the configuration the metric "... at 1/2/4/8 B200" is quoted on): synthetic
 all-pairs matching of 512 images x 4096 256-bit descriptors = 130 816 image pairs = 2.195e12 distance evaluations,
@@ -55,7 +55,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[1]/[2]/[3], knn and float-L2 extras")
     ap.add_argument("--no-full-unit", action="store_true", help="reference arm: skip the one full-size 4096x4096 pair")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def workload_name(args, world):
@@ -255,8 +262,8 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     stream.synchronize()
 
     def step_dev():
-        m.match_pairs_batch_dev(d_all.data_ptr(), offs, mine, BITS, STRIDE, d_out[0].data_ptr(), d_out[1].data_ptr(),
-                                d_out[2].data_ptr(), rows)
+        return m.match_pairs_batch_dev(d_all.data_ptr(), offs, mine, BITS, STRIDE, d_out[0].data_ptr(),
+                                       d_out[1].data_ptr(), d_out[2].data_ptr(), rows)
 
     # ---- value: device-resident, CUDA events on the launching stream.  The job's working set (64 MB of descriptors,
     # >1 GB of matcher state per chunk of 4096 pairs, 6.4 GB / N of triples) is far larger than the 126 MB L2.
@@ -272,10 +279,12 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     with torch.cuda.stream(stream):
         for k in range(args.steps):
             ev[k][0].record(stream)
-            step_dev()
+            counts = step_dev()
             ev[k][1].record(stream)
     stream.synchronize()
     barrier()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d_out, counts, len(pairs), lo, hi, per, rank, world, dev)
     step_ms = [a.elapsed_time(b) for a, b in ev]
     T_ms = max_over_ranks(float(np.sum(step_ms)))
     value = total_evals * args.steps / (T_ms * 1e-3)
@@ -412,6 +421,46 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     m.close()
     if rank == 0:
         print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 64_000_000        # --dump-outputs writes at most this much (64 MB)
+
+
+def dump_outputs(out_dir, d_out, counts, n_pairs, lo, hi, per, rank, world, dev):
+    """--dump-outputs: what the timed call returned to its caller in the last timed step, as float64 arrays (exact for
+    every int32), so that two builds can be compared output for output on the same seeded job.
+
+        counts.npy       [n_pairs]   triples written for each pair of the job (the counts the call returns)
+        pair_index.npy   [S]         a fixed sample of the job's pairs (seed 0, ascending): as many as fit DUMP_BYTES
+        query_index.npy  [S, per]    the sampled pairs' triples (query index, train index, Hamming distance) in the
+        train_index.npy  [S, per]    order the call wrote them
+        distance.npy     [S, per]
+
+    Every rank contributes the pairs of its block [lo, hi) of the pair list; rank 0 writes the files."""
+    import torch
+    import torch.distributed as dist
+
+    room = DUMP_BYTES - 5 * 256 - 8 * n_pairs                   # five .npy headers and counts.npy
+    n_sample = min(n_pairs, max(0, room // (8 + 3 * 8 * per)))
+    sample = np.sort(np.random.default_rng(0).choice(n_pairs, n_sample, replace=False))
+    owned = np.flatnonzero((sample >= lo) & (sample < hi))
+    tri = torch.zeros((3, n_sample, per), dtype=torch.int32, device=dev)
+    cnt = torch.zeros(n_pairs, dtype=torch.int32, device=dev)
+    if len(owned):
+        # every image has `per` descriptors, so pair p of the block owns rows (p - lo) * per ... + per
+        rows = torch.from_numpy((sample[owned] - lo) * per).to(dev)[:, None] + torch.arange(per, device=dev)[None, :]
+        tri[:, torch.from_numpy(owned).to(dev)] = d_out[:, rows]
+    cnt[lo:hi] = torch.from_numpy(np.ascontiguousarray(counts, dtype=np.int32)).to(dev)
+    if world > 1:
+        dist.all_reduce(tri)
+        dist.all_reduce(cnt)
+    if rank != 0:
+        return
+    tri, cnt = tri.cpu().numpy(), cnt.cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"counts": cnt, "pair_index": sample, "query_index": tri[0], "train_index": tri[1], "distance": tri[2]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
 
 
 # --------------------------------------------------------------------------

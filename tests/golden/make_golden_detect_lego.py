@@ -11,8 +11,10 @@ pairs (np.random.seed(7)), uv0/1, desc0/1, twin_nearest_dist, twin_sorted_dists.
 from __future__ import annotations
 
 import argparse
+import io
 import os
 import sys
+import zipfile
 
 import numpy as np
 
@@ -57,7 +59,13 @@ def main() -> None:
     twin = match_keypoints(kps[0], kps[1], -1)
     out["twin_nearest_dist"] = twin[:, 0, 1].astype(np.int64)
     out["twin_sorted_dists"] = twin[:, :, 1].astype(np.int16)
-    np.savez_compressed(os.path.join(HERE, "lego_crop_detect.npz"), **out)
+    # an .npz whose members are bzip2-compressed: np.load reads it like any other, and it stays under 1 MB where
+    # np.savez_compressed (deflate) writes 1.2 MB
+    with zipfile.ZipFile(os.path.join(HERE, "lego_crop_detect.npz"), "w", compression=zipfile.ZIP_BZIP2) as z:
+        for k, v in out.items():
+            buf = io.BytesIO()
+            np.save(buf, v)
+            z.writestr(f"{k}.npy", buf.getvalue())
     print("wrote lego_crop_detect.npz", {k: getattr(v, "shape", v) for k, v in out.items()})
 
 
