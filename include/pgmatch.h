@@ -316,7 +316,8 @@ int pgm_ransac_score(pgm_handle *h, const float *F, const uint8_t *valid, int32_
  * pgm_match_pairs_batch_dev: d_all_desc holds every image's descriptors, image_offsets[n_images + 1] (host) delimits
  * them, pair_list[n_pairs][2] (host) names the pairs; pair p's kept triples (ascending query index) start at the sum
  * of the query sizes of the pairs before it, out_counts[p] (host) says how many.  One CTA per pair with both descriptor
- * sets in shared memory: (n1 + n2) * stride_bytes + 4 * n2 must not exceed 200 KB, else PGM_E_INVALID_ARG. */
+ * sets in shared memory: (n1 + n2) * stride_bytes + 4 * n2 + 16 must not exceed 200 KB (204 800 bytes), else
+ * PGM_E_INVALID_ARG. */
 int pgm_match_ratio_crosscheck_batch_dev(pgm_handle *h, const uint8_t *d_all_desc, const int64_t *image_offsets,
                                          int32_t n_images, const int32_t *pair_list, int32_t n_pairs, int32_t desc_bits,
                                          int32_t stride_bytes, float ratio, int32_t cross_check, int32_t max_dist,
