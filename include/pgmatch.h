@@ -231,10 +231,10 @@ int pgm_match_ratio_crosscheck(pgm_handle *h,
  * relative); indices equal the oracle's except where two candidates' exact fp32 distances
  * differ only by summation order (near-ties).  Ranking operands: one fp16 term per component
  * under a global power-of-two scale (band 2^-9 (3|q|^2 + 2d)); a query whose band could hide a
- * train row that the kernel's per-column-group top-4 lists dropped is recomputed exhaustively on
+ * train row that the kernel's per-column-group top-8 lists dropped is recomputed exhaustively on
  * the device, so the guarantee does not depend on the data (pgm_l2_last_fallback_rows counts
- * them).  PGM_L2_MODE=bf16x3 selects the round-1 three-term bf16 split (three GEMM passes),
- * which n1 <= 128 always uses.  d_debug_dist (optional, device float[n1][n2]) receives the
+ * them).  n1 <= 128 ranks with a three-term bf16 split (three GEMM passes) instead.
+ * d_debug_dist (optional, device float[n1][n2]) receives the
  * approximate GEMM distances. */
 int pgm_knn2_l2(pgm_handle *h, const float *q, int32_t n1, const float *t, int32_t n2, int32_t dim,
                 int32_t *best_j, float *best_d, int32_t *second_j, float *second_d);

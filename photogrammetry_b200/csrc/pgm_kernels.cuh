@@ -115,7 +115,6 @@ struct PairDesc {
     int32_t cand_cap, ledge_cap;
 };
 constexpr int PAIR_FLAG_NO_FINISHER = 1;   // never hand this pair to the single-CTA finisher
-constexpr int PAIR_FLAG_NO_EMIT = 2;       // no candidate edges for this pair
 constexpr int PAIR_FLAG_SHARD = 4;         // one rank's slice of a train-sharded pair (keys carry global column ids)
 
 struct PairStat {            // per pair, written by the init kernel
@@ -176,7 +175,7 @@ struct Chunk {
     uint32_t *fin_rb, *fin_cb;    // latency mode: [n_pairs][FIN_PARTS][FIN_MAX_DIM] first-round row / column minima (partial)
     int32_t *fin_ids;             // latency mode: [n_pairs][2][FIN_MAX_DIM] rank-sorted row / column ids
     long long large_min_evals;    // a round with at least this many live cells uses the large (RQ = 4) tiles
-    // candidate edges (nullptr: the classic one-accept-per-pass rounds only)
+    // candidate edges
     unsigned long long *cand;     // raw candidate records of the current pass, per pair region, two words each:
                                   // (d << 40 | i << 20 | j) with d <= T, and (RQ << 20 | first live-list slot of the emitting thread)
     unsigned long long *ledge;    // the raw edges whose row and column both survived the pass's accept
@@ -188,7 +187,7 @@ struct Chunk {
     int32_t words;                // descriptor words (runtime copy of the kernels' template parameter)
     int32_t *order_cnt;           // latency mode: [n_pairs][ORDER_MAX_SLICES][ORDER_BIN_PITCH] per-slice distance histograms
     int32_t shard_n2_total;       // train-sharded pair: columns of the whole pair
-    float cand_target;            // expected candidate edges per row of the smaller side (CAND_TARGET; PGM_CAND_TARGET overrides)
+    float cand_target;            // expected candidate edges per row of the smaller side (CAND_TARGET, _BATCH or _SHARD)
     float cand_row_max;           // upper bound of the per-row target of a pass (later passes: few live rows share the list budget)
     LatState *lat;                // latency mode: the self-cleaning plan + statistics block (plan == &lat->plan), else nullptr
     int32_t sp_slots_max;         // edge slots per thread a sparse phase may use (SP_EPT; smaller values force its truncation path in tests)
@@ -245,7 +244,6 @@ __device__ __forceinline__ void plan_pair_emit(const Chunk &c, int p, uint8_t st
     // a tile stages at most SCAND records between two flushes (one stage of columns): keep the expected number per stage
     // below half of that, whatever the list budget would allow
     const float p_max = 0.4f * (float)SCAND / (float)(ROUND_THREADS * rq * (rq == RQ_LARGE ? STAGE_LARGE : STAGE_SMALL));
-    if (!c.cand) return;
     uint32_t thr = 0u;
     const PairDesc &pd = c.pairs[p];
     if (!(pd.flags & PAIR_FLAG_SHARD) && __ldcg(c.cand_cnt + p) > pd.cand_cap) c.pstat[p].cscale *= 0.25f;   // the last pass overflowed
@@ -261,7 +259,7 @@ __device__ __forceinline__ void plan_pair_emit(const Chunk &c, int p, uint8_t st
             const float T = floorf(ps.mu - z * ps.sd - 0.5f);
             if (T >= 0.0f) thr = ((uint32_t)fminf(T, 1022.0f) + 1u) << KEY_IDX_BITS;
         }
-    } else if (st == PAIR_BIG && pd.cand_cap > 0 && !(pd.flags & PAIR_FLAG_NO_EMIT)) {
+    } else if (st == PAIR_BIG && pd.cand_cap > 0) {
         const PairStat ps = c.pstat[p];
         // about cand_target x max(n1, n2) raw edges in EVERY pass: later passes have fewer live rows, so each row may
         // list more candidates for the same list size (8192 x 8192: 6 per row in pass 0, ~36 per row of the 1236 left
@@ -284,7 +282,6 @@ __device__ __forceinline__ void plan_pair_emit(const Chunk &c, int p, uint8_t st
 // result, never a match.
 __device__ __forceinline__ void sample_pair_stats(const Chunk &c, int p, const PairDesc &pd) {
     __shared__ unsigned s_sum, s_sum2;
-    if (!c.cand) return;                                    // (uniform)
     const int tid = threadIdx.x;
     if (tid == 0) { s_sum = 0u; s_sum2 = 0u; }
     __syncthreads();
@@ -587,7 +584,7 @@ __global__ void __launch_bounds__(ACCEPT_THREADS) init_kernel(Chunk c, PairPack 
         int32_t *c1 = cnt_ptr(c, 1, p), *c2 = cnt_ptr(c, 2, p);
         c1[0] = c1[1] = 0; c2[0] = c2[1] = 0;
         c.status[p] = PAIR_BIG;                      // classified by plan(0)
-        if (c.cand) { c.cand_cnt[p] = 0; c.ledge_cnt[p] = 0; c.thr[p] = 0u; }
+        c.cand_cnt[p] = 0; c.ledge_cnt[p] = 0; c.thr[p] = 0u;
     }
     if (blockIdx.x == 0) {                                 // (block-uniform)
         PairDesc sp = pd;
@@ -732,9 +729,9 @@ __device__ __forceinline__ void round_tiles(const Chunk &c, int r, int total, in
         const int32_t *live_cols = c.live_cols[cur] + pd.col_base;
         // candidate edges: every (i, j) of this tile with distance <= T goes to the pair's list (staged in shared
         // memory, one global append per tile).  thr = (T + 1) << 20 as a key bound; 0 = this pass emits nothing.
-        uint32_t thr = c.cand ? __ldcg(c.thr + p) : 0u;
+        uint32_t thr = __ldcg(c.thr + p);
         if (thr && __ldcg(c.cand_cnt + p) > pd.cand_cap) thr = 0u;     // the list already overflowed: stop feeding it
-        if (c.cand && tid == 0) s_cctl[0] = 0;                         // (ordered by the stage loop's first barrier)
+        if (tid == 0) s_cctl[0] = 0;                                   // (ordered by the stage loop's first barrier)
         const uint32_t aux = ((uint32_t)RQ << KEY_IDX_BITS) | (uint32_t)(rt * tile_rows + tid);
         // Append the staged records to the pair's list once at least `at_least` (+1) are waiting.  Called by every thread
         // of the group right after a group barrier (the count is uniform); leaves the staging buffer empty.
@@ -879,13 +876,13 @@ __device__ __forceinline__ void round_tiles(const Chunk &c, int r, int total, in
                 if (jk != KEY_INVALID && v < KEY_INVALID)      // jk carries the global id; the state arrays are local
                     atomicMin(c.colbest[cur] + pd.col_base + (jk - (uint32_t)pd.col_id_offset), v);
             }
-            if (c.cand) flush_cands(SCAND / 2);              // wide tiles (batches of pairs) see more records than one staging buffer holds
+            flush_cands(SCAND / 2);                          // wide tiles (batches of pairs) see more records than one staging buffer holds
         }
 #pragma unroll
         for (int k = 0; k < RQ; k++)
             if (ikey[k] != KEY_INVALID && rowkey[k] < KEY_INVALID)
                 atomicMin(c.rowbest[cur] + pd.row_base + ikey[k], rowkey[k]);
-        if (c.cand) { bar.sync(); flush_cands(0); }     // the tile's remaining staged candidate records
+        bar.sync(); flush_cands(0);                     // the tile's remaining staged candidate records
         tstamp(c, vb, tid, 5);
     }
 }
@@ -961,8 +958,8 @@ __device__ __forceinline__ void accept_blocks(const Chunk &c, int r, int vb, int
             if (survive) {
                 const int pos = base + __popc(m & ((1u << lane) - 1u));
                 PGM_ASSERT(pos >= 0 && pos < (is_row ? nlr : nlc));
-                if (is_row) { c.live_rows[nxt][pd.row_base + pos] = id; if (c.cand) c.row_pos[pd.row_base + id] = pos; }
-                else { c.live_cols[nxt][pd.col_base + pos] = id; if (c.cand) c.col_pos[pd.col_base + id] = pos; }
+                if (is_row) { c.live_rows[nxt][pd.row_base + pos] = id; c.row_pos[pd.row_base + id] = pos; }
+                else { c.live_cols[nxt][pd.col_base + pos] = id; c.col_pos[pd.col_base + id] = pos; }
             }
         }
     }
@@ -1076,7 +1073,7 @@ __device__ __forceinline__ void filter_edges(const Chunk &c, int r, int p, int s
 // ---------------------------------------------------------------------------
 template <int NT>
 __device__ __forceinline__ void sparse_body(const Chunk &c, int r, int p, unsigned char *smem) {
-    if (!c.cand || __ldcg(c.status + p) != PAIR_BIG) return;
+    if (__ldcg(c.status + p) != PAIR_BIG) return;
     const int tid = threadIdx.x, lane = tid & 31;
     const PairDesc &pdr = c.pairs[p];
     const int nL = __ldcg(c.ledge_cnt + p);
@@ -1326,16 +1323,12 @@ __device__ __forceinline__ void sparse_body(const Chunk &c, int r, int p, unsign
 // (5 CTAs per SM: the kernel is a chain of dependent L2 / HBM accesses per record, more resident warps is what it needs)
 __global__ void __launch_bounds__(ACCEPT_THREADS, 5) accept_kernel(Chunk c, int r) {
     accept_blocks(c, r, blockIdx.x, gridDim.x, threadIdx.x);
-    if (c.cand) {
-        // a pair's raw list is dealt out in FILTER_SEGS interleaved segments: with one CTA per pair a grid of ~1200
-        // CTAs walked 2016 lists as two unequal waves of ~100 dependent iterations each
-        constexpr int FILTER_SEGS = 8;
-        for (int item = blockIdx.x; item < c.n_pairs * FILTER_SEGS; item += gridDim.x) {
-            const int p = item / FILTER_SEGS, seg = item - p * FILTER_SEGS;
-            filter_edges(c, r, p, seg * ACCEPT_THREADS + (int)(threadIdx.x & ~31u), ACCEPT_THREADS * FILTER_SEGS);
-        }
-    } else {
-        plan_in_last_block(c, r + 1, gridDim.x);
+    // a pair's raw list is dealt out in FILTER_SEGS interleaved segments: with one CTA per pair a grid of ~1200
+    // CTAs walked 2016 lists as two unequal waves of ~100 dependent iterations each
+    constexpr int FILTER_SEGS = 8;
+    for (int item = blockIdx.x; item < c.n_pairs * FILTER_SEGS; item += gridDim.x) {
+        const int p = item / FILTER_SEGS, seg = item - p * FILTER_SEGS;
+        filter_edges(c, r, p, seg * ACCEPT_THREADS + (int)(threadIdx.x & ~31u), ACCEPT_THREADS * FILTER_SEGS);
     }
 }
 
@@ -1813,25 +1806,19 @@ __global__ void __launch_bounds__(TAIL_THREADS, 1) tail_kernel(Chunk c, int r_st
     // pair p in CTA p, the last of them plans pass r + 1 | barrier
     auto after_pass = [&](int r) {
         accept_blocks(c, r, (tid >> 8) * gridDim.x + blockIdx.x, gridDim.x * 2, tid & (ACCEPT_THREADS - 1));
-        if (c.cand) {
-            const int gw32 = (int)((blockIdx.x * TAIL_THREADS + tid) & ~31u);
-            for (int p = 0; p < c.n_pairs; p++) filter_edges(c, r, p, gw32, (int)gridDim.x * TAIL_THREADS);
-        } else {
-            plan_in_last_block(c, r + 1, gridDim.x);
+        const int gw32 = (int)((blockIdx.x * TAIL_THREADS + tid) & ~31u);
+        for (int p = 0; p < c.n_pairs; p++) filter_edges(c, r, p, gw32, (int)gridDim.x * TAIL_THREADS);
+        stamp(c, slot);
+        grid_barrier(bar_counter, gridDim.x, epoch);
+        stamp(c, slot);
+        if ((int)blockIdx.x < c.n_pairs) {
+            sparse_body<TAIL_THREADS>(c, r, blockIdx.x, dyn_smem);
+            if (c.n_pairs == 1) { __syncthreads(); if (tid < 32) plan_warp(c, r + 1); }   // (no ticket to take)
+            else plan_in_last_block(c, r + 1, (unsigned)c.n_pairs);
         }
         stamp(c, slot);
         grid_barrier(bar_counter, gridDim.x, epoch);
         stamp(c, slot);
-        if (c.cand) {
-            if ((int)blockIdx.x < c.n_pairs) {
-                sparse_body<TAIL_THREADS>(c, r, blockIdx.x, dyn_smem);
-                if (c.n_pairs == 1) { __syncthreads(); if (tid < 32) plan_warp(c, r + 1); }   // (no ticket to take)
-                else plan_in_last_block(c, r + 1, (unsigned)c.n_pairs);
-            }
-            stamp(c, slot);
-            grid_barrier(bar_counter, gridDim.x, epoch);
-            stamp(c, slot);
-        }
     };
     // (one copy of the pass body: the kernel's code size is what its short phases pay for in instruction-cache misses)
     bool have_pass = (flags & TAIL_FLAG_ACCEPT_FIRST) != 0;         // round r_start - 1 ran as a standalone launch

@@ -6,18 +6,17 @@
 //
 //     ||q - t||^2 = ||q||^2 + ||t||^2 - 2 q.t          (N1 x N2 x D GEMM)
 //
-// The GEMM only RANKS.  Default (CTA-pair kernel): every component becomes ONE fp16 value under a global
-// power-of-two scale (absmax_kernel + split16_kernel), one GEMM pass of K = Dp.  PGM_L2_MODE=bf16x3 (and the
-// single-CTA kernel, n1 <= 128): bf16 hi + lo split, q.t ~ hi.hi + lo.hi + hi.lo as three passes into the same
-// fp32 TMEM accumulator.  Operand rows are stored once as [x16 | norm] (resp. [x_hi | x_lo | norm]).  The norm
-// chunk folds ||q||^2 and ||t||^2 into the SAME accumulator: the query row carries -||q||^2/2 as three 16-bit
-// terms against constants on the train side and vice versa, so one extra K = 16 MMA per tile leaves
-// q.t - (||q||^2 + ||t||^2)/2 = -d/2 in TMEM and the epilogue needs no arithmetic at all: a distance's rank is
-// its bit pattern.  The epilogue keeps, per query and column group, the columns within the ranking's error band
-// of the second best one (RowTop below); l2_refine_kernel recomputes those few distances exactly in fp32 (sum of
-// squared differences), picks best/second and certifies that the lists cannot have hidden a better column; rows
-// it cannot certify are recomputed exhaustively by l2_exact_rows_kernel.  Reported distances are exact to fp32
-// rounding; indices can differ from the oracle only where exact fp32 distances tie up to summation order.
+// The GEMM only RANKS.  CTA-pair kernel (n1 > 128): every component becomes ONE fp16 value under a global power-of-two
+// scale (absmax_kernel + split16_kernel), one GEMM pass of K = Dp.  Single-CTA kernel (n1 <= 128): bf16 hi + lo split,
+// q.t ~ hi.hi + lo.hi + hi.lo as three passes into the same fp32 TMEM accumulator.  Operand rows are stored once as
+// [x16 | norm] (resp. [x_hi | x_lo | norm]).  The norm chunk folds ||q||^2 and ||t||^2 into the SAME accumulator: the
+// query row carries -||q||^2/2 as three 16-bit terms against constants on the train side and vice versa, so one extra
+// K = 16 MMA per tile leaves q.t - (||q||^2 + ||t||^2)/2 = -d/2 in TMEM and the epilogue needs no arithmetic at all: a
+// distance's rank is its bit pattern.  The epilogue keeps, per query and column group, the columns within the
+// ranking's error band of the second best one (RowTop below); l2_refine_kernel recomputes those few distances exactly
+// in fp32 (sum of squared differences), picks best/second and certifies that the lists cannot have hidden a better
+// column; rows it cannot certify are recomputed exhaustively by l2_exact_rows_kernel.  Reported distances are exact to
+// fp32 rounding; indices can differ from the oracle only where exact fp32 distances tie up to summation order.
 //
 // Kernel anatomy (sm_100a, hand-written PTX; layouts follow the canonical K-major
 // SWIZZLE_128B UMMA atoms):
@@ -45,15 +44,9 @@ constexpr int CHUNK_K = 64;        // bf16 elements per 128-byte swizzle row
 constexpr int UMMA_K = 16;         // K of one tcgen05.mma for 16-bit inputs
 constexpr int MAX_CHUNKS = 5;      // resident A' chunks: [hi | lo | norm], Dp <= 128
 constexpr int STAGES = 8;          // B' ring of chunk slots: two whole tiles deep at Dp = 128
-#ifndef PGM_L2_EPI_GROUPS
-#define PGM_L2_EPI_GROUPS 2
-#endif
-constexpr int EPI_GROUPS = PGM_L2_EPI_GROUPS;   // each epilogue warpgroup reduces an equal share of the accumulator's columns
+constexpr int EPI_GROUPS = 2;      // each epilogue warpgroup reduces an equal share of the accumulator's columns
 constexpr int THREADS = 128 + 128 * EPI_GROUPS; // warps 0-3: TMA / MMA / TMEM alloc / spare; then the epilogue warpgroups
-#ifndef PGM_L2_TOPK
-#define PGM_L2_TOPK 8
-#endif
-constexpr int TOPK = PGM_L2_TOPK;   // candidates kept per (query, column split, epilogue warpgroup)
+constexpr int TOPK = 8;            // candidates kept per (query, column split, epilogue warpgroup)
 constexpr int CAND = TOPK * EPI_GROUPS;
 constexpr uint32_t CHUNK_BYTES = TILE_N * CHUNK_K * 2;   // 16 KB (A' and B' chunks have the same shape)
 constexpr uint32_t TMEM_COLS = 256;                      // two fp32 accumulators of 128 columns
@@ -312,16 +305,13 @@ __global__ void __launch_bounds__(256) split16_kernel(const float *__restrict__ 
     *reinterpret_cast<__half2 *>(o + dp + 2 * lane) = ext;
 }
 
-// ---- the GEMM + top-4 kernel ----------------------------------------------------------------
+// ---- the GEMM + top-8 kernel ----------------------------------------------------------------
 struct L2Params {
     int n1, n2, dpc;               // dpc = Dp / 64: chunks per operand part (hi or lo)
     int tiles_per_split;           // single-CTA kernel: column tiles handled by one blockIdx.y
-    int col_tiles, items, flat;    // pair kernel: column tiles per row pair, row pairs x column tiles, work distribution
+    int col_tiles, items;          // pair kernel: column tiles per row pair, row pairs x column tiles
     uint32_t key_mask;             // 0x7FFFFFE0, passed as data so that (acc & mask) | column is ONE LOP3
-    int dbg_flags;                 // developer experiments (PGM_L2_DBG): 1 = the epilogue releases accumulators without reading them
-    int nparts;                    // operand parts per row: 2 = bf16 hi + lo (three GEMM passes), 1 = one fp16 term (one pass)
-    uint32_t idesc;                // tcgen05 instruction descriptor of the pair kernel (bf16 or fp16 inputs)
-    const unsigned *absmax_bits;   // fp16 mode: bit pattern of max |x| over both operand sets (the scale derives from it), else null
+    const unsigned *absmax_bits;   // pair kernel (fp16): bit pattern of max |x| over both operand sets (the scale derives from it)
     float band_rel, band_abs_sqrt, band_abs_const;   // error band of one accumulator comparison (see RowTop)
     const float *qnorm;            // [n1] |q|^2 in the accumulator's units (written by the split kernel)
     float *cand_drop;              // [splits][n1][EPI_GROUPS] approximate distance of a FULL list's last entry (3.4e38: list not full)
@@ -599,18 +589,15 @@ l2_topk_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 //   leader      warp 1: issues the MMAs; tcgen05.commit.multicast arrives on both CTAs' barriers
 //   both CTAs   warps 4-11: epilogue over the CTA's own 128 rows x 256 columns (TMEM is per SM);
 //               accumulator release arrives on the leader's tempty barrier (remote arrive for rank 1)
-#ifndef PGM_L2_PAIR_N
-#define PGM_L2_PAIR_N 256
-#endif
-constexpr int TILE_N2 = PGM_L2_PAIR_N;        // train rows per accumulator in pair mode (half per CTA)
+constexpr int TILE_N2 = 256;                  // train rows per accumulator in pair mode (half per CTA)
 constexpr uint32_t TMEM_COLS2 = 512;
 constexpr int NACC2 = 512 / TILE_N2;          // accumulators in flight: all 512 TMEM columns
 constexpr int B_ROWS2 = TILE_N2 / 2;          // train rows each CTA stages per tile
 constexpr uint32_t B_CHUNK_BYTES2 = B_ROWS2 * CHUNK_K * 2;
 constexpr int STAGES2 = (int)((size_t)STAGES * CHUNK_BYTES / B_CHUNK_BYTES2);   // same 128 KB ring
-static_assert(TILE_N2 == 256 || TILE_N2 == 128, "pair tile width");
-constexpr uint32_t IDESC_BF16_M256_N2 =
-    (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TILE_N2 >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
+static_assert(TILE_N2 == 256, "pair tile width");
+// f32 accumulator (bit 4), A and B format F16 (0 in bits 7-9 and 10-12), N = TILE_N2, M = 256
+constexpr uint32_t IDESC_F16_M256_N2 = (1u << 4) | ((uint32_t)(TILE_N2 >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
 constexpr uint32_t PEER_BIT_MASK = 0xFEFFFFFFu;   // shared::cluster address of the same offset in the pair's even CTA
 
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -647,10 +634,9 @@ __device__ __forceinline__ void tc_mma_bf16_pair(uint32_t tmem_d, uint64_t adesc
         ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
 
-// Work distribution, two forms (the host picks by a cost model): (a) cluster = (row pair, column split), grid
-// 2*row_pairs x splits, run in waves; (b) "flat": the (row pair, column tile) items are flattened row-major and
-// cut into gridDim.x / 2 contiguous, equally long segments, one per cluster (persistent: as many clusters as are
-// co-resident) -- no wave quantisation, for shapes whose row pairs x splits do not fill the machine.  A segment that crosses into the next row pair reloads A' (after the MMAs of the old rows have
+// Work distribution: the (row pair, column tile) items are flattened row-major and cut into gridDim.x / 2
+// contiguous, equally long segments, one per cluster (persistent: as many clusters as are co-resident) -- no wave
+// quantisation.  A segment that crosses into the next row pair reloads A' (after the MMAs of the old rows have
 // retired) and its epilogue flushes the finished rows' candidates; a row pair's candidates therefore arrive
 // from several segments, each writing its own slot (segment index minus the index of the first segment that
 // touches the row pair).  Unused slots keep the -1 the split kernel wrote.
@@ -679,9 +665,7 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
     const bool leader = rank == 0;
     const int clusters = (int)(gridDim.x >> 1), cid = (int)(blockIdx.x >> 1);
     const int CT = p.col_tiles, items = p.items;
-    // flat: equal segments of the flattened item list; otherwise cluster = (row pair, column split blockIdx.y)
-    const int it0 = p.flat ? l2_segment_start(cid, items, clusters) : cid * CT + (int)blockIdx.y * p.tiles_per_split;
-    const int it1 = p.flat ? l2_segment_start(cid + 1, items, clusters) : min(it0 + p.tiles_per_split, (cid + 1) * CT);
+    const int it0 = l2_segment_start(cid, items, clusters), it1 = l2_segment_start(cid + 1, items, clusters);
     if (threadIdx.x == 0) l2_stamp(p, 0);
 
     if (warp == 1 && lane == 0) {
@@ -706,7 +690,7 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 
     if (warp == 0 && lane == 0) {
         // ===== TMA producer (both CTAs): own A' rows, own half of every B' tile =====
-        const int nch = p.nparts * p.dpc + 1;             // hi chunks, lo chunks (three-pass mode only), norm chunk
+        const int nch = p.dpc + 1;                        // x16 chunks, norm chunk
         int s = 0; uint32_t ph = 0;
         int cur_rp = -1; uint32_t n_a = 0;
         for (int it = it0; it < it1; it++) {
@@ -717,7 +701,7 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                 for (int kc = 0; kc < nch; kc++) tma_load_2d_pair(sa + (size_t)kc * CHUNK_BYTES, &map_a, a_bar, kc * CHUNK_K, m0);
                 cur_rp = rp; n_a++;
             }
-            for (int kc = 0; kc < nch; kc++) {                 // t_hi chunks, t_lo chunks, norm chunk
+            for (int kc = 0; kc < nch; kc++) {                 // t16 chunks, norm chunk
                 mbar_wait(&empty[s], ph ^ 1);                  // the pair's MMAs no longer read this stage (multicast commit)
                 if (leader) mbar_expect_tx(&full[s], 2u * B_CHUNK_BYTES2);
                 tma_load_2d_pair(sb + (size_t)s * B_CHUNK_BYTES2, &map_b, &full[s], kc * CHUNK_K,
@@ -747,32 +731,25 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             tc_fence_after();
             if (t < 36) l2_stamp(p, 4 + t);
             const uint32_t d_tmem = tmem_base + (uint32_t)acc * TILE_N2;
-            // three-pass mode: pass 0 q_hi . t_hi (waits for the hi slots), pass 1 q_lo . t_hi (frees them), pass 2 q_hi . t_lo;
-            // fp16 mode: the one pass waits for and frees its slots
-            const int np = p.nparts, npass = np == 2 ? 3 : 1;
-            const uint32_t idesc = p.idesc;
-            for (int pass = 0; pass < npass; pass++) {
-                for (int c = 0; c < dpc; c++) {
-                    const uint32_t i = g + (uint32_t)(pass == 2 ? dpc + c : c), s = i % STAGES2, ph = (i / STAGES2) & 1u;
-                    if (pass != 1) { mbar_wait(&full[s], ph); tc_fence_after(); }
-                    const int ac = pass == 1 ? dpc + c : c;
-                    const uint64_t adesc = umma_desc_sw128(smem_u32(sa + (size_t)ac * CHUNK_BYTES));
-                    const uint64_t bdesc = umma_desc_sw128(smem_u32(sb + (size_t)s * B_CHUNK_BYTES2));
-#pragma unroll
-                    for (int k = 0; k < CHUNK_K / UMMA_K; k++)
-                        tc_mma_bf16_pair(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc,
-                                         (uint32_t)((pass | c | k) != 0));
-                    if (pass != 0 || np == 1) tc_commit_pair(&empty[s]);
-                }
-            }
-            {   // norm chunk: one K = 16 step adds -(||q||^2 + ||t||^2) / 2
-                const uint32_t i = g + (uint32_t)(np * dpc), s = i % STAGES2, ph = (i / STAGES2) & 1u;
+            for (int c = 0; c < dpc; c++) {
+                const uint32_t i = g + (uint32_t)c, s = i % STAGES2, ph = (i / STAGES2) & 1u;
                 mbar_wait(&full[s], ph); tc_fence_after();
-                tc_mma_bf16_pair(d_tmem, umma_desc_sw128(smem_u32(sa + (size_t)(np * dpc) * CHUNK_BYTES)),
-                                 umma_desc_sw128(smem_u32(sb + (size_t)s * B_CHUNK_BYTES2)), idesc, 1u);
+                const uint64_t adesc = umma_desc_sw128(smem_u32(sa + (size_t)c * CHUNK_BYTES));
+                const uint64_t bdesc = umma_desc_sw128(smem_u32(sb + (size_t)s * B_CHUNK_BYTES2));
+#pragma unroll
+                for (int k = 0; k < CHUNK_K / UMMA_K; k++)
+                    tc_mma_bf16_pair(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), IDESC_F16_M256_N2,
+                                     (uint32_t)((c | k) != 0));
                 tc_commit_pair(&empty[s]);
             }
-            g += (uint32_t)(np * dpc) + 1u;
+            {   // norm chunk: one K = 16 step adds -(||q||^2 + ||t||^2) / 2
+                const uint32_t i = g + (uint32_t)dpc, s = i % STAGES2, ph = (i / STAGES2) & 1u;
+                mbar_wait(&full[s], ph); tc_fence_after();
+                tc_mma_bf16_pair(d_tmem, umma_desc_sw128(smem_u32(sa + (size_t)dpc * CHUNK_BYTES)),
+                                 umma_desc_sw128(smem_u32(sb + (size_t)s * B_CHUNK_BYTES2)), IDESC_F16_M256_N2, 1u);
+                tc_commit_pair(&empty[s]);
+            }
+            g += (uint32_t)dpc + 1u;
             tc_commit_pair(&tfull[acc]);
             if (it + 1 < it1 && (it + 1) / CT != rp) tc_commit_pair(a_empty);   // A' may be overwritten once these retire
         }
@@ -784,11 +761,12 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         const BandParams bp{p.band_rel, p.band_abs_sqrt, p.band_abs_const};
         constexpr int NCOLS = TILE_N2 / EPI_GROUPS;
         int cur_rp = -1, row = 0;
-        float out_scale = 2.f;                                  // accumulator -> distance: -2, and 1/s^2 in fp16 mode
-        if (p.absmax_bits) { float s_, is2, mp; l2_scale_from_bits(__ldcg(p.absmax_bits), s_, is2, mp); out_scale = 2.f * is2; }
+        float s_, is2, mp;                                      // accumulator -> distance: -2 / s^2
+        l2_scale_from_bits(__ldcg(p.absmax_bits), s_, is2, mp);
+        const float out_scale = 2.f * is2;
         auto flush = [&]() {
             if (cur_rp < 0 || row >= p.n1) return;
-            const int slot = p.flat ? cid - l2_segment_of_item(cur_rp * CT, items, clusters) : (int)blockIdx.y;
+            const int slot = cid - l2_segment_of_item(cur_rp * CT, items, clusters);
             const size_t o = ((size_t)slot * p.n1 + row) * CAND + (size_t)eg * TOPK;
 #pragma unroll
             for (int k = 0; k < TOPK; k++) {
@@ -812,7 +790,6 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             if (warp == 4 && lane == 0 && t < 36) l2_stamp(p, 40 + t);
             const int jbase = ct * TILE_N2 + eg * NCOLS;
             const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + (uint32_t)(acc * TILE_N2 + eg * NCOLS);
-            if (!(p.dbg_flags & 1))
             epilogue_reduce<NCOLS, DBG>(taddr, jbase, p.n2, p.key_mask, rt, bp,
                                         DBG && p.dbg_dist && row < p.n1 ? p.dbg_dist + (size_t)row * p.n2 : nullptr, out_scale);
             tc_fence_before();

@@ -66,20 +66,16 @@ struct pgm_handle {
     bool tail_attr_set[5] = {false, false, false, false, false};
     bool l2_attr_set = false;         // cudaFuncSetAttribute is per device, hence per handle
     int l2_max_clusters = 1;          // co-resident CTA pairs of the float pair kernel (persistent grid)
-    bool l2_force_single = false;     // PGM_L2_SINGLE=1: never use the CTA-pair (cta_group::2) float kernel
     unsigned *l2_hdr = nullptr;       // fp16 ranking mode of the last float call: [max |x| bits, rows recomputed exhaustively]
-    bool force_multilaunch = false;   // PGM_FORCE_MULTILAUNCH=1: never use the persistent tail kernel
     DevBuf lat_state;             // LatState of latency mode (pgm_kernels.cuh): zeroed before its first use, left clean by every call
     bool lat_dirty = false;       // a latency-mode call was cut short between its launches: zero lat_state before the next
     bool stats_pending = false;   // rounds / evals of the last latency-mode call still sit in lat_state (device) ...
     bool stats_copied = false;    // ... or, once a read-back has been enqueued, in the pinned slot pending_plan points at
     void *pending_plan = nullptr;
-    bool tail_plain_launch = false;  // PGM_TAIL_PLAIN_LAUNCH=1 (experiment): non-cooperative launch of the tail kernel
     bool tail_timeline = false;      // PGM_TAIL_TIMELINE=1: dump the tail kernel's phase timeline to stderr (debug)
     DevBuf timeline;
     bool fin_attr_set[5] = {false, false, false, false, false};
     bool sparse_attr_set = false;
-    bool no_cand = false;            // PGM_NO_CAND=1: classic rounds only, no candidate edges / sparse sub-rounds (A/B)
     // profiling mode (pgm_set_profiling): events around every round-kernel launch
     bool profiling = false;
     std::vector<cudaEvent_t> prof_events;   // 2 per round
@@ -200,14 +196,6 @@ extern "C" int pgm_create(int device_ordinal, pgm_handle **out) {
         return PGM_E_CUDA;
     }
     h->stream = h->own_stream;
-    const char *fm = getenv("PGM_FORCE_MULTILAUNCH");
-    h->force_multilaunch = fm && fm[0] == '1';
-    const char *ls = getenv("PGM_L2_SINGLE");
-    h->l2_force_single = ls && ls[0] == '1';
-    const char *pl = getenv("PGM_TAIL_PLAIN_LAUNCH");
-    h->tail_plain_launch = pl && pl[0] == '1';
-    const char *nc = getenv("PGM_NO_CAND");
-    h->no_cand = nc && nc[0] == '1';
     const char *tl = getenv("PGM_TAIL_TIMELINE");
     h->tail_timeline = tl && tl[0] == '1';
     *out = h;
@@ -306,10 +294,6 @@ static cudaError_t launch_tail(pgm_handle *h, Chunk c, int r_start, int nbins, u
         if (e != cudaSuccess) return e;
         h->tail_attr_set[WORDS / 4] = true;
     }
-    if (h->tail_plain_launch) {
-        tail_kernel<WORDS><<<h->num_sms, TAIL_THREADS, smem, s>>>(c, r_start, nbins, flags, oq, ot, od);
-        return cudaGetLastError();
-    }
     void *args[] = {&c, &r_start, &nbins, &flags, &oq, &ot, &od};
     return cudaLaunchCooperativeKernel((void *)tail_kernel<WORDS>, dim3(h->num_sms), dim3(TAIL_THREADS), args, smem, s);
 }
@@ -371,16 +355,12 @@ struct HostPair {
     const uint8_t *d_q, *d_t;   // device pointers
     int32_t n1, n2;
     int64_t out_base;           // in rows, relative to the chunk's output arrays
-    int32_t col_id_offset = 0;
-    int32_t flags = 0;
 };
 
 static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // Rounds with at least this many live cells use the large (512-row, RQ = 4) tiles: two such tiles per SM.
-// PGM_LARGE_TILE_MIN_EVALS overrides it (tuning experiments).
 static long long large_tile_min_evals(const pgm_handle *h) {
-    if (const char *e = getenv("PGM_LARGE_TILE_MIN_EVALS")) return atoll(e);
     return 2ll * h->num_sms * ROUND_THREADS * RQ_LARGE * STAGE_LARGE;
 }
 
@@ -407,7 +387,7 @@ static int run_chunk(pgm_handle *h, const HostPair *pairs, int n_pairs, int desc
     const size_t o_st = take(n_pairs);
     const size_t o_small = take(sizeof(SmallInfo) * n_pairs);
     const size_t o_plan = take(sizeof(PlanInfo));
-    const bool latency_mode = n_pairs <= LATENCY_MODE_MAX_PAIRS && !h->force_multilaunch;
+    const bool latency_mode = n_pairs <= LATENCY_MODE_MAX_PAIRS;
     // latency mode: global scratch for the finisher's matrices / first-round minima (finisher_prepare)
     const size_t o_find = latency_mode ? take((size_t)n_pairs * FIN_D_STRIDE * 2) : 0;
     const size_t o_finr = latency_mode ? take((size_t)n_pairs * FIN_PARTS * FIN_MAX_DIM * 4) : 0;
@@ -416,26 +396,21 @@ static int run_chunk(pgm_handle *h, const HostPair *pairs, int n_pairs, int desc
     const size_t o_ocnt = latency_mode ? take((size_t)n_pairs * ORDER_MAX_SLICES * ORDER_BIN_PITCH * 4) : 0;
     // candidate edges (pgm_kernels.cuh): per pair a raw list of about 2 x CAND_TARGET entries per row and a list of the
     // edges that survive the accept, sized for the sparse phase's shared memory
-    const bool use_cand = !h->no_cand;
     // a few pairs (latency mode): the single-CTA sparse phase is on the critical path, keep its edge list short; batches:
     // the sparse phases of different pairs run side by side, a longer list saves more recomputation than it costs
-    float cand_target = n_pairs <= LATENCY_MODE_MAX_PAIRS ? CAND_TARGET : CAND_TARGET_BATCH;
-    if (const char *e = getenv("PGM_CAND_TARGET")) cand_target = std::max(0.1f, (float)atof(e));   // tuning experiments
+    const float cand_target = n_pairs <= LATENCY_MODE_MAX_PAIRS ? CAND_TARGET : CAND_TARGET_BATCH;
     std::vector<int64_t> cand_off(n_pairs + 1, 0), ledge_off(n_pairs + 1, 0);
-    if (use_cand) {
-        for (int p = 0; p < n_pairs; p++) {
-            const int64_t cells = (int64_t)pairs[p].n1 * pairs[p].n2;
-            const int64_t cap = pairs[p].flags & PAIR_FLAG_NO_EMIT ? 0
-                                : std::min<int64_t>(cells, (int64_t)(2.0f * cand_target + 1.0f) * std::max(pairs[p].n1, pairs[p].n2) + 1024);
-            cand_off[p + 1] = cand_off[p] + cap;
-            ledge_off[p + 1] = ledge_off[p] + std::min<int64_t>(cap, SP_LCAP_MAX);
-        }
+    for (int p = 0; p < n_pairs; p++) {
+        const int64_t cells = (int64_t)pairs[p].n1 * pairs[p].n2;
+        const int64_t cap = std::min<int64_t>(cells, (int64_t)(2.0f * cand_target + 1.0f) * std::max(pairs[p].n1, pairs[p].n2) + 1024);
+        cand_off[p + 1] = cand_off[p] + cap;
+        ledge_off[p + 1] = ledge_off[p] + std::min<int64_t>(cap, SP_LCAP_MAX);
     }
-    const size_t o_cand = use_cand ? take(16 * (size_t)cand_off[n_pairs]) : 0;   // two words per record
-    const size_t o_ledge = use_cand ? take(8 * (size_t)ledge_off[n_pairs]) : 0;
-    const size_t o_ccnt = use_cand ? take(4 * (size_t)n_pairs) : 0, o_lcnt = use_cand ? take(4 * (size_t)n_pairs) : 0;
-    const size_t o_thr = use_cand ? take(4 * (size_t)n_pairs) : 0, o_pstat = use_cand ? take(sizeof(PairStat) * (size_t)n_pairs) : 0;
-    const size_t o_rpos = use_cand ? take(4 * rows) : 0, o_cpos = use_cand ? take(4 * cols) : 0;
+    const size_t o_cand = take(16 * (size_t)cand_off[n_pairs]);   // two words per record
+    const size_t o_ledge = take(8 * (size_t)ledge_off[n_pairs]);
+    const size_t o_ccnt = take(4 * (size_t)n_pairs), o_lcnt = take(4 * (size_t)n_pairs);
+    const size_t o_thr = take(4 * (size_t)n_pairs), o_pstat = take(sizeof(PairStat) * (size_t)n_pairs);
+    const size_t o_rpos = take(4 * rows), o_cpos = take(4 * cols);
     int rc = ensure_dev(h, h->state, off);
     if (rc) return rc;
     rc = ensure_host(h, h->pin_meta, sizeof(PairDesc) * n_pairs + 512);
@@ -452,7 +427,6 @@ static int run_chunk(pgm_handle *h, const HostPair *pairs, int n_pairs, int desc
     c.num_sms = h->num_sms;
     c.ctas_per_sm = latency_mode ? TAIL_THREADS / ROUND_THREADS : ctas_per_sm;
     c.ctas_per_sm0 = latency_mode ? ctas_per_sm : 0;    // round 0 of latency mode is a standalone launch at full occupancy
-    if (const char *e = getenv("PGM_SLOTS_PER_SM")) c.ctas_per_sm = c.ctas_per_sm0 = std::max(1, atoi(e));   // tuning experiments
     c.fin_max_evals = latency_mode ? FIN_MAX_EVALS_TAIL : FIN_MAX_EVALS;
     c.large_min_evals = large_tile_min_evals(h);
     if (latency_mode) {
@@ -489,13 +463,10 @@ static int run_chunk(pgm_handle *h, const HostPair *pairs, int n_pairs, int desc
     // a few pairs: later passes list at most 16 candidates per row (the sparse phase of a pass runs on ONE SM and sits on
     // the call's critical path; measured best at 4096^2 ... 16384^2); batches: the list budget alone decides
     c.cand_row_max = latency_mode ? 16.0f : 1e9f;
-    if (const char *e = getenv("PGM_CAND_ROW_MAX")) c.cand_row_max = std::max(0.1f, (float)atof(e));   // tuning experiments
-    if (use_cand) {
-        c.cand = (unsigned long long *)(base + o_cand); c.ledge = (unsigned long long *)(base + o_ledge);
-        c.cand_cnt = (int32_t *)(base + o_ccnt); c.ledge_cnt = (int32_t *)(base + o_lcnt);
-        c.thr = (uint32_t *)(base + o_thr); c.pstat = (PairStat *)(base + o_pstat);
-        c.row_pos = (int32_t *)(base + o_rpos); c.col_pos = (int32_t *)(base + o_cpos);
-    }
+    c.cand = (unsigned long long *)(base + o_cand); c.ledge = (unsigned long long *)(base + o_ledge);
+    c.cand_cnt = (int32_t *)(base + o_ccnt); c.ledge_cnt = (int32_t *)(base + o_lcnt);
+    c.thr = (uint32_t *)(base + o_thr); c.pstat = (PairStat *)(base + o_pstat);
+    c.row_pos = (int32_t *)(base + o_rpos); c.col_pos = (int32_t *)(base + o_cpos);
     c.timeline = nullptr;
     if (h->tail_timeline) {
         if ((rc = ensure_dev(h, h->timeline, 1000 * 8))) return rc;
@@ -512,7 +483,7 @@ static int run_chunk(pgm_handle *h, const HostPair *pairs, int n_pairs, int desc
         hp[p].t = (const uint32_t *)pairs[p].d_t;
         hp[p].n1 = pairs[p].n1; hp[p].n2 = pairs[p].n2;
         hp[p].row_base = rb; hp[p].col_base = cb; hp[p].out_base = pairs[p].out_base;
-        hp[p].col_id_offset = pairs[p].col_id_offset; hp[p].flags = pairs[p].flags;
+        hp[p].col_id_offset = 0; hp[p].flags = 0;
         hp[p].cand_off = cand_off[p]; hp[p].ledge_off = ledge_off[p];
         hp[p].cand_cap = (int32_t)(cand_off[p + 1] - cand_off[p]); hp[p].ledge_cap = (int32_t)(ledge_off[p + 1] - ledge_off[p]);
         rb += pairs[p].n1; cb += pairs[p].n2;
@@ -612,19 +583,16 @@ static int run_chunk(pgm_handle *h, const HostPair *pairs, int n_pairs, int desc
             dispatch_round(words, c, r, round_grid, s);
             if (pr) CU_CHECK(h, cudaEventRecord(h->prof_events[2 * r + 1], s));
             accept_kernel<<<accept_grid, ACCEPT_THREADS, 0, s>>>(c, r);        // + candidate-edge filter
-            if (use_cand) {                                                     // sparse sub-rounds, then the plan of r + 1
-                if (!h->sparse_attr_set) {
-                    CU_CHECK(h, cudaFuncSetAttribute(sparse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SP_SMEM_BYTES));
-                    h->sparse_attr_set = true;
-                }
-                sparse_kernel<<<std::min(n_pairs, h->num_sms * 4), SP_THREADS, SP_SMEM_BYTES, s>>>(c, r);
-                h->stats.kernel_launches += 1;
+            if (!h->sparse_attr_set) {                                          // sparse sub-rounds, then the plan of r + 1
+                CU_CHECK(h, cudaFuncSetAttribute(sparse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SP_SMEM_BYTES));
+                h->sparse_attr_set = true;
             }
+            sparse_kernel<<<std::min(n_pairs, h->num_sms * 4), SP_THREADS, SP_SMEM_BYTES, s>>>(c, r);
             if (pr) {
                 CU_CHECK(h, cudaMemcpyAsync(&prof_plan[r + 1], c.plan, sizeof(PlanInfo), cudaMemcpyDeviceToHost, s));
                 h->prof_rounds = r + 1;
             }
-            h->stats.kernel_launches += 2;
+            h->stats.kernel_launches += 3;
         }
         // pairs that became small wait in place (SmallInfo) until this launch
         CU_CHECK(h, dispatch_fin(h, words, c, s));
@@ -1337,12 +1305,9 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
     cudaStream_t s = h->stream;
     const int dp = (dim + CHUNK_K - 1) / CHUNK_K * CHUNK_K, dpc = dp / CHUNK_K;
     const int row_tiles = (n1 + TILE_M - 1) / TILE_M;
-    // CTA pairs (cta_group::2, M = 256 x N = 256) whenever there are at least two row tiles
-    const bool pair = row_tiles >= 2 && !h->l2_force_single;
-    // ranking precision: one fp16 term + certified band + exhaustive fallback (pair kernel, default), or the
-    // three-term bf16 split (PGM_L2_MODE=bf16x3, and always for the single-CTA kernel)
-    const char *mode_env = getenv("PGM_L2_MODE");
-    const bool fp16 = pair && !(mode_env && !strcmp(mode_env, "bf16x3"));
+    // CTA pairs (cta_group::2, M = 256 x N = 256) whenever there are at least two row tiles.  Ranking precision: one
+    // fp16 term + certified band + exhaustive fallback (pair kernel), or the three-term bf16 split (single-CTA kernel)
+    const bool pair = row_tiles >= 2, fp16 = pair;
     const int kprime = fp16 ? dp + CHUNK_K : 2 * dp + CHUNK_K;   // rows = [x16 | norm] or [hi | lo | norm]
     if (!h->l2_attr_set) {
         CU_CHECK(h, cudaFuncSetAttribute(l2_topk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_smem_bytes()));
@@ -1364,40 +1329,31 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
         h->l2_max_clusters = std::min(nc, std::max(1, h->num_sms / 2));
         h->l2_attr_set = true;
     }
-    int splits = 1, tps = 0, gx = row_tiles, col_tiles, items = 0, clusters = 0, flat = 0;
+    int splits = 1, tps = 0, items = 0, clusters = 0;
     const int row_pairs = (row_tiles + 1) / 2;
-    const int slots_avail = pair ? h->l2_max_clusters : h->num_sms;      // co-resident work units
-    col_tiles = (n2 + (pair ? TILE_N2 : TILE_N) - 1) / (pair ? TILE_N2 : TILE_N);
-    {
+    const int col_tiles = (n2 + (pair ? TILE_N2 : TILE_N) - 1) / (pair ? TILE_N2 : TILE_N);
+    if (pair) {
+        // equal contiguous segments of the row-major (row pair, column tile) list, one per resident cluster: no wave
+        // quantisation (DESIGN.md section 4.2)
+        const long long total = (long long)row_pairs * col_tiles;
+        if (total > 0x7FFFFFFFll) return fail(h, PGM_E_INVALID_ARG, "problem too large for the float path");
+        items = (int)total;
+        clusters = std::min(h->l2_max_clusters, items);
+        // a row pair's candidates come from every segment that touches it: slots = the most any row pair sees
+        for (int rp = 0; rp < row_pairs; rp++) {
+            const long long x0 = (long long)rp * col_tiles, x1 = x0 + col_tiles - 1;
+            const int k0 = (int)(((x0 + 1) * clusters - 1) / items), k1 = (int)(((x1 + 1) * clusters - 1) / items);
+            splits = std::max(splits, k1 - k0 + 1);
+        }
+    } else {
         // column splits: the run time is (waves) x (tiles per split); pick the split count that minimises it
         // (half a tile of fixed cost per unit for the resident A' load)
-        const int units = pair ? row_pairs : row_tiles;
         tps = col_tiles;
         double best_cost = 1e300;
         for (int sp = 1; sp <= std::min(col_tiles, 32); sp++) {
             const int t = (col_tiles + sp - 1) / sp, se = (col_tiles + t - 1) / t;
-            const double cost = (double)(((long long)units * se + slots_avail - 1) / slots_avail) * (t + 0.5);
+            const double cost = (double)(((long long)row_tiles * se + h->num_sms - 1) / h->num_sms) * (t + 0.5);
             if (cost < best_cost - 1e-9) { best_cost = cost; splits = se; tps = t; }
-        }
-        if (pair) {
-            // flat form (default): equal contiguous segments of the row-major (row pair, column tile) list, one per
-            // resident cluster -- no wave quantisation.  A/B on one B200 (PGM_L2_FLAT=0 forces the split form):
-            // 8k 63.3 vs 64.9 us, 32k 0.557 vs 0.618 ms, 65k 2.08 vs 2.15 ms, 32k x D=64 0.45 vs 0.53 ms.
-            const long long total = (long long)row_pairs * col_tiles;
-            if (total > 0x7FFFFFFFll) return fail(h, PGM_E_INVALID_ARG, "problem too large for the float path");
-            items = (int)total;
-            clusters = std::min(h->l2_max_clusters, items);
-            const char *force = getenv("PGM_L2_FLAT");
-            flat = force ? (force[0] == '1') : 1;
-            if (flat) {
-                // a row pair's candidates come from every segment that touches it: slots = the most any row pair sees
-                splits = 1;
-                for (int rp = 0; rp < row_pairs; rp++) {
-                    const long long x0 = (long long)rp * col_tiles, x1 = x0 + col_tiles - 1;
-                    const int k0 = (int)(((x0 + 1) * clusters - 1) / items), k1 = (int)(((x1 + 1) * clusters - 1) / items);
-                    splits = std::max(splits, k1 - k0 + 1);
-                }
-            }
         }
     }
     // scratch: A' | B' | cand_j | cand_d
@@ -1418,7 +1374,7 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
     char *base = (char *)h->misc.p;
     __nv_bfloat16 *a = (__nv_bfloat16 *)(base + o_a), *b = (__nv_bfloat16 *)(base + o_b);
     L2Params p{};
-    p.n1 = n1; p.n2 = n2; p.dpc = dpc; p.tiles_per_split = tps; p.col_tiles = col_tiles; p.items = items; p.flat = flat;
+    p.n1 = n1; p.n2 = n2; p.dpc = dpc; p.tiles_per_split = tps; p.col_tiles = col_tiles; p.items = items;
     p.key_mask = 0x7FFFFFE0u;
     unsigned *hdr = fp16 ? (unsigned *)h->l2_state.p : nullptr;
     int32_t *ovf_rows = fp16 ? (int32_t *)(base + o_ovf) : nullptr;
@@ -1432,9 +1388,6 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
     p.band_rel = 0.5f * slack_rel;
     p.band_abs_sqrt = fp16 ? 4.8828125e-7f * sqrtf((float)dp) : 0.f;     // 2^-21 sqrt(D) sqrt(3|q|^2 + 4|a|)
     p.band_abs_const = fp16 ? 2.44140625e-4f : 0.f;                        // 2^-12
-    { const char *df = getenv("PGM_L2_DBG"); p.dbg_flags = df ? atoi(df) : 0; }
-    p.nparts = fp16 ? 1 : 2;
-    p.idesc = fp16 ? (IDESC_BF16_M256_N2 & ~((1u << 7) | (1u << 10))) : IDESC_BF16_M256_N2;   // A/B format field 0 = F16, 1 = BF16
     p.absmax_bits = hdr;
     h->l2_hdr = hdr;
     p.cand_j = (int32_t *)(base + o_cj); p.cand_d = (float *)(base + o_cd); p.dbg_dist = d_dbg;
@@ -1466,12 +1419,12 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
     if ((rc = make_operand_map(h, &map_b, b, n2, kprime, pair ? B_ROWS2 : TILE_N))) return rc;
     cfg.blockDim = dim3(THREADS);
     if (pair) {
-        cfg.gridDim = flat ? dim3(2 * (unsigned)clusters) : dim3(2 * (unsigned)row_pairs, (unsigned)splits);
+        cfg.gridDim = dim3(2 * (unsigned)clusters);
         cfg.dynamicSmemBytes = l2_pair_smem_bytes();
         if (d_dbg) CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_pair_kernel<true>, map_a, map_b, p));
         else CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_pair_kernel<false>, map_a, map_b, p));
     } else {
-        cfg.gridDim = dim3(gx, splits); cfg.dynamicSmemBytes = l2_smem_bytes();
+        cfg.gridDim = dim3(row_tiles, splits); cfg.dynamicSmemBytes = l2_smem_bytes();
         if (d_dbg) CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_kernel<true>, map_a, map_b, p));
         else CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_kernel<false>, map_a, map_b, p));
     }
@@ -1479,9 +1432,7 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
     CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_refine_kernel, d_q, n1, d_t, n2, dim, (const int32_t *)p.cand_j,
                                    (const float *)p.cand_d, (const float *)p.cand_drop, splits, d_bj, d_bd, d_sj, d_sd,
                                    slack_rel, hdr, ovf_rows));
-    if (fp16 && getenv("PGM_L2_NO_FALLBACK")) {        // (debug switch: time the call without the exhaustive fallback)
-        CU_CHECK(h, cudaMemsetAsync(hdr, 0, 4, s));
-    } else if (fp16) {
+    if (fp16) {
         cfg.gridDim = dim3((unsigned)h->num_sms * 4); cfg.blockDim = dim3(EX_THREADS);
         CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_exact_rows_kernel, d_q, (int)n1, d_t, (int)n2, (int)dim, hdr,
                                        (const int32_t *)ovf_rows, (float4 *)(base + o_part), d_bj, d_bd, d_sj, d_sd));
@@ -1490,8 +1441,8 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
         std::vector<unsigned long long> v(256);
         CU_CHECK(h, cudaMemcpyAsync(v.data(), h->timeline.p, 256 * 8, cudaMemcpyDeviceToHost, s));
         CU_CHECK(h, cudaStreamSynchronize(s));
-        fprintf(stderr, "[pgm l2 plan] pair %d flat %d max_clusters %d clusters %d row_pairs %d col_tiles %d splits %d tps %d\n", (int)pair,
-                flat, h->l2_max_clusters, clusters, row_pairs, col_tiles, splits, tps);
+        fprintf(stderr, "[pgm l2 plan] pair %d max_clusters %d clusters %d row_pairs %d col_tiles %d splits %d tps %d\n", (int)pair,
+                h->l2_max_clusters, clusters, row_pairs, col_tiles, splits, tps);
         fprintf(stderr, "[pgm l2 timeline us] sync %.2f pdl %.2f a_ready %.2f |", (v[1] - v[0]) * 1e-3, (v[2] - v[0]) * 1e-3,
                 (v[3] - v[0]) * 1e-3);
         for (int t = 0; t < 36 && v[4 + t]; t++)
@@ -2053,11 +2004,10 @@ extern "C" int pgm_shard_create(pgm_handle *h, const uint8_t *d_q, int32_t n1, c
     sh->q_host_ptr = (const uint32_t *)d_q; sh->t_host_ptr = (const uint32_t *)d_t_local;
     const int64_t rows = n1, cols = std::max(n2_local, 1);
     const int n_blocks = (n1 + SHARD_BLOCK - 1) / SHARD_BLOCK;
-    const bool use_cand = !h->no_cand;
     // this rank's share of the pass's candidate records (x 1.25 slack), by its share of the columns
-    sh->raw_cap = use_cand ? (int)std::min<int64_t>(
+    sh->raw_cap = (int)std::min<int64_t>(
         (int64_t)((2.0f * CAND_TARGET_SHARD + 1.0f) * 1.25f * (float)std::max(n1, n2_total) * ((float)cols / (float)n2_total)) + 4096,
-        (int64_t)n1 * cols) : 0;
+        (int64_t)n1 * cols);
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
     const size_t o_pairs = take(sizeof(PairDesc));
@@ -2090,7 +2040,6 @@ extern "C" int pgm_shard_create(pgm_handle *h, const uint8_t *d_q, int32_t n1, c
     c.cand_target = CAND_TARGET_SHARD;
     c.cand_row_max = 1e9f;
     c.sp_slots_max = SP_EPT;
-    if (const char *e = getenv("PGM_CAND_TARGET")) c.cand_target = std::max(0.1f, (float)atof(e));
     c.rowbest[0] = (uint32_t *)(base + o_rb0); c.rowbest[1] = (uint32_t *)(base + o_rb1);
     c.colbest[0] = (uint32_t *)(base + o_cb0); c.colbest[1] = (uint32_t *)(base + o_cb1);
     c.live_rows[0] = (int32_t *)(base + o_lr0); c.live_rows[1] = (int32_t *)(base + o_lr1);
@@ -2099,11 +2048,10 @@ extern "C" int pgm_shard_create(pgm_handle *h, const uint8_t *d_q, int32_t n1, c
     c.tile_base = (int32_t *)(base + o_tb); c.ablock_base = (int32_t *)(base + o_ab);
     c.status = (uint8_t *)(base + o_st); c.small = (SmallInfo *)(base + o_small); c.plan = (PlanInfo *)(base + o_plan);
     c.row_pos = (int32_t *)(base + o_rpos);
-    if (use_cand) {                // candidate records of the pass; the edges themselves live in the caller's exchange buffer
-        c.cand = (unsigned long long *)(base + o_cand);
-        c.cand_cnt = (int32_t *)(base + o_ccnt); c.ledge_cnt = c.cand_cnt;   // (ledge_cnt is only reset by the planner here)
-        c.thr = (uint32_t *)(base + o_thr); c.pstat = (PairStat *)(base + o_pstat);
-    }
+    // candidate records of the pass; the edges themselves live in the caller's exchange buffer
+    c.cand = (unsigned long long *)(base + o_cand);
+    c.cand_cnt = (int32_t *)(base + o_ccnt); c.ledge_cnt = c.cand_cnt;   // (ledge_cnt is only reset by the planner here)
+    c.thr = (uint32_t *)(base + o_thr); c.pstat = (PairStat *)(base + o_pstat);
     c.timeline = nullptr;
     sh->coldead = (uint8_t *)(base + o_dead);
     sh->blockcnt = (int32_t *)(base + o_bcnt);
@@ -2156,13 +2104,9 @@ static int shard_enqueue_commit(pgm_shard *sh, const uint32_t *d_x, int bound, u
     shard_commit_mark_kernel<<<nb, SHARD_BLOCK, 0, s>>>(sh->c, r, d_x, bound, sh->coldead);
     h->stats.kernel_launches += 1;
     if (d_edges) {
-        if (sh->c.cand) {
-            shard_filter_kernel<<<h->num_sms * 4, ACCEPT_THREADS, 0, s>>>(sh->c, r, sh->coldead, d_edges, edge_cap, &sh->dev->edge_cnt,
-                                                                         &sh->dev->ticket);
-            h->stats.kernel_launches += 1;
-        } else {
-            CU_CHECK(h, cudaMemsetAsync(d_edges, 0, 8, s));       // no candidate edges: count 0
-        }
+        shard_filter_kernel<<<h->num_sms * 4, ACCEPT_THREADS, 0, s>>>(sh->c, r, sh->coldead, d_edges, edge_cap, &sh->dev->edge_cnt,
+                                                                     &sh->dev->ticket);
+        h->stats.kernel_launches += 1;
     }
     return PGM_OK;
 }
@@ -2172,7 +2116,7 @@ static int shard_enqueue_finish_round(pgm_shard *sh, const unsigned long long *d
                                       cudaStream_t s) {
     pgm_handle *h = sh->h;
     const int r = sh->round;
-    if (d_edges_all && sh->c.cand && n_ranks >= 1) {
+    if (d_edges_all && n_ranks >= 1) {
         int rc = ensure_dev(h, sh->est, (size_t)n_ranks * edge_cap);
         if (rc) return rc;
         Chunk c = sh->c;
@@ -2485,7 +2429,7 @@ extern "C" int pgm_multi_match_train_sharded_dev(pgm_multi *mh, const uint8_t *d
         if (cudaSetDevice(h->device) != cudaSuccess) { rc = PGM_E_CUDA; }
         cudaStream_t s = h->stream;
         const int edge_cap = shard_edge_capacity(n1, n2_total, mh->world);
-        const bool edges_on = sh->c.cand != nullptr && mh->world <= 64;
+        const bool edges_on = mh->world <= 64;
         const size_t x_bytes = align_up((size_t)2 * n1 * 4, 256);
         if (!rc) rc = ensure_dev(h, mh->xbuf, x_bytes + (edges_on ? (size_t)mh->world * (1 + (size_t)edge_cap) * 8 : 0));
         uint32_t *X = (uint32_t *)mh->xbuf.p;
@@ -2494,7 +2438,6 @@ extern "C" int pgm_multi_match_train_sharded_dev(pgm_multi *mh, const uint8_t *d
         // nothing), then the replicated finish.  Every rank reads the same status, so all ranks take the same path.
         int bound = n1;
         bool done = false;
-        const bool no_fin = getenv("PGM_SHARD_NO_REPLICATED_FINISH") != nullptr;
         const bool timing = getenv("PGM_SHARD_TIMING") != nullptr;      // debug: host wall time of every round (stream is idle at each mark)
         auto t_prev = std::chrono::steady_clock::now();
         auto mark = [&](const char *what, int a) {
@@ -2530,7 +2473,7 @@ extern "C" int pgm_multi_match_train_sharded_dev(pgm_multi *mh, const uint8_t *d
             done = sh->h_ctl[0].done != 0;
             mark("round, live rows after", live);
             bound = std::min(bound, std::max(SHARD_BLOCK, (live + SHARD_BLOCK - 1) / SHARD_BLOCK * SHARD_BLOCK));
-            if (!done && !no_fin && live <= SHARD_FINISH_MAX && (int64_t)n2_total - (n1 - live) <= SHARD_FINISH_MAX) {
+            if (!done && live <= SHARD_FINISH_MAX && (int64_t)n2_total - (n1 - live) <= SHARD_FINISH_MAX) {
                 rc = shard_replicated_finish(mh, sh, live, s);
                 done = true;
                 mark("replicated finish of rows", live);

@@ -325,7 +325,7 @@ class Matcher:
 
     def l2_last_fallback_rows(self) -> int:
         """Queries of the last float call that were recomputed exhaustively (their candidate band could not be
-        certified from the kernel's top-4 lists); -1 if that call used the three-term bf16 ranking."""
+        certified from the kernel's top-8 lists); -1 if that call used the three-term bf16 ranking."""
         return int(self._lib.pgm_l2_last_fallback_rows(self._h))
 
     # -- the producer of the matcher's inputs: FAST-12, BRIEF, NMS ----------

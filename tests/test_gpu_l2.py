@@ -36,6 +36,8 @@ def test_l2_knn2_random(matcher, n1, n2, dim):
     q = rng.standard_normal((n1, dim)).astype(np.float32)
     t = rng.standard_normal((n2, dim)).astype(np.float32)
     _check(matcher, q, t)
+    if n1 <= 128:                                   # the single-CTA kernel ranks with the three-term bf16 split
+        assert matcher.l2_last_fallback_rows() == -1
 
 
 def test_l2_noisy_copies_small_distances(matcher):
@@ -82,12 +84,10 @@ def test_l2_zero_rows(matcher):
     _check(matcher, q, t)
 
 
-@pytest.mark.parametrize("flat", ["0", "1"])
 @pytest.mark.parametrize("n1,n2,dim", [(300, 500, 128), (1000, 2100, 64), (2600, 1300, 128), (257, 9000, 32)])
-def test_l2_both_work_distributions(matcher, monkeypatch, flat, n1, n2, dim):
-    # the CTA-pair kernel distributes (row pair, column tile) items either as (row pair, column split) waves or as
-    # equal flat segments (a segment may cross row pairs: A' reload, candidate slots per segment); same answers
-    monkeypatch.setenv("PGM_L2_FLAT", flat)
+def test_l2_both_work_distributions(matcher, n1, n2, dim):
+    # the CTA-pair kernel cuts the (row pair, column tile) items into equal segments, one per resident cluster (a
+    # segment may cross row pairs: A' reload, candidate slots per segment)
     rng = np.random.default_rng(n1 + n2 + dim)
     q = rng.standard_normal((n1, dim)).astype(np.float32)
     t = rng.standard_normal((n2, dim)).astype(np.float32)
@@ -103,18 +103,7 @@ def test_l2_underfilled_grid_shape(matcher):
     _check(matcher, q, t)
 
 
-# ---- ranking modes (round 2): one fp16 term + certified band + exhaustive fallback (default for n1 > 128) vs the
-# ---- three-term bf16 split ------------------------------------------------------------------------------------
-@pytest.mark.parametrize("n1,n2,dim", [(300, 500, 128), (2600, 1300, 128), (1000, 2100, 64)])
-def test_l2_bf16x3_mode_still_agrees(matcher, monkeypatch, n1, n2, dim):
-    monkeypatch.setenv("PGM_L2_MODE", "bf16x3")
-    rng = np.random.default_rng(n1 + 3 * n2 + dim)
-    q = rng.standard_normal((n1, dim)).astype(np.float32)
-    t = rng.standard_normal((n2, dim)).astype(np.float32)
-    _check(matcher, q, t)
-    assert matcher.l2_last_fallback_rows() == -1
-
-
+# ---- ranking of the CTA-pair kernel (n1 > 128): one fp16 term + certified band + exhaustive fallback --------------
 def test_l2_fp16_mode_is_the_default_and_certifies_random_data(matcher):
     rng = np.random.default_rng(31)
     q = rng.random((4096, 128), dtype=np.float32)

@@ -97,6 +97,21 @@ def test_product_never_imports_the_oracle():
                 assert "liborc" not in src and "pgm_oracle" not in src, f
 
 
+def test_every_environment_variable_the_library_reads_is_documented():
+    """The library's getenv names are exactly the INTEGRATION.md section 5 table (PGM_LIB is read by the Python side)."""
+    csrc = os.path.join(ROOT, "photogrammetry_b200", "csrc")
+    read = set()
+    for f in os.listdir(csrc):
+        if f.endswith((".cu", ".cuh", ".h")):
+            read |= set(re.findall(r'getenv\(\s*"(PGM_[A-Z0-9_]+)"', open(os.path.join(csrc, f)).read()))
+    doc = open(os.path.join(ROOT, "INTEGRATION.md")).read()
+    section = doc.split("## 5. Diagnostics", 1)[1].split("\n## ", 1)[0]
+    documented = {m for line in section.splitlines() if line.startswith("| `PGM_")
+                  for m in re.findall(r"`(PGM_[A-Z0-9_]+)", line.split("|")[1])}
+    assert read, "no getenv calls found"
+    assert read == documented - {"PGM_LIB"}, (sorted(read - documented), sorted(documented - read - {"PGM_LIB"}))
+
+
 def test_no_gpu_fails_loudly():
     import torch
     if torch.cuda.is_available():

@@ -19,10 +19,8 @@ for n, dim in [(8192, 128), (32768, 128), (65536, 128), (32768, 64)]:
     e1.record(stream); e1.synchronize()
     ms = e0.elapsed_time(e1) / 10
     dp = (dim + 63) // 64 * 64
-    mode = os.environ.get("PGM_L2_MODE", "fp16")
-    terms = 3 if mode == "bf16x3" else 1
     alg = 2.0 * dim * n * n / (ms * 1e-3) / 1e12
-    print(json.dumps({"n": n, "dim": dim, "mode": mode, "ms": ms, "evals_per_s": n * n / (ms * 1e-3), "algorithmic_tflops(2D per eval)": alg,
+    print(json.dumps({"n": n, "dim": dim, "ms": ms, "evals_per_s": n * n / (ms * 1e-3), "algorithmic_tflops(2D per eval)": alg,
                       "algorithmic_frac_of_measured_bf16_peak": alg / peaks["bf16_tflops"],
-                      "executed_frac": 2.0 * terms * dp * n * n / (ms * 1e-3) / 1e12 / peaks["bf16_tflops"],
+                      "executed_frac": 2.0 * dp * n * n / (ms * 1e-3) / 1e12 / peaks["bf16_tflops"],
                       "fallback_rows": m.l2_last_fallback_rows()}))
