@@ -317,12 +317,25 @@ int pgm_ransac_score(pgm_handle *h, const float *F, const uint8_t *valid, int32_
  * them, pair_list[n_pairs][2] (host) names the pairs; pair p's kept triples (ascending query index) start at the sum
  * of the query sizes of the pairs before it, out_counts[p] (host) says how many.  One CTA per pair with both descriptor
  * sets in shared memory: (n1 + n2) * stride_bytes + 4 * n2 + 16 must not exceed 200 KB (204 800 bytes), else
- * PGM_E_INVALID_ARG. */
+ * PGM_E_INVALID_ARG.  Larger pairs: pgm_match_ratio_crosscheck_pairs_batch_dev, same arguments. */
 int pgm_match_ratio_crosscheck_batch_dev(pgm_handle *h, const uint8_t *d_all_desc, const int64_t *image_offsets,
                                          int32_t n_images, const int32_t *pair_list, int32_t n_pairs, int32_t desc_bits,
                                          int32_t stride_bytes, float ratio, int32_t cross_check, int32_t max_dist,
                                          int32_t *d_out_qi, int32_t *d_out_tj, int32_t *d_out_dist, int64_t capacity,
                                          int32_t *out_counts);
+
+/* The same filter for many pairs of ANY size (0 <= n1, n2 < 2^20; e.g. all pairs of an image set, BASELINE configs[4]),
+ * with the arguments, output layout and status codes of pgm_match_ratio_crosscheck_batch_dev.  Per pair the result is
+ * bit-identical to pgm_match_ratio_crosscheck on that pair; a pair with n1 == 0 or n2 == 0 keeps nothing.  One fused
+ * distance pass gives every query's best and second best train row under (distance, j) and, with cross_check, every
+ * train row's best query under (distance, i), so pgm_stats.evals_computed == distance_evals.  The pair list is processed
+ * in chunks of at most 4096 pairs and 24 M query + train rows, whose scratch is reused; the call reads back the counts
+ * once at the end (pgm_stats.host_syncs == 2) and writes no slot beyond a pair's count. */
+int pgm_match_ratio_crosscheck_pairs_batch_dev(pgm_handle *h, const uint8_t *d_all_desc, const int64_t *image_offsets,
+                                               int32_t n_images, const int32_t *pair_list, int32_t n_pairs,
+                                               int32_t desc_bits, int32_t stride_bytes, float ratio, int32_t cross_check,
+                                               int32_t max_dist, int32_t *d_out_qi, int32_t *d_out_tj,
+                                               int32_t *d_out_dist, int64_t capacity, int32_t *out_counts);
 
 /* ---- train-sharded single pair (multi-GPU, SURVEY.md section 8e) ----------
  * For ONE huge pair (BASELINE configs[3]: 200k x 200k; the call it shards is MatchKeypoints,

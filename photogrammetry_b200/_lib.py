@@ -35,7 +35,7 @@ EXPORTED_SYMBOLS = (
     "pgm_match_hamming_greedy", "pgm_match_hamming_greedy_dev",
     "pgm_match_pairs_batch", "pgm_match_pairs_batch_dev",
     "pgm_knn2_hamming", "pgm_knn2_hamming_dev", "pgm_match_ratio_crosscheck", "pgm_match_ratio_crosscheck_batch_dev",
-    "pgm_pack_top2_keys_dev", "pgm_merge_top2_dev", "pgm_ratio_crosscheck_filter_dev",
+    "pgm_match_ratio_crosscheck_pairs_batch_dev", "pgm_pack_top2_keys_dev", "pgm_merge_top2_dev", "pgm_ratio_crosscheck_filter_dev",
     "pgm_match_keypoints_sorted", "pgm_match_keypoints_sorted_dev", "pgm_knn2_l2", "pgm_knn2_l2_dev", "pgm_l2_last_fallback_rows",
     "pgm_fast_detect", "pgm_brief_describe", "pgm_nms", "pgm_detect_describe_dev", "pgm_detect_describe_batch_dev",
     "pgm_ransac_score",
@@ -142,6 +142,7 @@ def load() -> C.CDLL:
         lib.pgm_match_ratio_crosscheck_batch_dev.argtypes = [C.c_void_p, u8p, i64p, C.c_int32, i32p, C.c_int32, C.c_int32,
                                                              C.c_int32, C.c_float, C.c_int32, C.c_int32, i32p, i32p, i32p,
                                                              C.c_int64, i32p]
+        lib.pgm_match_ratio_crosscheck_pairs_batch_dev.argtypes = lib.pgm_match_ratio_crosscheck_batch_dev.argtypes
         lib.pgm_fast_detect.argtypes = [C.c_void_p, vp, C.c_int32, C.c_int32, C.c_float, C.c_uint32, i32p, i32p,
                                         C.c_int32, C.POINTER(C.c_int32)]
         lib.pgm_brief_describe.argtypes = [C.c_void_p, vp, C.c_int32, C.c_int32, i32p, C.c_int32, i32p, C.c_int32,

@@ -2540,6 +2540,214 @@ __global__ void __launch_bounds__(RCB_THREADS) ratio_crosscheck_batch_kernel(con
 }
 
 // ---------------------------------------------------------------------------
+// Many pairs of any size (BASELINE configs[4]): nearest / second nearest, best query of every train descriptor, ratio
+// test, cross-check and max-distance filter.  Three launches per chunk of pairs:
+//   knn2_cols_pairs_kernel    one fused distance pass over flattened (pair, row tile, column split) items: the round
+//                             kernel's inner loop with top-2 row keys (d << 20 | j) in registers and, with CROSS, the
+//                             column minimum (d << 20 | i) through shared and global atomicMin -- the second distance
+//                             pass of pgm_match_ratio_crosscheck is not needed
+//   rcp_filter_kernel         merges a row's split partials as knn2_merge_kernel does, applies the filter expression of
+//                             ratio_crosscheck_kernel and counts the kept rows of each block of RCF_THREADS rows
+//   rcp_scatter_kernel        prefix of the block counts of the block's pair, ordered write of the kept triples
+// A large pair's ordered compaction is spread over ceil(n1 / RCF_THREADS) CTAs rather than walked by one.
+// ---------------------------------------------------------------------------
+struct RcpPair {
+    const uint32_t *q, *t;
+    int32_t n1, n2;
+    int64_t out_base;      // first slot of this pair's triples in the caller's output arrays
+    int64_t part_base;     // row i, split s: partial (best, second) at part[part_base + i * splits + s]
+    int64_t col_base;      // this pair's column minima in the chunk's colbest
+    int64_t row_base;      // this pair's rows in the chunk's per-row filter results
+    int32_t splits, cols_per_split;
+    int32_t pair_id;       // index in the caller's pair list (out_counts)
+    int32_t pad;
+};
+constexpr int RCF_THREADS = 1024;   // rows per filter / scatter block (n1 < 2^20: at most 1024 blocks per pair)
+
+template <int WORDS, bool CROSS>
+__global__ void __launch_bounds__(ROUND_THREADS, WORDS <= 8 ? 6 : (WORDS == 12 ? 5 : 4))
+knn2_cols_pairs_kernel(const RcpPair *__restrict__ pairs, const int32_t *__restrict__ tile_base, int n_pairs,
+                       uint2 *__restrict__ part, int64_t part_cap, uint32_t *__restrict__ colbest, int64_t col_cap) {
+    constexpr int V4 = WORDS / 4, RQ = RQ_LARGE, STAGE = STAGE_LARGE, tile_rows = ROUND_THREADS * RQ;
+    __shared__ uint4 s_t[STAGE * V4];
+    __shared__ uint32_t s_jkey[STAGE];
+    __shared__ uint32_t s_col[CROSS ? STAGE : 1];
+    const int tid = threadIdx.x, g = blockIdx.x;
+    const int p = find_pair(tile_base, n_pairs, g);
+    const RcpPair pr = pairs[p];
+    const int local = g - __ldg(tile_base + p);
+    const int rt = local / pr.splits, sp = local - rt * pr.splits;
+
+    uint32_t q[RQ][WORDS], ikey[RQ], best[RQ], second[RQ];
+#pragma unroll
+    for (int k = 0; k < RQ; k++) {
+        const int i = rt * tile_rows + k * ROUND_THREADS + tid;
+        best[k] = KEY_NONE; second[k] = KEY_NONE;
+        if (i < pr.n1) {
+            ikey[k] = (uint32_t)i;
+            const uint4 *src = reinterpret_cast<const uint4 *>(pr.q + (size_t)i * WORDS);
+#pragma unroll
+            for (int v = 0; v < V4; v++) {
+                const uint4 x = __ldg(src + v);
+                q[k][4 * v + 0] = x.x; q[k][4 * v + 1] = x.y; q[k][4 * v + 2] = x.z; q[k][4 * v + 3] = x.w;
+            }
+        } else {
+            ikey[k] = KEY_INVALID;             // a padded row never wins a column
+#pragma unroll
+            for (int w = 0; w < WORDS; w++) q[k][w] = 0u;
+        }
+    }
+
+    const int c0 = sp * pr.cols_per_split, c1 = min(pr.n2, c0 + pr.cols_per_split);
+    for (int s0 = c0; s0 < c1; s0 += STAGE) {
+        __syncthreads();                       // previous stage fully consumed
+        for (int k = tid; k < STAGE * V4; k += ROUND_THREADS) {
+            const int col = k / V4, part_i = k - col * V4, j = s0 + col;
+            uint4 x = make_uint4(0u, 0u, 0u, 0u);
+            uint32_t jk = KEY_INVALID;         // a padded column's keys exceed every real key: it never becomes a best
+            if (j < c1) {
+                x = __ldg(reinterpret_cast<const uint4 *>(pr.t + (size_t)j * WORDS) + part_i);
+                jk = (uint32_t)j;
+            }
+            s_t[k] = x;
+            if (part_i == 0) s_jkey[col] = jk;
+        }
+        if (CROSS && tid < STAGE) s_col[tid] = KEY_NONE;
+        __syncthreads();
+
+        const int ncs = min(STAGE, (c1 - s0 + 3) & ~3);
+        // as in round_tiles: no store, atomic or branch between the columns of a 4-column block
+        for (int jj0 = 0; jj0 < ncs; jj0 += 4) {
+            uint32_t cm[4];
+#pragma unroll
+            for (int u = 0; u < 4; u++) {
+                const int jj = jj0 + u;
+                uint32_t t[WORDS];
+#pragma unroll
+                for (int v = 0; v < V4; v++) {
+                    const uint4 x = s_t[jj * V4 + v];
+                    t[4 * v + 0] = x.x; t[4 * v + 1] = x.y; t[4 * v + 2] = x.z; t[4 * v + 3] = x.w;
+                }
+                const uint32_t jk = s_jkey[jj];
+                uint32_t cmin = KEY_NONE;
+#pragma unroll
+                for (int k = 0; k < RQ; k++) {
+                    // (rows alternate between the 5-POPC and the 4-POPC popcount so that the XU and ALU pipes balance)
+                    const uint32_t d = ((k & 1) ? hamming_words_deep<WORDS>(q[k], t) : hamming_words<WORDS>(q[k], t)) << KEY_IDX_BITS;
+                    const uint32_t key = d + jk;
+                    second[k] = min(second[k], max(best[k], key));
+                    best[k] = min(best[k], key);
+                    if (CROSS) cmin = min(cmin, d + ikey[k]);
+                }
+                cm[u] = cmin;
+            }
+            if (CROSS) {
+                // one warp-aggregated shared atomicMin per (warp, column)
+#pragma unroll
+                for (int u = 0; u < 4; u++) atomicMin(&s_col[jj0 + u], cm[u]);
+            }
+        }
+        if (CROSS) {
+            __syncthreads();
+            if (tid < STAGE) {
+                const uint32_t jk = s_jkey[tid], v = s_col[tid];
+                if (jk != KEY_INVALID && v < KEY_INVALID) {
+                    PGM_ASSERT((int)jk < pr.n2 && pr.col_base + (int64_t)jk < col_cap);
+                    atomicMin(colbest + pr.col_base + jk, v);
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < RQ; k++) {
+        const int i = rt * tile_rows + k * ROUND_THREADS + tid;
+        if (i < pr.n1) {
+            const int64_t slot = pr.part_base + (int64_t)i * pr.splits + sp;
+            PGM_ASSERT(slot >= 0 && slot < part_cap);
+            part[slot] = make_uint2(best[k], second[k]);
+        }
+    }
+}
+
+// res[row] = the row's best key if it passes the filter, else KEY_NONE; bcnt[block] = kept rows of the block
+__global__ void __launch_bounds__(RCF_THREADS) rcp_filter_kernel(const RcpPair *__restrict__ pairs,
+                                                                 const int32_t *__restrict__ fblk_base, int n_pairs,
+                                                                 const uint2 *__restrict__ part, int64_t part_cap,
+                                                                 const uint32_t *__restrict__ colbest, int64_t col_cap,
+                                                                 float ratio, int cross_check, int max_dist,
+                                                                 uint32_t *__restrict__ res, int32_t *__restrict__ bcnt) {
+    const int g = blockIdx.x, tid = threadIdx.x;
+    const int p = find_pair(fblk_base, n_pairs, g);
+    const RcpPair pr = pairs[p];
+    const int i = (g - __ldg(fblk_base + p)) * RCF_THREADS + tid;
+    bool keep = false;
+    if (i < pr.n1) {
+        uint32_t b = KEY_NONE, s = KEY_NONE;
+        for (int sp = 0; sp < pr.splits; sp++) {
+            const int64_t slot = pr.part_base + (int64_t)i * pr.splits + sp;
+            PGM_ASSERT(slot >= 0 && slot < part_cap);
+            const uint2 x = part[slot];
+            s = min(min(s, x.y), max(b, x.x));
+            b = min(b, x.x);
+        }
+        const int bj = (int)(b & KEY_IDX_MASK), bd = (int)(b >> KEY_IDX_BITS), sd = (int)(s >> KEY_IDX_BITS);
+        PGM_ASSERT(b < KEY_INVALID && bj < pr.n2);
+        // the expression of ratio_crosscheck_kernel (n2 >= 1 here: a pair without train rows is never launched)
+        keep = true;
+        if (keep && ratio > 0.0f && pr.n2 >= 2 && !((float)bd < ratio * (float)sd)) keep = false;
+        if (keep && cross_check) {
+            PGM_ASSERT(pr.col_base + bj < col_cap);
+            if ((int)(colbest[pr.col_base + bj] & KEY_IDX_MASK) != i) keep = false;
+        }
+        if (keep && max_dist >= 0 && bd > max_dist) keep = false;
+        res[pr.row_base + i] = keep ? b : KEY_NONE;
+    }
+    const int n = __syncthreads_count(keep);
+    if (tid == 0) bcnt[g] = n;
+}
+
+// kept triples of one block, in ascending i, at the pair's output offset + the kept rows of the pair's earlier blocks
+__global__ void __launch_bounds__(RCF_THREADS) rcp_scatter_kernel(const RcpPair *__restrict__ pairs,
+                                                                  const int32_t *__restrict__ fblk_base, int n_pairs,
+                                                                  const uint32_t *__restrict__ res,
+                                                                  const int32_t *__restrict__ bcnt, int64_t capacity,
+                                                                  int32_t *__restrict__ out_qi, int32_t *__restrict__ out_tj,
+                                                                  int32_t *__restrict__ out_dist, int32_t *__restrict__ counts) {
+    __shared__ int s_before[RCF_THREADS / 32], s_total[RCF_THREADS / 32], s_w[RCF_THREADS / 32];
+    const int g = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int p = find_pair(fblk_base, n_pairs, g);
+    const RcpPair pr = pairs[p];
+    const int first = __ldg(fblk_base + p), nb = __ldg(fblk_base + p + 1) - first, b = g - first;
+    // kept rows of the pair's blocks before this one, and of all of them (nb <= RCF_THREADS)
+    const int c = tid < nb ? __ldg(bcnt + first + tid) : 0;
+    int before = tid < b ? c : 0, total = c;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        before += __shfl_xor_sync(0xffffffffu, before, o);
+        total += __shfl_xor_sync(0xffffffffu, total, o);
+    }
+    const int i = b * RCF_THREADS + tid;
+    const uint32_t key = i < pr.n1 ? __ldg(res + pr.row_base + i) : KEY_NONE;
+    const bool keep = key != KEY_NONE;
+    const unsigned m = __ballot_sync(0xffffffffu, keep);
+    if (lane == 0) { s_before[wid] = before; s_total[wid] = total; s_w[wid] = __popc(m); }
+    __syncthreads();
+    int off = 0;
+    before = 0; total = 0;
+#pragma unroll 4
+    for (int w = 0; w < RCF_THREADS / 32; w++) {
+        before += s_before[w]; total += s_total[w];
+        if (w < wid) off += s_w[w];
+    }
+    if (keep) {
+        const int64_t o = pr.out_base + before + off + __popc(m & ((1u << lane) - 1u));
+        PGM_ASSERT(o >= pr.out_base && o < pr.out_base + pr.n1 && o < capacity);
+        out_qi[o] = i; out_tj[o] = (int32_t)(key & KEY_IDX_MASK); out_dist[o] = (int32_t)(key >> KEY_IDX_BITS);
+    }
+    if (b == nb - 1 && tid == 0) counts[pr.pair_id] = total;
+}
+
+// ---------------------------------------------------------------------------
 // train-sharded nearest / second-nearest neighbour (SURVEY.md section 8e, "top-2 merge"):
 // every rank searches its slice of the train set, the (best, second) pairs travel as packed keys
 // (distance << 20 | GLOBAL train index, XKEY_NONE where absent -- integer order == the (distance, j)

@@ -1112,7 +1112,7 @@ extern "C" int pgm_match_ratio_crosscheck_batch_dev(pgm_handle *h, const uint8_t
     }
     if (capacity < total) return fail(h, PGM_E_CAPACITY, "capacity < sum of query sizes");
     if (smem > RCB_SMEM_MAX)
-        return fail(h, PGM_E_INVALID_ARG, "a pair is too large for the small-pair batch kernel (use pgm_match_ratio_crosscheck per pair)");
+        return fail(h, PGM_E_INVALID_ARG, "a pair is too large for the small-pair batch kernel (use pgm_match_ratio_crosscheck_pairs_batch_dev)");
     const size_t pb = align_up(sizeof(RcbPair) * n_pairs, 256);
     if ((rc = ensure_dev(h, h->misc, pb + (size_t)n_pairs * 4))) return rc;
     if ((rc = ensure_host(h, h->pin_in, pb + (size_t)n_pairs * 4))) return rc;
@@ -1135,6 +1135,163 @@ extern "C" int pgm_match_ratio_crosscheck_batch_dev(pgm_handle *h, const uint8_t
     h->stats.kernel_launches += 1; h->stats.host_syncs += 2; h->stats.pairs = n_pairs;
     for (int p = 0; p < n_pairs; p++) { h->stats.distance_evals += (int64_t)hp[p].n1 * hp[p].n2; h->stats.matched += out_counts[p]; }
     h->stats.evals_computed = h->stats.distance_evals * (cross_check ? 2 : 1);
+    return PGM_OK;
+}
+
+// ---------------------------------------------------------------------------
+// many pairs of any size: the same result through one fused distance pass per chunk (pgm_kernels.cuh, RcpPair).
+// The host plans every chunk first, uploads the whole plan in one copy and then only enqueues: three kernels per
+// chunk, no read-back until the counts at the end.
+// ---------------------------------------------------------------------------
+template <int WORDS, bool CROSS>
+static int rcp_occupancy() {
+    int nb = 0;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, knn2_cols_pairs_kernel<WORDS, CROSS>, ROUND_THREADS, 0);
+    return std::max(nb, 1);
+}
+template <int WORDS>
+static void launch_rcp_dist(bool cross, int grid, const RcpPair *pairs, const int32_t *tile_base, int n, uint2 *part,
+                            int64_t part_cap, uint32_t *colbest, int64_t col_cap, cudaStream_t s) {
+    if (cross) knn2_cols_pairs_kernel<WORDS, true><<<grid, ROUND_THREADS, 0, s>>>(pairs, tile_base, n, part, part_cap, colbest, col_cap);
+    else knn2_cols_pairs_kernel<WORDS, false><<<grid, ROUND_THREADS, 0, s>>>(pairs, tile_base, n, part, part_cap, colbest, col_cap);
+}
+
+struct RcpChunk {
+    int first, n;              // its pairs: plan[first, first + n)
+    int base_off;              // tile_base at bases[base_off], fblk_base at bases[base_off + n + 1]
+    int32_t items, fblocks;    // distance-kernel CTAs, filter / scatter CTAs
+    int64_t part_slots, cols, rows;
+};
+
+extern "C" int pgm_match_ratio_crosscheck_pairs_batch_dev(pgm_handle *h, const uint8_t *d_all_desc, const int64_t *image_offsets,
+                                                          int32_t n_images, const int32_t *pair_list, int32_t n_pairs,
+                                                          int32_t desc_bits, int32_t stride_bytes, float ratio, int32_t cross_check,
+                                                          int32_t max_dist, int32_t *d_out_qi, int32_t *d_out_tj,
+                                                          int32_t *d_out_dist, int64_t capacity, int32_t *out_counts) {
+    if (!h || !out_counts || n_pairs < 0 || n_images < 0 || (n_pairs > 0 && (!image_offsets || !pair_list))) return PGM_E_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    int rc = check_format(h, desc_bits, stride_bytes);
+    if (rc) return rc;
+    h->stats = pgm_stats{};
+    h->stats_pending = false;
+    if (n_pairs == 0) return PGM_OK;
+    if (!d_all_desc || !d_out_qi || !d_out_tj || !d_out_dist) return fail(h, PGM_E_INVALID_ARG, "null pointer");
+    int64_t total = 0, evals = 0;
+    for (int p = 0; p < n_pairs; p++) {
+        const int a = pair_list[2 * p], b = pair_list[2 * p + 1];
+        if (a < 0 || a >= n_images || b < 0 || b >= n_images) return fail(h, PGM_E_INVALID_ARG, "pair index out of range");
+        const int64_t n1 = image_offsets[a + 1] - image_offsets[a], n2 = image_offsets[b + 1] - image_offsets[b];
+        if (n1 < 0 || n2 < 0 || n1 >= MAX_N || n2 >= MAX_N) return fail(h, PGM_E_INVALID_ARG, "bad image sizes");
+        total += n1;
+        evals += n1 * n2;
+    }
+    if (capacity < total) return fail(h, PGM_E_CAPACITY, "capacity < sum of query sizes");
+    CU_CHECK(h, cudaSetDevice(h->device));
+    cudaStream_t s = h->stream;
+    const int words = stride_bytes / 4;
+    const bool cross = cross_check != 0;
+    int ctas_per_sm;
+    switch (words) {
+        case 4: ctas_per_sm = cross ? rcp_occupancy<4, true>() : rcp_occupancy<4, false>(); break;
+        case 8: ctas_per_sm = cross ? rcp_occupancy<8, true>() : rcp_occupancy<8, false>(); break;
+        case 12: ctas_per_sm = cross ? rcp_occupancy<12, true>() : rcp_occupancy<12, false>(); break;
+        default: ctas_per_sm = cross ? rcp_occupancy<16, true>() : rcp_occupancy<16, false>(); break;
+    }
+    // few row tiles (one big pair): split the columns until the distance kernel has about two waves of CTAs
+    const int64_t target_items = 2ll * h->num_sms * ctas_per_sm;
+    constexpr int tile_rows = ROUND_THREADS * RQ_LARGE;
+
+    // plan: chunks of <= MAX_CHUNK_PAIRS pairs and <= MAX_CHUNK_SLOTS rows + columns (as batch_impl); a pair without
+    // query or train rows keeps no triple and is not launched
+    std::vector<RcpPair> plan;
+    std::vector<int32_t> bases;
+    std::vector<RcpChunk> chunks;
+    int64_t out_base = 0, max_part = 0, max_cols = 0, max_rows = 0, max_fblocks = 0;
+    for (int p = 0; p < n_pairs;) {
+        RcpChunk c{(int)plan.size(), 0, (int)bases.size(), 0, 0, 0, 0, 0};
+        int64_t row_tiles = 0;
+        for (; p < n_pairs && c.n < MAX_CHUNK_PAIRS; p++) {
+            const int a = pair_list[2 * p], b = pair_list[2 * p + 1];
+            const int32_t n1 = (int32_t)(image_offsets[a + 1] - image_offsets[a]), n2 = (int32_t)(image_offsets[b + 1] - image_offsets[b]);
+            if (n1 > 0 && n2 > 0) {
+                if (c.n > 0 && c.rows + c.cols + n1 + n2 > MAX_CHUNK_SLOTS) break;
+                RcpPair r{};
+                r.q = (const uint32_t *)(d_all_desc + (size_t)image_offsets[a] * stride_bytes);
+                r.t = (const uint32_t *)(d_all_desc + (size_t)image_offsets[b] * stride_bytes);
+                r.n1 = n1; r.n2 = n2; r.out_base = out_base; r.col_base = c.cols; r.row_base = c.rows; r.pair_id = p;
+                plan.push_back(r);
+                c.n++; c.cols += n2; c.rows += n1;
+                row_tiles += (n1 + tile_rows - 1) / tile_rows;
+            }
+            out_base += n1;
+        }
+        if (c.n == 0) continue;
+        const int64_t want = row_tiles >= target_items ? 1 : (target_items + row_tiles - 1) / row_tiles;
+        bases.resize(bases.size() + 2 * (size_t)(c.n + 1));
+        int32_t *tb = bases.data() + c.base_off, *fb = tb + c.n + 1;
+        for (int k = 0; k < c.n; k++) {
+            RcpPair &r = plan[c.first + k];
+            const int64_t col_stages = (r.n2 + STAGE_LARGE - 1) / STAGE_LARGE;
+            const int64_t splits = std::min(want, col_stages);
+            r.cols_per_split = (int32_t)((col_stages + splits - 1) / splits * STAGE_LARGE);
+            r.splits = (r.n2 + r.cols_per_split - 1) / r.cols_per_split;
+            r.part_base = c.part_slots;
+            c.part_slots += (int64_t)r.n1 * r.splits;
+            tb[k] = c.items; fb[k] = c.fblocks;
+            c.items += (r.n1 + tile_rows - 1) / tile_rows * r.splits;
+            c.fblocks += (r.n1 + RCF_THREADS - 1) / RCF_THREADS;
+        }
+        tb[c.n] = c.items; fb[c.n] = c.fblocks;
+        max_part = std::max(max_part, c.part_slots); max_cols = std::max(max_cols, c.cols);
+        max_rows = std::max(max_rows, c.rows); max_fblocks = std::max<int64_t>(max_fblocks, c.fblocks);
+        chunks.push_back(c);
+    }
+
+    // h->misc: plan | bases | counts | partials | column minima | per-row results | block counts (reused by every chunk)
+    const size_t o_bases = align_up(sizeof(RcpPair) * std::max<size_t>(plan.size(), 1), 256);
+    const size_t o_counts = o_bases + align_up(4 * std::max<size_t>(bases.size(), 1), 256);
+    const size_t o_part = o_counts + align_up(4 * (size_t)n_pairs, 256);
+    const size_t o_col = o_part + align_up(8 * (size_t)std::max<int64_t>(max_part, 1), 256);
+    const size_t o_res = o_col + align_up(4 * (size_t)std::max<int64_t>(max_cols, 1), 256);
+    const size_t o_bcnt = o_res + align_up(4 * (size_t)std::max<int64_t>(max_rows, 1), 256);
+    const size_t o_end = o_bcnt + align_up(4 * (size_t)std::max<int64_t>(max_fblocks, 1), 256);
+    if ((rc = ensure_dev(h, h->misc, o_end))) return rc;
+    if ((rc = ensure_host(h, h->pin_in, o_part))) return rc;
+    CU_CHECK(h, cudaStreamSynchronize(s));                 // the staging buffer may still feed an earlier call's copy
+    char *pin = (char *)h->pin_in.p, *dev = (char *)h->misc.p;
+    memcpy(pin, plan.data(), sizeof(RcpPair) * plan.size());
+    memcpy(pin + o_bases, bases.data(), 4 * bases.size());
+    CU_CHECK(h, cudaMemcpyAsync(dev, pin, o_counts, cudaMemcpyHostToDevice, s));
+    CU_CHECK(h, cudaMemsetAsync(dev + o_counts, 0, 4 * (size_t)n_pairs, s));
+    const RcpPair *d_plan = (const RcpPair *)dev;
+    const int32_t *d_bases = (const int32_t *)(dev + o_bases);
+    int32_t *d_counts = (int32_t *)(dev + o_counts), *d_bcnt = (int32_t *)(dev + o_bcnt);
+    uint2 *d_part = (uint2 *)(dev + o_part);
+    uint32_t *d_col = (uint32_t *)(dev + o_col), *d_res = (uint32_t *)(dev + o_res);
+    for (const RcpChunk &c : chunks) {
+        const RcpPair *cp = d_plan + c.first;
+        const int32_t *tb = d_bases + c.base_off, *fb = tb + c.n + 1;
+        if (cross) CU_CHECK(h, cudaMemsetAsync(d_col, 0xFF, 4 * (size_t)c.cols, s));     // KEY_NONE
+        switch (words) {
+            case 4: launch_rcp_dist<4>(cross, c.items, cp, tb, c.n, d_part, c.part_slots, d_col, c.cols, s); break;
+            case 8: launch_rcp_dist<8>(cross, c.items, cp, tb, c.n, d_part, c.part_slots, d_col, c.cols, s); break;
+            case 12: launch_rcp_dist<12>(cross, c.items, cp, tb, c.n, d_part, c.part_slots, d_col, c.cols, s); break;
+            default: launch_rcp_dist<16>(cross, c.items, cp, tb, c.n, d_part, c.part_slots, d_col, c.cols, s); break;
+        }
+        rcp_filter_kernel<<<c.fblocks, RCF_THREADS, 0, s>>>(cp, fb, c.n, d_part, c.part_slots, d_col, c.cols, ratio,
+                                                            cross ? 1 : 0, max_dist, d_res, d_bcnt);
+        rcp_scatter_kernel<<<c.fblocks, RCF_THREADS, 0, s>>>(cp, fb, c.n, d_res, d_bcnt, capacity, d_out_qi, d_out_tj,
+                                                             d_out_dist, d_counts);
+        CU_CHECK(h, cudaGetLastError());
+        h->stats.kernel_launches += 3;
+    }
+    CU_CHECK(h, cudaMemcpyAsync(pin + o_counts, d_counts, 4 * (size_t)n_pairs, cudaMemcpyDeviceToHost, s));
+    CU_CHECK(h, cudaStreamSynchronize(s));
+    memcpy(out_counts, pin + o_counts, 4 * (size_t)n_pairs);
+    h->stats.host_syncs += 2; h->stats.pairs = n_pairs;
+    h->stats.distance_evals = evals;
+    h->stats.evals_computed = evals;                       // one fused pass, cross-check or not
+    for (int p = 0; p < n_pairs; p++) h->stats.matched += out_counts[p];
     return PGM_OK;
 }
 

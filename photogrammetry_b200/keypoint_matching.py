@@ -284,6 +284,18 @@ class Matcher:
         """Nearest neighbour + ratio test + cross-check for many small pairs in ONE launch (a frame sequence).
         ``d_all_desc``: torch uint8 ``[sum, stride]`` on the GPU.  Returns ``(out int32[3, sum of n1], starts int64[n_pairs],
         counts int32[n_pairs])``; pair ``p`` owns ``out[:, starts[p]:starts[p] + counts[p]]`` (ascending query index)."""
+        return self._ratio_batch_dev(self._lib.pgm_match_ratio_crosscheck_batch_dev, d_all_desc, image_offsets, pair_list,
+                                     desc_bits, ratio, cross_check, max_dist)
+
+    def match_ratio_crosscheck_pairs_batch_dev(self, d_all_desc, image_offsets, pair_list, desc_bits: int = 256,
+                                               ratio: float = 0.8, cross_check: bool = True, max_dist: int = -1):
+        """:meth:`match_ratio_crosscheck_batch_dev` for pairs of any size (e.g. all pairs of a large image set): one
+        fused distance pass per chunk of pairs instead of one CTA per pair.  Same arguments, same return value; per pair
+        the same triples as :meth:`match_ratio_crosscheck`."""
+        return self._ratio_batch_dev(self._lib.pgm_match_ratio_crosscheck_pairs_batch_dev, d_all_desc, image_offsets,
+                                     pair_list, desc_bits, ratio, cross_check, max_dist)
+
+    def _ratio_batch_dev(self, fn, d_all_desc, image_offsets, pair_list, desc_bits, ratio, cross_check, max_dist):
         import torch
         offs = np.ascontiguousarray(image_offsets, dtype=np.int64)
         pairs = np.ascontiguousarray(pair_list, dtype=np.int32).reshape(-1, 2)
@@ -294,7 +306,7 @@ class Matcher:
         out = torch.empty((3, max(total, 1)), dtype=torch.int32, device=d_all_desc.device)
         counts = np.zeros(max(len(pairs), 1), dtype=np.int32)
         with self.torch_ordered(d_all_desc.device):
-            self._check(self._lib.pgm_match_ratio_crosscheck_batch_dev(
+            self._check(fn(
                 self._h, d_all_desc.data_ptr(), offs.ctypes.data, len(offs) - 1, pairs.ctypes.data, len(pairs), int(desc_bits),
                 int(d_all_desc.shape[1]), float(ratio), int(bool(cross_check)), int(max_dist), out[0].data_ptr(),
                 out[1].data_ptr(), out[2].data_ptr(), total, counts.ctypes.data))

@@ -8,6 +8,8 @@
   3. 24 pairs of 512 x 512: throughput mode (standalone round / accept+filter / sparse / finisher / order kernels)
   4. float L2 512 x 512, D = 128: the tcgen05 CTA-pair kernel with its cluster mbarriers
   5. 3 emulated train shards of a 700 x 650 pair (export / propose / stable commit kernels)
+  6. ratio test + cross-check of 7 pairs of any size, empty and split ones included (fused distance pass with
+     column splits, split-partial merge, block-parallel ordered compaction)
 Every result is checked against the oracle, so a sanitizer run is also a parity run."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -43,5 +45,17 @@ outs, rounds = sharding.match_train_sharded_emulated(m, q, t, 3)
 exp = orc.match_sweep(q, t)
 assert all((o == exp).all() for o in outs)
 print("case 5 ok", rounds)
+sizes = [0, 1, 700, 2600, 900]
+base = synthetic.uniform_descriptors(7, max(sizes), 256)
+imgs = [base[:n] if k % 2 == 0 else synthetic.noisy_copy_descriptors(8 + k, base, 256)[:n] for k, n in enumerate(sizes)]
+offs = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+pairs = [(2, 3), (3, 2), (3, 4), (4, 4), (1, 3), (3, 1), (0, 2), (2, 0)]
+d_all = torch.from_numpy(np.concatenate(imgs)).cuda()
+for ratio, cc, md in [(0.8, True, -1), (0.0, False, 60)]:
+    out, starts, counts = m.match_ratio_crosscheck_pairs_batch_dev(d_all, offs, pairs, 256, ratio, cc, md)
+    out = out.cpu().numpy()
+    for p, (a, b) in enumerate(pairs):
+        assert (out[:, starts[p]:starts[p] + counts[p]].T == orc.match_ratio_crosscheck(imgs[a], imgs[b], ratio, cc, md)).all()
+print("case 6 ok", m.stats())
 m.close()
 print("ALL OK")
