@@ -242,8 +242,46 @@ int pgm_knn2_l2_dev(pgm_handle *h, const float *d_q, int32_t n1, const float *d_
                     int32_t *d_best_j, float *d_best_d, int32_t *d_second_j, float *d_second_d,
                     float *d_debug_dist);
 /* Rows of the handle's last float call that took the exhaustive fallback (synchronises the stream);
- * -1 if that call did not run in the fp16 ranking mode. */
+ * -1 if that call did not run in the fp16 ranking mode.  After a batch call below: the call's
+ * total over all chunks and, with cross-check, both directions. */
 int pgm_l2_last_fallback_rows(pgm_handle *h);
+
+/* ---- float descriptors, many image pairs per call ---------------------------------------
+ * Layout as pgm_match_ratio_crosscheck_pairs_batch_dev: d_all_desc is device float[rows][dim],
+ * 1 <= dim <= 128; image_offsets[n_images + 1] and pair_list[n_pairs][2] (query image, train
+ * image) are host arrays; pair p's rows start at the sum of the query-image sizes n1 of the pairs
+ * before it.  0 <= n1, n2 < 2^20 per pair.  PGM_E_INVALID_ARG: bad dim, pair index, image size or
+ * null pointer; PGM_E_CAPACITY: capacity < sum of n1.
+ *
+ * pgm_knn2_l2_pairs_batch_dev: per pair the contract of pgm_knn2_l2_dev (squared L2, best and
+ * second best under (distance, train index), index -1 and distance -1.0 where absent); a pair
+ * with n1 = 0 writes nothing.  Every pair, n1 <= 128 included, ranks on the CTA-pair fp16 path
+ * (certified band + exhaustive fallback), so a pair with n1 > 128 gets bit-identically the
+ * pgm_knn2_l2_dev result.  The fp16 operands use one power-of-two scale per chunk of pairs, from
+ * max |x| over the images the chunk references: results do not depend on it, but an image far
+ * smaller in magnitude than the chunk's largest goes subnormal in fp16 and its rows take the
+ * exhaustive fallback -- correct, slower.
+ *
+ * pgm_match_l2_ratio_crosscheck_pairs_batch_dev: keeps (i, j1, d1) of a pair iff
+ *   n2 < 2 || ratio <= 0 || d1 < (ratio * ratio) * d2   (fp32, ratio * ratio rounded to fp32 first:
+ *                                                        Lowe's ratio on Euclidean distances),
+ *   !cross_check || the best query of train row j1 under (distance, query index) is i,
+ *   max_sq_dist < 0 || d1 <= max_sq_dist,
+ * on the squared distances knn2 reports.  Output in ascending i at the pair's rows; out_counts[p]
+ * = kept triples, no slot beyond a pair's count is written.  Every exact distance is a per-lane
+ * sum of fmaf((q - t), (q - t), .) and a butterfly, bit-symmetric in q and t, so the column best
+ * of pair (a, b) is the row best of (b, a): with cross_check the library runs the top-2 pass of
+ * the reversed pairs too, in the same chunk -- twice the GEMM work (pgm_stats.evals_computed =
+ * 2 distance_evals). */
+int pgm_knn2_l2_pairs_batch_dev(pgm_handle *h, const float *d_all_desc, const int64_t *image_offsets, int32_t n_images,
+                                const int32_t *pair_list, int32_t n_pairs, int32_t dim,
+                                int32_t *d_best_j, float *d_best_d, int32_t *d_second_j, float *d_second_d,
+                                int64_t capacity);
+int pgm_match_l2_ratio_crosscheck_pairs_batch_dev(pgm_handle *h, const float *d_all_desc, const int64_t *image_offsets,
+                                int32_t n_images, const int32_t *pair_list, int32_t n_pairs, int32_t dim,
+                                float ratio, int32_t cross_check, float max_sq_dist,
+                                int32_t *d_out_qi, int32_t *d_out_tj, float *d_out_dist,
+                                int64_t capacity, int32_t *out_counts);
 
 /* ---- the producer of the matcher's inputs (SURVEY.md section 8, rows f1/f2) ----------
  * gray: float[height][width] = Grayscale.K (Images.Abstractions/Pixels/Grayscale.cs:19-23),

@@ -37,6 +37,7 @@ EXPORTED_SYMBOLS = (
     "pgm_knn2_hamming", "pgm_knn2_hamming_dev", "pgm_match_ratio_crosscheck", "pgm_match_ratio_crosscheck_batch_dev",
     "pgm_match_ratio_crosscheck_pairs_batch_dev", "pgm_pack_top2_keys_dev", "pgm_merge_top2_dev", "pgm_ratio_crosscheck_filter_dev",
     "pgm_match_keypoints_sorted", "pgm_match_keypoints_sorted_dev", "pgm_knn2_l2", "pgm_knn2_l2_dev", "pgm_l2_last_fallback_rows",
+    "pgm_knn2_l2_pairs_batch_dev", "pgm_match_l2_ratio_crosscheck_pairs_batch_dev",
     "pgm_fast_detect", "pgm_brief_describe", "pgm_nms", "pgm_detect_describe_dev", "pgm_detect_describe_batch_dev",
     "pgm_ransac_score",
     "pgm_shard_create", "pgm_shard_edge_capacity", "pgm_shard_round", "pgm_shard_commit", "pgm_shard_finish_round",
@@ -136,6 +137,11 @@ def load() -> C.CDLL:
         lib.pgm_knn2_l2.argtypes = [C.c_void_p, vp, C.c_int32, vp, C.c_int32, C.c_int32, i32p, vp, i32p, vp]
         lib.pgm_knn2_l2_dev.argtypes = [C.c_void_p, vp, C.c_int32, vp, C.c_int32, C.c_int32, i32p, vp, i32p, vp, vp]
         lib.pgm_l2_last_fallback_rows.argtypes = [C.c_void_p]
+        lib.pgm_knn2_l2_pairs_batch_dev.argtypes = [C.c_void_p, vp, i64p, C.c_int32, i32p, C.c_int32, C.c_int32, i32p, vp, i32p,
+                                                    vp, C.c_int64]
+        lib.pgm_match_l2_ratio_crosscheck_pairs_batch_dev.argtypes = [C.c_void_p, vp, i64p, C.c_int32, i32p, C.c_int32,
+                                                                      C.c_int32, C.c_float, C.c_int32, C.c_float, i32p, i32p,
+                                                                      vp, C.c_int64, i32p]
         lib.pgm_match_ratio_crosscheck.argtypes = [C.c_void_p, u8p, C.c_int32, u8p, C.c_int32, C.c_int32, C.c_int32,
                                                    C.c_float, C.c_int32, C.c_int32, i32p, i32p, i32p, C.c_int32,
                                                    C.POINTER(C.c_int32)]

@@ -214,27 +214,22 @@ __device__ __forceinline__ void l2_scale_from_bits(unsigned bits, float &s, floa
 // hdr[0] = max |x| bits, one atomicMax per block.  hdr lives in a buffer of its own that is zeroed when allocated; every
 // call leaves hdr[0] = 0 behind (l2_exact_rows_kernel, the last kernel of the chain) and its ticket hdr[2] self-cleans, so no
 // memset sits in front of the chain.
-__global__ void __launch_bounds__(256) absmax_kernel(const float *__restrict__ q, size_t nq, const float *__restrict__ t, size_t nt,
-                                                     unsigned *__restrict__ hdr) {
-    pdl_trigger();
-    if (blockIdx.x == 0 && threadIdx.x == 0) hdr[1] = 0;      // flagged-row count of this call (the refinement fills it)
-    unsigned m = 0;
-    const size_t stride = (size_t)gridDim.x * blockDim.x, tid = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    for (int side = 0; side < 2; side++) {
-        const float *x = side ? t : q;
-        const size_t n = side ? nt : nq;
-        if ((reinterpret_cast<uintptr_t>(x) & 15) == 0) {
-            const size_t n4 = n >> 2;
-            const uint4 *x4 = reinterpret_cast<const uint4 *>(x);
-            for (size_t i = tid; i < n4; i += stride) {
-                const uint4 v = __ldg(x4 + i);
-                m = max(max(m, v.x & 0x7FFFFFFFu), max(max(v.y & 0x7FFFFFFFu, v.z & 0x7FFFFFFFu), v.w & 0x7FFFFFFFu));
-            }
-            for (size_t i = (n4 << 2) + tid; i < n; i += stride) m = max(m, __float_as_uint(__ldg(x + i)) & 0x7FFFFFFFu);
-        } else {
-            for (size_t i = tid; i < n; i += stride) m = max(m, __float_as_uint(__ldg(x + i)) & 0x7FFFFFFFu);
+__device__ __forceinline__ unsigned absmax_span(const float *__restrict__ x, size_t n, size_t tid, size_t stride, unsigned m) {
+    if ((reinterpret_cast<uintptr_t>(x) & 15) == 0) {
+        const size_t n4 = n >> 2;
+        const uint4 *x4 = reinterpret_cast<const uint4 *>(x);
+        for (size_t i = tid; i < n4; i += stride) {
+            const uint4 v = __ldg(x4 + i);
+            m = max(max(m, v.x & 0x7FFFFFFFu), max(max(v.y & 0x7FFFFFFFu, v.z & 0x7FFFFFFFu), v.w & 0x7FFFFFFFu));
         }
+        for (size_t i = (n4 << 2) + tid; i < n; i += stride) m = max(m, __float_as_uint(__ldg(x + i)) & 0x7FFFFFFFu);
+    } else {
+        for (size_t i = tid; i < n; i += stride) m = max(m, __float_as_uint(__ldg(x + i)) & 0x7FFFFFFFu);
     }
+    return m;
+}
+// block maximum, one atomicMax into hdr[0] (blockDim.x <= 256)
+__device__ __forceinline__ void absmax_commit(unsigned m, unsigned *__restrict__ hdr) {
     m = __reduce_max_sync(0xffffffffu, m);
     __shared__ unsigned sm[8];
     if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = m;
@@ -243,6 +238,58 @@ __global__ void __launch_bounds__(256) absmax_kernel(const float *__restrict__ q
         for (int w = 1; w < (int)(blockDim.x >> 5); w++) m = max(m, sm[w]);
         if (m) atomicMax(hdr, m);
     }
+}
+__global__ void __launch_bounds__(256) absmax_kernel(const float *__restrict__ q, size_t nq, const float *__restrict__ t, size_t nt,
+                                                     unsigned *__restrict__ hdr) {
+    pdl_trigger();
+    if (blockIdx.x == 0 && threadIdx.x == 0) hdr[1] = 0;      // flagged-row count of this call (the refinement fills it)
+    const size_t stride = (size_t)gridDim.x * blockDim.x, tid = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    absmax_commit(absmax_span(t, nt, tid, stride, absmax_span(q, nq, tid, stride, 0u)), hdr);
+}
+
+// One fp16 operand row: lane l holds components 4l .. 4l + 3 (Dp <= 128).  split16_load reads them (before the scale is
+// known), split16_store writes [x16 (Dp) | norm chunk (64)] and returns the scaled |x|^2.
+__device__ __forceinline__ void split16_load(const float *__restrict__ x, int dim, int dp, int lane, float (&v)[4]) {
+    const bool vec = (dim & 3) == 0 && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
+    v[0] = v[1] = v[2] = v[3] = 0.f;
+    const int k = 4 * lane;
+    if (k < dp) {
+        if (vec && k + 3 < dim) {
+            const float4 f = __ldg(reinterpret_cast<const float4 *>(x + k));
+            v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w;
+        } else {
+#pragma unroll
+            for (int e = 0; e < 4; e++) v[e] = k + e < dim ? __ldg(x + k + e) : 0.f;
+        }
+    }
+}
+__device__ __forceinline__ float split16_store(float (&v)[4], float s, int dp, int lane, bool train, __half *__restrict__ o) {
+    const int k = 4 * lane;
+    float acc = 0.f;
+    if (k < dp) {
+        __half2 h[2];
+#pragma unroll
+        for (int e = 0; e < 4; e++) v[e] *= s;
+        h[0] = __floats2half2_rn(v[0], v[1]);
+        h[1] = __floats2half2_rn(v[2], v[3]);
+        *reinterpret_cast<uint2 *>(o + k) = make_uint2(*reinterpret_cast<uint32_t *>(&h[0]), *reinterpret_cast<uint32_t *>(&h[1]));
+#pragma unroll
+        for (int e = 0; e < 4; e++) acc = fmaf(v[e], v[e], acc);
+    }
+    for (int sh = 16; sh; sh >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, sh);
+    const float hn = -0.5f * acc * (1.f / NORM_C);
+    const __half e0 = __float2half_rn(hn);
+    const float r1 = hn - __half2float(e0);
+    const __half e1 = __float2half_rn(r1);
+    const __half e2 = __float2half_rn(r1 - __half2float(e1));
+    const __half cc = __float2half_rn(NORM_C), zero = __float2half_rn(0.f);
+    const __half n0 = train ? cc : e0, n1v = train ? cc : e1, n2v = train ? cc : e2;
+    const __half n3 = train ? e0 : cc, n4 = train ? e1 : cc, n5 = train ? e2 : cc;
+    __half2 ext;
+    ext.x = lane == 0 ? n0 : lane == 1 ? n2v : lane == 2 ? n4 : zero;
+    ext.y = lane == 0 ? n1v : lane == 1 ? n3 : lane == 2 ? n5 : zero;
+    *reinterpret_cast<__half2 *>(o + dp + 2 * lane) = ext;
+    return acc;
 }
 
 // Row layout in fp16 mode: [x16 (Dp) | norm chunk (64)].  One warp per row, as split_kernel.
@@ -263,49 +310,17 @@ __global__ void __launch_bounds__(256) split16_kernel(const float *__restrict__ 
     }
     const float *x = (train ? t : q) + (size_t)row * dim;
     __half *o = (train ? b : a) + (size_t)row * (dp + CHUNK_K);
-    const bool vec = (dim & 3) == 0 && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
-    float v[4] = {0.f, 0.f, 0.f, 0.f};
-    const int k = 4 * lane;                          // Dp <= 128: one group of four components per lane
-    if (k < dp) {
-        if (vec && k + 3 < dim) {
-            const float4 f = __ldg(reinterpret_cast<const float4 *>(x + k));
-            v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w;
-        } else {
-#pragma unroll
-            for (int e = 0; e < 4; e++) v[e] = k + e < dim ? __ldg(x + k + e) : 0.f;
-        }
-    }
+    float v[4];
+    split16_load(x, dim, dp, lane, v);
     pdl_wait();                                      // the scale comes from absmax_kernel
     float s, inv_s2, mprime;
     l2_scale_from_bits(__ldcg(hdr), s, inv_s2, mprime);
-    float acc = 0.f;
-    if (k < dp) {
-        __half2 h[2];
-#pragma unroll
-        for (int e = 0; e < 4; e++) v[e] *= s;
-        h[0] = __floats2half2_rn(v[0], v[1]);
-        h[1] = __floats2half2_rn(v[2], v[3]);
-        *reinterpret_cast<uint2 *>(o + k) = make_uint2(*reinterpret_cast<uint32_t *>(&h[0]), *reinterpret_cast<uint32_t *>(&h[1]));
-#pragma unroll
-        for (int e = 0; e < 4; e++) acc = fmaf(v[e], v[e], acc);
-    }
-    for (int sh = 16; sh; sh >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, sh);
+    const float acc = split16_store(v, s, dp, lane, train, o);
     if (!train && lane == 0) qnorm[row] = acc;       // scaled, like the accumulator
-    const float hn = -0.5f * acc * (1.f / NORM_C);
-    const __half e0 = __float2half_rn(hn);
-    const float r1 = hn - __half2float(e0);
-    const __half e1 = __float2half_rn(r1);
-    const __half e2 = __float2half_rn(r1 - __half2float(e1));
-    const __half cc = __float2half_rn(NORM_C), zero = __float2half_rn(0.f);
-    const __half n0 = train ? cc : e0, n1v = train ? cc : e1, n2v = train ? cc : e2;
-    const __half n3 = train ? e0 : cc, n4 = train ? e1 : cc, n5 = train ? e2 : cc;
-    __half2 ext;
-    ext.x = lane == 0 ? n0 : lane == 1 ? n2v : lane == 2 ? n4 : zero;
-    ext.y = lane == 0 ? n1v : lane == 1 ? n3 : lane == 2 ? n5 : zero;
-    *reinterpret_cast<__half2 *>(o + dp + 2 * lane) = ext;
 }
 
 // ---- the GEMM + top-8 kernel ----------------------------------------------------------------
+struct L2BPair;
 struct L2Params {
     int n1, n2, dpc;               // dpc = Dp / 64: chunks per operand part (hi or lo)
     int tiles_per_split;           // single-CTA kernel: column tiles handled by one blockIdx.y
@@ -319,7 +334,37 @@ struct L2Params {
     float *cand_d;                 // [splits][n1][CAND] approximate distances (diagnostic)
     float *dbg_dist;               // optional [n1][n2] approximate distance matrix (tests)
     unsigned long long *timeline;  // optional (PGM_L2_TIMELINE=1): %globaltimer stamps of cluster 0's leader CTA
+    // many pairs (l2_topk_pair_kernel<DBG, true>): the items of pair k are [item_base[k], item_base[k + 1]), the
+    // candidate lists have `rows` (the chunk's query rows) rows per slot
+    const L2BPair *bpairs;
+    const int32_t *item_base;
+    int n_pairs, rows;
 };
+// One pair of a batched chunk (pgm_knn2_l2_pairs_batch_dev).  Pairs without query rows are not in the plan.
+struct L2BPair {
+    int64_t q_row, t_row;          // first row of the query / train image in the caller's descriptor array
+    int64_t out_row;               // first result row: the caller's output arrays (knn2) or the chunk's knn2 scratch
+    int32_t a_row, b_row;          // first row of the query / train image in the chunk's A' / B' operands
+    int32_t n1, n2;
+    int32_t row0;                  // first query row of the chunk: candidate lists, flagged-row ids
+    int32_t item0, col_tiles;      // first GEMM item; column tiles (0 when n2 = 0: such a pair has no GEMM item)
+    int32_t pad;
+};
+// One image of a chunk converted into fp16 operand rows: once per role (query form into A', train form into B').
+struct L2BImage {
+    int64_t src_row;               // first row in the caller's descriptor array
+    int32_t dst_row, n;            // first operand row, rows
+    int32_t train, pad;
+};
+// Largest k with base[k] <= g (base is an exclusive prefix over n entries, base[n] = total).
+__device__ __forceinline__ int l2_find(const int32_t *__restrict__ base, int n, int g) {
+    int lo = 0, hi = n;
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (__ldg(base + mid) <= g) lo = mid; else hi = mid;
+    }
+    return lo;
+}
 __device__ __forceinline__ void l2_stamp(const L2Params &p, int slot) {
     if (p.timeline && blockIdx.x == 0 && blockIdx.y == 0) {
         unsigned long long t;
@@ -647,7 +692,38 @@ __device__ __forceinline__ int l2_segment_of_item(int x, int items, int clusters
     return (int)((((long long)x + 1) * clusters - 1) / items);
 }
 
-template <bool DBG>
+// One work item decoded: its row pair (identified by the item that starts it), column tile and pair.  With BATCH the
+// items of the chunk's pairs are concatenated (pair-major, then row pair, then column tile); the cursor `pp` only moves
+// forward, as the roles walk their segment in order.
+struct L2Item {
+    int first, ct, col_tiles;      // first item of the row pair, column tile, column tiles of the pair
+    int m0;                        // the row pair's first query row (pair-local)
+    int n1, n2, a_row, b_row, row0;
+};
+template <bool BATCH>
+__device__ __forceinline__ void l2_item(const L2Params &p, int it, int &pp, L2Item &x) {
+    if constexpr (BATCH) {
+        while (it >= __ldg(p.item_base + pp + 1)) pp++;
+        PGM_ASSERT(pp >= 0 && pp < p.n_pairs);
+        const L2BPair *b = p.bpairs + pp;
+        const int i0 = __ldg(&b->item0), ct_n = __ldg(&b->col_tiles);
+        PGM_ASSERT(ct_n > 0 && it >= i0);
+        const int rp = (it - i0) / ct_n;
+        x.ct = it - i0 - rp * ct_n; x.first = i0 + rp * ct_n; x.col_tiles = ct_n; x.m0 = 2 * rp * TILE_M;
+        x.n1 = __ldg(&b->n1); x.n2 = __ldg(&b->n2); x.a_row = __ldg(&b->a_row); x.b_row = __ldg(&b->b_row);
+        x.row0 = __ldg(&b->row0);
+    } else {
+        const int rp = it / p.col_tiles;
+        x.ct = it - rp * p.col_tiles; x.first = rp * p.col_tiles; x.col_tiles = p.col_tiles; x.m0 = 2 * rp * TILE_M;
+        x.n1 = p.n1; x.n2 = p.n2; x.a_row = 0; x.b_row = 0; x.row0 = 0;
+    }
+}
+
+// BATCH: many pairs in one launch (pgm_knn2_l2_pairs_batch_dev).  A' / B' hold every image of the chunk once; a tile's
+// TMA rows are the pair's first operand row plus the tile offset, so rows past the end of an image are the NEXT image's
+// rows, not zeros: query rows >= n1 do not exist (never trigger, never flushed) and columns >= n2 are masked by
+// epilogue_reduce.  Candidate lists are indexed by the chunk's query row (row0 + local row), `rows` of them per slot.
+template <bool DBG, bool BATCH>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, L2Params p) {
     extern __shared__ unsigned char smem_raw[];
@@ -664,8 +740,10 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
     const uint32_t rank = cluster_ctarank();
     const bool leader = rank == 0;
     const int clusters = (int)(gridDim.x >> 1), cid = (int)(blockIdx.x >> 1);
-    const int CT = p.col_tiles, items = p.items;
+    const int items = p.items;
     const int it0 = l2_segment_start(cid, items, clusters), it1 = l2_segment_start(cid + 1, items, clusters);
+    const int cand_rows = BATCH ? p.rows : p.n1;
+    int pp = BATCH && it0 < it1 ? l2_find(p.item_base, p.n_pairs, it0) : 0;     // pair cursor of this thread's role
     if (threadIdx.x == 0) l2_stamp(p, 0);
 
     if (warp == 1 && lane == 0) {
@@ -694,28 +772,28 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         int s = 0; uint32_t ph = 0;
         int cur_rp = -1; uint32_t n_a = 0;
         for (int it = it0; it < it1; it++) {
-            const int rp = it / CT, ct = it - rp * CT;
-            if (rp != cur_rp && cur_rp < 0) {                  // first rows of the segment: A' first
+            L2Item x;
+            l2_item<BATCH>(p, it, pp, x);
+            const int m0 = x.a_row + x.m0 + (int)rank * TILE_M;
+            if (x.first != cur_rp && cur_rp < 0) {             // first rows of the segment: A' first
                 if (leader) mbar_expect_tx(a_bar, 2u * (uint32_t)nch * CHUNK_BYTES);
-                const int m0 = (2 * rp + (int)rank) * TILE_M;
                 for (int kc = 0; kc < nch; kc++) tma_load_2d_pair(sa + (size_t)kc * CHUNK_BYTES, &map_a, a_bar, kc * CHUNK_K, m0);
-                cur_rp = rp; n_a++;
+                cur_rp = x.first; n_a++;
             }
             for (int kc = 0; kc < nch; kc++) {                 // t16 chunks, norm chunk
                 mbar_wait(&empty[s], ph ^ 1);                  // the pair's MMAs no longer read this stage (multicast commit)
                 if (leader) mbar_expect_tx(&full[s], 2u * B_CHUNK_BYTES2);
                 tma_load_2d_pair(sb + (size_t)s * B_CHUNK_BYTES2, &map_b, &full[s], kc * CHUNK_K,
-                                 ct * TILE_N2 + (int)rank * B_ROWS2);
+                                 x.b_row + x.ct * TILE_N2 + (int)rank * B_ROWS2);
                 if (++s == STAGES2) { s = 0; ph ^= 1; }
             }
-            if (rp != cur_rp) {
+            if (x.first != cur_rp) {
                 // next row pair: its first B' tile is already on its way into the ring (the slots free up while the
                 // old rows' last MMAs run); A' can only be replaced once those MMAs have retired
                 mbar_wait(a_empty, (n_a - 1u) & 1u);
                 if (leader) mbar_expect_tx(a_bar, 2u * (uint32_t)nch * CHUNK_BYTES);
-                const int m0 = (2 * rp + (int)rank) * TILE_M;
                 for (int kc = 0; kc < nch; kc++) tma_load_2d_pair(sa + (size_t)kc * CHUNK_BYTES, &map_a, a_bar, kc * CHUNK_K, m0);
-                cur_rp = rp; n_a++;
+                cur_rp = x.first; n_a++;
             }
         }
     } else if (warp == 1 && lane == 0 && leader) {
@@ -724,8 +802,10 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         uint32_t g = 0;                                         // running chunk-slot counter of the B' ring
         int cur_rp = -1; uint32_t n_a = 0;
         for (int it = it0; it < it1; it++) {
-            const int t = it - it0, rp = it / CT;
-            if (rp != cur_rp) { mbar_wait(a_bar, n_a & 1u); tc_fence_after(); cur_rp = rp; n_a++; l2_stamp(p, 3); }
+            L2Item x;
+            l2_item<BATCH>(p, it, pp, x);
+            const int t = it - it0;
+            if (x.first != cur_rp) { mbar_wait(a_bar, n_a & 1u); tc_fence_after(); cur_rp = x.first; n_a++; l2_stamp(p, 3); }
             const int acc = t % NACC2;
             mbar_wait(&tempty[acc], ((t / NACC2) & 1) ^ 1);    // both CTAs' epilogues drained this accumulator
             tc_fence_after();
@@ -751,7 +831,7 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             }
             g += (uint32_t)dpc + 1u;
             tc_commit_pair(&tfull[acc]);
-            if (it + 1 < it1 && (it + 1) / CT != rp) tc_commit_pair(a_empty);   // A' may be overwritten once these retire
+            if (it + 1 < it1 && it + 1 - x.first >= x.col_tiles) tc_commit_pair(a_empty);   // A' may be overwritten once these retire
         }
     } else if (warp >= 4) {
         // ===== epilogue: one query row per thread, this CTA's 128 rows x 256 columns =====
@@ -760,38 +840,41 @@ l2_topk_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         RowTop rt;
         const BandParams bp{p.band_rel, p.band_abs_sqrt, p.band_abs_const};
         constexpr int NCOLS = TILE_N2 / EPI_GROUPS;
-        int cur_rp = -1, row = 0;
+        int cur_rp = -1, row = 0, n1 = 0, crow = 0;             // crow: the row's candidate-list row
         float s_, is2, mp;                                      // accumulator -> distance: -2 / s^2
         l2_scale_from_bits(__ldcg(p.absmax_bits), s_, is2, mp);
         const float out_scale = 2.f * is2;
         auto flush = [&]() {
-            if (cur_rp < 0 || row >= p.n1) return;
-            const int slot = cid - l2_segment_of_item(cur_rp * CT, items, clusters);
-            const size_t o = ((size_t)slot * p.n1 + row) * CAND + (size_t)eg * TOPK;
+            if (cur_rp < 0 || row >= n1) return;
+            const int slot = cid - l2_segment_of_item(cur_rp, items, clusters);
+            const size_t o = ((size_t)slot * cand_rows + crow) * CAND + (size_t)eg * TOPK;
 #pragma unroll
             for (int k = 0; k < TOPK; k++) {
                 p.cand_j[o + k] = rt.bk[k] != 0xFFFFFFFFu ? rt.bj[k] : -1;
                 p.cand_d[o + k] = rt.bk[k] != 0xFFFFFFFFu ? out_scale * __uint_as_float(rt.bk[k]) : 3.4e38f;
             }
-            p.cand_drop[((size_t)slot * p.n1 + row) * EPI_GROUPS + eg] =
+            p.cand_drop[((size_t)slot * cand_rows + crow) * EPI_GROUPS + eg] =
                 rt.bk[TOPK - 1] != 0xFFFFFFFFu ? out_scale * __uint_as_float(rt.bk[TOPK - 1]) : 3.4e38f;
         };
         for (int it = it0; it < it1; it++) {
-            const int t = it - it0, rp = it / CT, ct = it - rp * CT;
-            if (rp != cur_rp) {
+            L2Item x;
+            l2_item<BATCH>(p, it, pp, x);
+            const int t = it - it0;
+            if (x.first != cur_rp) {
                 flush();
-                cur_rp = rp;
-                row = (2 * rp + (int)rank) * TILE_M + ew * 32 + lane;
-                rowtop_reset(rt, row < p.n1, row < p.n1 ? __ldcg(p.qnorm + row) : 0.f);
+                cur_rp = x.first; n1 = x.n1;
+                row = x.m0 + (int)rank * TILE_M + ew * 32 + lane;
+                crow = x.row0 + row;
+                rowtop_reset(rt, row < n1, row < n1 ? __ldcg(p.qnorm + x.a_row + row) : 0.f);
             }
             const int acc = t % NACC2;
             mbar_wait(&tfull[acc], (t / NACC2) & 1);
             tc_fence_after();
             if (warp == 4 && lane == 0 && t < 36) l2_stamp(p, 40 + t);
-            const int jbase = ct * TILE_N2 + eg * NCOLS;
+            const int jbase = x.ct * TILE_N2 + eg * NCOLS;
             const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + (uint32_t)(acc * TILE_N2 + eg * NCOLS);
-            epilogue_reduce<NCOLS, DBG>(taddr, jbase, p.n2, p.key_mask, rt, bp,
-                                        DBG && p.dbg_dist && row < p.n1 ? p.dbg_dist + (size_t)row * p.n2 : nullptr, out_scale);
+            epilogue_reduce<NCOLS, DBG>(taddr, jbase, x.n2, p.key_mask, rt, bp,
+                                        DBG && p.dbg_dist && row < n1 ? p.dbg_dist + (size_t)row * p.n2 : nullptr, out_scale);
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive_remote(&tempty[acc], 0);      // the leader's barrier counts both CTAs' warps
@@ -829,18 +912,18 @@ inline size_t l2_smem_bytes() {
 // 2^-12 (3|q|^2 + 2 d_approx) covers both approximations with a factor 2.8 to spare.
 // Step 2: the survivors four at a time, so sixteen independent train-row loads are in flight per lane.
 // Summation order per distance: each lane's strided partial sum, then a butterfly.
-__global__ void __launch_bounds__(256, 7) l2_refine_kernel(const float *__restrict__ q, int n1, const float *__restrict__ t, int n2,
-                                                        int dim, const int32_t *__restrict__ cand_j,
-                                                        const float *__restrict__ cand_d, const float *__restrict__ cand_drop, int splits,
-                                                        int32_t *best_j, float *best_d, int32_t *second_j, float *second_d,
-                                                        float slack_rel, unsigned *hdr, int32_t *ovf_rows) {
-    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (warp >= n1) return;
-    const int i = warp;
+// One warp refines candidate-list row i (n1 rows per slot) of the query q (one row); the results go to element o of the
+// output arrays, an uncertified row is flagged as i.
+__device__ __forceinline__ void l2_refine_row(const float *__restrict__ q, const float *__restrict__ t, int n2, int dim,
+                                              const int32_t *__restrict__ cand_j, const float *__restrict__ cand_d,
+                                              const float *__restrict__ cand_drop, int splits, int n1, int i, size_t o_out,
+                                              int32_t *best_j, float *best_d, int32_t *second_j, float *second_d,
+                                              float slack_rel, unsigned *hdr, int32_t *ovf_rows) {
+    const int lane = threadIdx.x & 31;
     float qv[4], qn = 0.f;
 #pragma unroll
     for (int k = 0; k < 4; k++) {
-        qv[k] = lane + 32 * k < dim ? __ldg(q + (size_t)i * dim + lane + 32 * k) : 0.f;
+        qv[k] = lane + 32 * k < dim ? __ldg(q + lane + 32 * k) : 0.f;
         qn = fmaf(qv[k], qv[k], qn);
     }
     for (int o = 16; o; o >>= 1) qn += __shfl_xor_sync(0xffffffffu, qn, o);
@@ -922,8 +1005,8 @@ __global__ void __launch_bounds__(256, 7) l2_refine_kernel(const float *__restri
         }
     }
     if (lane == 0) {
-        best_j[i] = bj; best_d[i] = bj < 0 ? -1.f : b;
-        second_j[i] = sj; second_d[i] = sj < 0 ? -1.f : s;
+        best_j[o_out] = bj; best_d[o_out] = bj < 0 ? -1.f : b;
+        second_j[o_out] = sj; second_d[o_out] = sj < 0 ? -1.f : s;
     }
     // Certificate.  A train row x that the GEMM kernel's lists do not hold either lay outside the band of the second
     // best approximation when it was seen (and the band only shrinks), or was turned away / evicted by a full list --
@@ -940,6 +1023,16 @@ __global__ void __launch_bounds__(256, 7) l2_refine_kernel(const float *__restri
         }
         if (__any_sync(0xffffffffu, overflow) && lane == 0) ovf_rows[atomicAdd(hdr + 1, 1u)] = i;
     }
+}
+__global__ void __launch_bounds__(256, 7) l2_refine_kernel(const float *__restrict__ q, int n1, const float *__restrict__ t, int n2,
+                                                        int dim, const int32_t *__restrict__ cand_j,
+                                                        const float *__restrict__ cand_d, const float *__restrict__ cand_drop, int splits,
+                                                        int32_t *best_j, float *best_d, int32_t *second_j, float *second_d,
+                                                        float slack_rel, unsigned *hdr, int32_t *ovf_rows) {
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (warp >= n1) return;
+    l2_refine_row(q + (size_t)warp * dim, t, n2, dim, cand_j, cand_d, cand_drop, splits, n1, warp, (size_t)warp, best_j, best_d,
+                  second_j, second_d, slack_rel, hdr, ovf_rows);
 }
 
 // ---- exhaustive fallback for the rows the refinement could not certify ----------------------------
@@ -1064,6 +1157,242 @@ __global__ void __launch_bounds__(EX_THREADS) l2_exact_rows_kernel(const float *
         }
     }
     if (threadIdx.x == 0) hdr[2] = 0;                                              // ticket ready for the next call
+}
+
+
+// ---- many pairs per launch (pgm_knn2_l2_pairs_batch_dev, pgm_match_l2_ratio_crosscheck_pairs_batch_dev) ----------
+// A chunk of pairs runs the single-pair chain of the CTA-pair path -- scale, fp16 operands, GEMM + top-8, refinement,
+// exhaustive fallback -- once over all its pairs:
+//   l2b_prep_kernel          max |x| over every image the chunk converts (one power-of-two scale per chunk), resets the
+//                            flagged-row count, fills the candidate lists with "absent"
+//   l2b_split16_kernel       each image once per role: query form into A', train form into B' (one warp per row)
+//   l2_topk_pair_kernel<DBG, true>  flattened (pair, row pair, column tile) items
+//   l2b_refine_kernel        one warp per query row of the chunk; every row knows its pair
+//   l2b_exact_rows_kernel    the flagged rows of all pairs, (flagged row, train slice) work, merged by the last CTA
+// The ratio entry point adds l2b_filter_kernel + l2b_scatter_kernel.  Distances are computed by the code of the single-
+// pair kernels (l2_refine_row; the fallback sums in the same order), so a pair's result is bit-identical to its
+// pgm_knn2_l2_dev result whatever scale the chunk uses: the band is certified, the scale only decides how many rows
+// need the fallback.
+__global__ void __launch_bounds__(256) l2b_prep_kernel(const float *__restrict__ all, int dim, const L2BImage *__restrict__ img,
+                                                       int n_img, unsigned *__restrict__ hdr, int32_t *__restrict__ cand_j,
+                                                       size_t n_cand, float *__restrict__ cand_drop, size_t n_drop) {
+    pdl_trigger();
+    if (blockIdx.x == 0 && threadIdx.x == 0) hdr[1] = 0;
+    const size_t stride = (size_t)gridDim.x * blockDim.x, tid = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    for (size_t e = tid; e < n_cand; e += stride) cand_j[e] = -1;
+    for (size_t e = tid; e < n_drop; e += stride) cand_drop[e] = 3.4e38f;
+    unsigned m = 0;
+    for (int k = 0; k < n_img; k++) m = absmax_span(all + (size_t)img[k].src_row * dim, (size_t)img[k].n * dim, tid, stride, m);
+    absmax_commit(m, hdr);
+}
+
+// img_base[k] = first conversion row of image entry k (exclusive prefix over n_img entries)
+__global__ void __launch_bounds__(256) l2b_split16_kernel(const float *__restrict__ all, int dim, int dp, const L2BImage *__restrict__ img,
+                                                          const int32_t *__restrict__ img_base, int n_img, __half *__restrict__ a,
+                                                          __half *__restrict__ b, const unsigned *__restrict__ hdr,
+                                                          float *__restrict__ qnorm) {
+    const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    pdl_trigger();
+    if (w >= __ldg(img_base + n_img)) return;
+    const int e = l2_find(img_base, n_img, w);
+    const int r = w - __ldg(img_base + e);
+    PGM_ASSERT(e >= 0 && e < n_img && r >= 0 && r < img[e].n);
+    const bool train = img[e].train != 0;
+    const int row = img[e].dst_row + r;
+    __half *o = (train ? b : a) + (size_t)row * (dp + CHUNK_K);
+    float v[4];
+    split16_load(all + (size_t)(img[e].src_row + r) * dim, dim, dp, lane, v);
+    pdl_wait();                                      // the scale comes from l2b_prep_kernel
+    float s, inv_s2, mprime;
+    l2_scale_from_bits(__ldcg(hdr), s, inv_s2, mprime);
+    const float acc = split16_store(v, s, dp, lane, train, o);
+    if (!train && lane == 0) qnorm[row] = acc;
+}
+
+// row_base[k] = pairs[k].row0 (exclusive prefix over the chunk's pairs, row_base[n_pairs] = rows)
+__global__ void __launch_bounds__(256, 7) l2b_refine_kernel(const float *__restrict__ all, int dim, const L2BPair *__restrict__ pairs,
+                                                         const int32_t *__restrict__ row_base, int n_pairs, int rows,
+                                                         const int32_t *__restrict__ cand_j, const float *__restrict__ cand_d,
+                                                         const float *__restrict__ cand_drop, int splits, int32_t *best_j,
+                                                         float *best_d, int32_t *second_j, float *second_d, float slack_rel,
+                                                         unsigned *hdr, int32_t *ovf_rows) {
+    const int r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (r >= rows) return;
+    const int k = l2_find(row_base, n_pairs, r);
+    const L2BPair &pr = pairs[k];
+    const int i = r - pr.row0;
+    PGM_ASSERT(k >= 0 && k < n_pairs && i >= 0 && i < pr.n1);
+    l2_refine_row(all + (size_t)(pr.q_row + i) * dim, all + (size_t)pr.t_row * dim, pr.n2, dim, cand_j, cand_d, cand_drop,
+                  splits, rows, r, (size_t)(pr.out_row + i), best_j, best_d, second_j, second_d, slack_rel, hdr, ovf_rows);
+}
+
+// Flagged rows of all pairs of the chunk: work item = (flagged row, one of S slices of its pair's train image), S chosen
+// from the flagged count so that the grid has work (at most EX_MAX_SLICES_PER_ROW: `part` holds rows x that many).  Each
+// CTA's warps take four train rows per step; a distance is summed exactly as l2_refine_row sums it.  The CTA that
+// finishes last merges every flagged row's slices, adds the count to hdr[3] (the call's total) and returns the ticket
+// to zero.
+__global__ void __launch_bounds__(EX_THREADS) l2b_exact_rows_kernel(const float *__restrict__ all, int dim,
+                                                                    const L2BPair *__restrict__ pairs,
+                                                                    const int32_t *__restrict__ row_base, int n_pairs, int rows,
+                                                                    unsigned *__restrict__ hdr, const int32_t *__restrict__ ovf_rows,
+                                                                    float4 *__restrict__ part, int32_t *best_j, float *best_d,
+                                                                    int32_t *second_j, float *second_d) {
+    pdl_wait();
+    const int count = (int)__ldcg(hdr + 1);
+    if (blockIdx.x == 0 && threadIdx.x == 0) hdr[0] = 0;       // every reader of the scale has finished: reset for the next chunk
+    if (count == 0) return;
+    PGM_ASSERT(count <= rows);
+    const int S = (int)min((long long)EX_MAX_SLICES_PER_ROW, max(1ll, (2ll * gridDim.x + count - 1) / count));
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    __shared__ Top2 s_top[EX_THREADS / 32];
+    __shared__ unsigned s_ticket;
+    for (long long w = blockIdx.x; w < (long long)count * S; w += gridDim.x) {
+        const int f = (int)(w / S), sl = (int)(w - (long long)f * S);
+        const int r = __ldcg(ovf_rows + f);
+        PGM_ASSERT(r >= 0 && r < rows);
+        const int k = l2_find(row_base, n_pairs, r);
+        PGM_ASSERT(k >= 0 && k < n_pairs && r - pairs[k].row0 < pairs[k].n1);
+        const int n2 = pairs[k].n2;
+        const float *q = all + (size_t)(pairs[k].q_row + (r - pairs[k].row0)) * dim;
+        const float *t = all + (size_t)pairs[k].t_row * dim;
+        const int len = ((n2 + S - 1) / S + 3) & ~3;
+        const int j0 = min(n2, sl * len), j1 = min(n2, j0 + len);
+        float qv[4];
+#pragma unroll
+        for (int k2 = 0; k2 < 4; k2++) qv[k2] = lane + 32 * k2 < dim ? __ldg(q + lane + 32 * k2) : 0.f;
+        Top2 x{0.f, 0.f, -1, -1};
+        for (int jb = j0 + 4 * warp; jb < j1; jb += 4 * (EX_THREADS / 32)) {
+            float tv[4][4], acc[4];
+#pragma unroll
+            for (int u = 0; u < 4; u++)
+#pragma unroll
+                for (int k2 = 0; k2 < 4; k2++)
+                    tv[u][k2] = (jb + u < j1 && lane + 32 * k2 < dim) ? __ldg(t + (size_t)(jb + u) * dim + lane + 32 * k2) : 0.f;
+#pragma unroll
+            for (int u = 0; u < 4; u++) {
+                acc[u] = 0.f;
+#pragma unroll
+                for (int k2 = 0; k2 < 4; k2++) {
+                    const float df = qv[k2] - tv[u][k2];
+                    if (lane + 32 * k2 < dim) acc[u] = fmaf(df, df, acc[u]);
+                }
+            }
+#pragma unroll
+            for (int sh = 16; sh; sh >>= 1)
+#pragma unroll
+                for (int u = 0; u < 4; u++) acc[u] += __shfl_xor_sync(0xffffffffu, acc[u], sh);
+#pragma unroll
+            for (int u = 0; u < 4; u++) top2_insert(x, acc[u], jb + u < j1 ? jb + u : -1);
+        }
+        if (lane == 0) s_top[warp] = x;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            Top2 m = s_top[0];
+            for (int v = 1; v < EX_THREADS / 32; v++) { top2_insert(m, s_top[v].b, s_top[v].bj); top2_insert(m, s_top[v].s, s_top[v].sj); }
+            part[(size_t)f * S + sl] = make_float4(m.b, __int_as_float(m.bj), m.s, __int_as_float(m.sj));
+        }
+        __syncthreads();
+    }
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) s_ticket = atomicAdd(hdr + 2, 1u);
+    __syncthreads();
+    if (s_ticket != gridDim.x - 1) return;
+    __threadfence();                                                               // last CTA: merge the slices of every flagged row
+    for (int f = warp; f < count; f += EX_THREADS / 32) {
+        Top2 m{0.f, 0.f, -1, -1};
+        if (lane < S) {
+            const float4 v = __ldcg(part + (size_t)f * S + lane);
+            top2_insert(m, v.x, __float_as_int(v.y));
+            top2_insert(m, v.z, __float_as_int(v.w));
+        }
+        m = top2_warp_merge(m);
+        if (lane == 0) {
+            const int r = __ldcg(ovf_rows + f);
+            const int k = l2_find(row_base, n_pairs, r);
+            PGM_ASSERT(k >= 0 && k < n_pairs && r - pairs[k].row0 >= 0 && r - pairs[k].row0 < pairs[k].n1);
+            const size_t o = (size_t)(pairs[k].out_row + (r - pairs[k].row0));
+            best_j[o] = m.bj; best_d[o] = m.bj < 0 ? -1.f : m.b;
+            second_j[o] = m.sj; second_d[o] = m.sj < 0 ? -1.f : m.s;
+        }
+    }
+    if (threadIdx.x == 0) { hdr[3] += (unsigned)count; hdr[2] = 0; }              // call total; ticket ready for the next chunk
+}
+
+// Ratio test + cross-check + distance bound on the chunk's knn2 results, then the ordered compaction, as
+// rcp_filter_kernel / rcp_scatter_kernel do for Hamming keys (L2 distances are floats, so the keys do not carry them).
+struct L2RPair {
+    int64_t out_base;          // first slot of this pair's triples in the caller's output arrays
+    int32_t row0, rrow0;       // knn2 rows of the pair and, with cross-check, of the reversed pair (train image as query)
+    int32_t n1, n2, pair_id, pad;
+};
+constexpr int L2F_THREADS = 1024;    // rows per filter / scatter block (n1 < 2^20: at most 1024 blocks per pair)
+__global__ void __launch_bounds__(L2F_THREADS) l2b_filter_kernel(const L2RPair *__restrict__ pairs, const int32_t *__restrict__ fblk_base,
+                                                                 int n_pairs, int rows, const int32_t *__restrict__ bj,
+                                                                 const float *__restrict__ bd, const float *__restrict__ sd,
+                                                                 float ratio, float rr, int cross_check, float max_sq_dist,
+                                                                 int32_t *__restrict__ keep_row, int32_t *__restrict__ bcnt) {
+    const int g = blockIdx.x;
+    const int k = l2_find(fblk_base, n_pairs, g);
+    const L2RPair pr = pairs[k];
+    const int i = (g - __ldg(fblk_base + k)) * L2F_THREADS + threadIdx.x;
+    bool keep = false;
+    if (i < pr.n1) {
+        const int r = pr.row0 + i;
+        PGM_ASSERT(r >= 0 && r < rows);
+        const int j = bj[r];
+        const float d1 = bd[r], d2 = sd[r];
+        PGM_ASSERT(j < pr.n2);
+        keep = j >= 0;
+        keep = keep && (pr.n2 < 2 || ratio <= 0.f || d1 < rr * d2);
+        if (keep && cross_check) {
+            PGM_ASSERT(pr.rrow0 + j >= 0 && pr.rrow0 + j < rows);
+            keep = bj[pr.rrow0 + j] == i;
+        }
+        keep = keep && (max_sq_dist < 0.f || d1 <= max_sq_dist);
+        keep_row[r] = keep ? 1 : 0;
+    }
+    const int n = __syncthreads_count(keep);
+    if (threadIdx.x == 0) bcnt[g] = n;
+}
+
+__global__ void __launch_bounds__(L2F_THREADS) l2b_scatter_kernel(const L2RPair *__restrict__ pairs, const int32_t *__restrict__ fblk_base,
+                                                                  int n_pairs, const int32_t *__restrict__ keep_row,
+                                                                  const int32_t *__restrict__ bj, const float *__restrict__ bd,
+                                                                  const int32_t *__restrict__ bcnt, int64_t capacity,
+                                                                  int32_t *__restrict__ out_qi, int32_t *__restrict__ out_tj,
+                                                                  float *__restrict__ out_dist, int32_t *__restrict__ counts) {
+    __shared__ int s_before[L2F_THREADS / 32], s_total[L2F_THREADS / 32], s_w[L2F_THREADS / 32];
+    const int g = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int k = l2_find(fblk_base, n_pairs, g);
+    const L2RPair pr = pairs[k];
+    const int first = __ldg(fblk_base + k), nb = __ldg(fblk_base + k + 1) - first, b = g - first;
+    // kept rows of the pair's blocks before this one, and of all of them (nb <= L2F_THREADS)
+    const int c = tid < nb ? __ldg(bcnt + first + tid) : 0;
+    int before = tid < b ? c : 0, total = c;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        before += __shfl_xor_sync(0xffffffffu, before, o);
+        total += __shfl_xor_sync(0xffffffffu, total, o);
+    }
+    const int i = b * L2F_THREADS + tid;
+    const bool keep = i < pr.n1 && __ldg(keep_row + pr.row0 + i) != 0;
+    const unsigned m = __ballot_sync(0xffffffffu, keep);
+    if (lane == 0) { s_before[wid] = before; s_total[wid] = total; s_w[wid] = __popc(m); }
+    __syncthreads();
+    int off = 0;
+    before = 0; total = 0;
+#pragma unroll 4
+    for (int w = 0; w < L2F_THREADS / 32; w++) {
+        before += s_before[w]; total += s_total[w];
+        if (w < wid) off += s_w[w];
+    }
+    if (keep) {
+        const int64_t o = pr.out_base + before + off + __popc(m & ((1u << lane) - 1u));
+        PGM_ASSERT(o >= pr.out_base && o < pr.out_base + pr.n1 && o < capacity);
+        out_qi[o] = i; out_tj[o] = __ldg(bj + pr.row0 + i); out_dist[o] = __ldg(bd + pr.row0 + i);
+    }
+    if (b == nb - 1 && tid == 0) counts[pr.pair_id] = total;
 }
 
 }  // namespace pgm_l2

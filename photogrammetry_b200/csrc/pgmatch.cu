@@ -55,7 +55,8 @@ struct pgm_handle {
     DevBuf misc;      // knn2 partials etc.
     DevBuf shard_pool_state, shard_pool_est;   // a destroyed pgm_shard parks its device buffers here: the next one reuses them
     void *shard_pool_hctl = nullptr;           // (cudaMalloc / cudaMallocHost / cudaFree cost ~1.5 ms per train-sharded call)
-    DevBuf l2_state;  // float path, fp16 ranking: [max |x| bits, flagged rows, fallback ticket]; zeroed on allocation, self-cleaning
+    DevBuf l2_state;  // float path, fp16 ranking: [max |x| bits, flagged rows, fallback ticket, batch call's flagged rows];
+                      // zeroed on allocation, words 0-2 self-cleaning
     HostBuf pin_in;   // pinned staging, host -> device
     HostBuf pin_out;  // pinned staging, device -> host
     HostBuf pin_meta; // pinned PairDesc array + PlanInfo readback
@@ -67,6 +68,7 @@ struct pgm_handle {
     bool l2_attr_set = false;         // cudaFuncSetAttribute is per device, hence per handle
     int l2_max_clusters = 1;          // co-resident CTA pairs of the float pair kernel (persistent grid)
     unsigned *l2_hdr = nullptr;       // fp16 ranking mode of the last float call: [max |x| bits, rows recomputed exhaustively]
+    int l2_fallback_word = 1;         // the word of l2_hdr that counts them: 1 (one pair), 3 (the batch entry points' call total)
     DevBuf lat_state;             // LatState of latency mode (pgm_kernels.cuh): zeroed before its first use, left clean by every call
     bool lat_dirty = false;       // a latency-mode call was cut short between its launches: zero lat_state before the next
     bool stats_pending = false;   // rounds / evals of the last latency-mode call still sit in lat_state (device) ...
@@ -1456,6 +1458,32 @@ static int make_operand_map(pgm_handle *h, CUtensorMap *map, void *base, int row
     return PGM_OK;
 }
 
+// kernel attributes and the co-resident cluster count of the CTA-pair kernel, once per handle
+static int l2_setup(pgm_handle *h) {
+    using namespace pgm_l2;
+    if (h->l2_attr_set) return PGM_OK;
+    CU_CHECK(h, cudaFuncSetAttribute(l2_topk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_smem_bytes()));
+    CU_CHECK(h, cudaFuncSetAttribute(l2_topk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_smem_bytes()));
+    CU_CHECK(h, cudaFuncSetAttribute(l2_topk_pair_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_pair_smem_bytes()));
+    CU_CHECK(h, cudaFuncSetAttribute(l2_topk_pair_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_pair_smem_bytes()));
+    CU_CHECK(h, cudaFuncSetAttribute(l2_topk_pair_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_pair_smem_bytes()));
+    // how many CTA pairs are co-resident: the pair kernel is persistent, one segment of the work per cluster
+    cudaLaunchAttribute ca{};
+    ca.id = cudaLaunchAttributeClusterDimension;
+    ca.val.clusterDim.x = 2; ca.val.clusterDim.y = 1; ca.val.clusterDim.z = 1;
+    cudaLaunchConfig_t qc{};
+    qc.gridDim = dim3(2 * (unsigned)h->num_sms); qc.blockDim = dim3(THREADS);
+    qc.dynamicSmemBytes = l2_pair_smem_bytes(); qc.attrs = &ca; qc.numAttrs = 1;
+    int nc = 0;
+    if (cudaOccupancyMaxActiveClusters(&nc, l2_topk_pair_kernel<false, false>, &qc) != cudaSuccess || nc < 1) {
+        (void)cudaGetLastError();
+        nc = std::max(1, h->num_sms / 2);
+    }
+    h->l2_max_clusters = std::min(nc, std::max(1, h->num_sms / 2));
+    h->l2_attr_set = true;
+    return PGM_OK;
+}
+
 static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float *d_t, int32_t n2, int32_t dim,
                        int32_t *d_bj, float *d_bd, int32_t *d_sj, float *d_sd, float *d_dbg) {
     using namespace pgm_l2;
@@ -1466,26 +1494,8 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
     // fp16 term + certified band + exhaustive fallback (pair kernel), or the three-term bf16 split (single-CTA kernel)
     const bool pair = row_tiles >= 2, fp16 = pair;
     const int kprime = fp16 ? dp + CHUNK_K : 2 * dp + CHUNK_K;   // rows = [x16 | norm] or [hi | lo | norm]
-    if (!h->l2_attr_set) {
-        CU_CHECK(h, cudaFuncSetAttribute(l2_topk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_smem_bytes()));
-        CU_CHECK(h, cudaFuncSetAttribute(l2_topk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_smem_bytes()));
-        CU_CHECK(h, cudaFuncSetAttribute(l2_topk_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_pair_smem_bytes()));
-        CU_CHECK(h, cudaFuncSetAttribute(l2_topk_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l2_pair_smem_bytes()));
-        // how many CTA pairs are co-resident: the pair kernel is persistent, one segment of the work per cluster
-        cudaLaunchAttribute ca{};
-        ca.id = cudaLaunchAttributeClusterDimension;
-        ca.val.clusterDim.x = 2; ca.val.clusterDim.y = 1; ca.val.clusterDim.z = 1;
-        cudaLaunchConfig_t qc{};
-        qc.gridDim = dim3(2 * (unsigned)h->num_sms); qc.blockDim = dim3(THREADS);
-        qc.dynamicSmemBytes = l2_pair_smem_bytes(); qc.attrs = &ca; qc.numAttrs = 1;
-        int nc = 0;
-        if (cudaOccupancyMaxActiveClusters(&nc, l2_topk_pair_kernel<false>, &qc) != cudaSuccess || nc < 1) {
-            (void)cudaGetLastError();
-            nc = std::max(1, h->num_sms / 2);
-        }
-        h->l2_max_clusters = std::min(nc, std::max(1, h->num_sms / 2));
-        h->l2_attr_set = true;
-    }
+    int rc = l2_setup(h);
+    if (rc) return rc;
     int splits = 1, tps = 0, items = 0, clusters = 0;
     const int row_pairs = (row_tiles + 1) / 2;
     const int col_tiles = (n2 + (pair ? TILE_N2 : TILE_N) - 1) / (pair ? TILE_N2 : TILE_N);
@@ -1522,8 +1532,7 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
     const size_t o_ovf = take(fp16 ? (size_t)n1 * 4 : 0);
     const size_t o_part = take(fp16 ? (size_t)n1 * EX_MAX_SLICES_PER_ROW * 16 : 0);
     const size_t o_qn = take((size_t)n1 * 4), o_drop = take((size_t)splits * n1 * EPI_GROUPS * 4);
-    int rc = ensure_dev(h, h->misc, off);
-    if (rc) return rc;
+    if ((rc = ensure_dev(h, h->misc, off))) return rc;
     if (fp16 && h->l2_state.cap < 16) {
         if ((rc = ensure_dev(h, h->l2_state, 16))) return rc;
         CU_CHECK(h, cudaMemsetAsync(h->l2_state.p, 0, h->l2_state.cap, s));
@@ -1547,6 +1556,7 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
     p.band_abs_const = fp16 ? 2.44140625e-4f : 0.f;                        // 2^-12
     p.absmax_bits = hdr;
     h->l2_hdr = hdr;
+    h->l2_fallback_word = 1;
     p.cand_j = (int32_t *)(base + o_cj); p.cand_d = (float *)(base + o_cd); p.dbg_dist = d_dbg;
     const bool tl = getenv("PGM_L2_TIMELINE") != nullptr;
     if (tl) {
@@ -1578,8 +1588,8 @@ static int l2_dev_impl(pgm_handle *h, const float *d_q, int32_t n1, const float 
     if (pair) {
         cfg.gridDim = dim3(2 * (unsigned)clusters);
         cfg.dynamicSmemBytes = l2_pair_smem_bytes();
-        if (d_dbg) CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_pair_kernel<true>, map_a, map_b, p));
-        else CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_pair_kernel<false>, map_a, map_b, p));
+        if (d_dbg) CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_pair_kernel<true, false>, map_a, map_b, p));
+        else CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_pair_kernel<false, false>, map_a, map_b, p));
     } else {
         cfg.gridDim = dim3(row_tiles, splits); cfg.dynamicSmemBytes = l2_smem_bytes();
         if (d_dbg) CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_kernel<true>, map_a, map_b, p));
@@ -1657,11 +1667,11 @@ extern "C" int pgm_l2_last_fallback_rows(pgm_handle *h) {
     if (!h) return -1;
     std::lock_guard<std::mutex> lk(h->mu);
     if (!h->l2_hdr) return -1;
-    unsigned v[2] = {0, 0};
+    unsigned v[4] = {0, 0, 0, 0};
     if (cudaSetDevice(h->device) != cudaSuccess) return -1;
-    if (cudaMemcpyAsync(v, h->l2_hdr, 8, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) return -1;
+    if (cudaMemcpyAsync(v, h->l2_hdr, 16, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) return -1;
     if (cudaStreamSynchronize(h->stream) != cudaSuccess) return -1;
-    return (int)v[1];
+    return (int)v[h->l2_fallback_word];
 }
 
 extern "C" int pgm_knn2_l2(pgm_handle *h, const float *q, int32_t n1, const float *t, int32_t n2, int32_t dim,
@@ -1700,6 +1710,323 @@ extern "C" int pgm_knn2_l2(pgm_handle *h, const float *q, int32_t n1, const floa
     memcpy(best_d, po + n1, (size_t)n1 * 4);
     memcpy(second_j, po + 2 * (size_t)n1, (size_t)n1 * 4);
     memcpy(second_d, po + 3 * (size_t)n1, (size_t)n1 * 4);
+    return PGM_OK;
+}
+
+// ---------------------------------------------------------------------------
+// float descriptors, many pairs per call (pgm_l2.cuh, "many pairs per launch").  The host plans every chunk first,
+// uploads the whole plan in one copy and then only enqueues: five kernels per chunk (seven with the ratio filter).
+// ---------------------------------------------------------------------------
+constexpr int64_t L2B_MAX_ROWS = 1ll << 22;            // query rows per chunk (with cross-check: both directions)
+constexpr int64_t L2B_MAX_CONV_ROWS = 1ll << 22;       // fp16 operand rows per chunk (A' + B')
+constexpr int64_t L2B_MAX_CAND_BYTES = 1ll << 30;      // candidate lists: slots x rows x (CAND 8 + EPI_GROUPS 4) bytes
+
+struct L2BChunk {
+    int first, n;                  // GEMM pairs: plan[first, first + n)
+    int img_first, n_img;          // converted images: imgs[img_first, img_first + n_img)
+    int rfirst, rn;                // ratio entry point: filter pairs rplan[rfirst, rfirst + rn)
+    int base_off;                  // bases[base_off]: item_base (n + 1), row_base (n + 1), img_base (n_img + 1), fblk_base (rn + 1)
+    int32_t items, rows, a_rows, b_rows, clusters, splits, fblocks;
+};
+
+struct L2BPlan {
+    std::vector<pgm_l2::L2BPair> plan;
+    std::vector<pgm_l2::L2BImage> imgs;
+    std::vector<pgm_l2::L2RPair> rplan;
+    std::vector<int32_t> bases;
+    std::vector<L2BChunk> chunks;
+};
+
+// Chunks of at most MAX_CHUNK_PAIRS caller pairs, L2B_MAX_ROWS query rows, L2B_MAX_CONV_ROWS operand rows and
+// L2B_MAX_CAND_BYTES of candidate lists.  ratio: the filter's pairs too; with cross_check every pair (a, b) brings its
+// reversed pair (b, a), whose row best is the column best of (a, b) (the refinement's distances are symmetric).
+static void l2b_plan(pgm_handle *h, const int64_t *offs, int32_t n_images, const int32_t *pair_list, int32_t n_pairs,
+                     bool ratio, bool cross, L2BPlan &P) {
+    using namespace pgm_l2;
+    std::vector<int32_t> qpos(n_images), tpos(n_images), stamp_q(n_images, -1), stamp_t(n_images, -1);
+    int attempt = 0;
+    int64_t out_base = 0;
+    for (int p = 0; p < n_pairs;) {
+        int cap = MAX_CHUNK_PAIRS;
+        for (;;) {
+            attempt++;
+            L2BChunk c{(int)P.plan.size(), 0, (int)P.imgs.size(), 0, (int)P.rplan.size(), 0, (int)P.bases.size(), 0, 0, 0, 0, 0, 0, 0};
+            int64_t conv = 0, ob = out_base;
+            int q = p, taken = 0;
+            auto image = [&](int im, bool train) {                 // operand row of image im in its role (added once)
+                std::vector<int32_t> &pos = train ? tpos : qpos, &st = train ? stamp_t : stamp_q;
+                if (st[im] != attempt) {
+                    st[im] = attempt;
+                    const int32_t n = (int32_t)(offs[im + 1] - offs[im]);
+                    int32_t &rows = train ? c.b_rows : c.a_rows;
+                    pos[im] = rows;
+                    P.imgs.push_back(L2BImage{offs[im], rows, n, train ? 1 : 0, 0});
+                    rows += n; conv += n;
+                }
+                return pos[im];
+            };
+            auto gemm_pair = [&](int a, int b, int64_t out_row) {
+                L2BPair r{};
+                r.q_row = offs[a]; r.t_row = offs[b];
+                r.n1 = (int32_t)(offs[a + 1] - offs[a]); r.n2 = (int32_t)(offs[b + 1] - offs[b]);
+                r.a_row = image(a, false);
+                r.b_row = r.n2 > 0 ? image(b, true) : 0;
+                r.row0 = c.rows; r.out_row = ratio ? c.rows : out_row;
+                r.item0 = c.items; r.col_tiles = (r.n2 + TILE_N2 - 1) / TILE_N2;
+                c.items += (r.n1 + 2 * TILE_M - 1) / (2 * TILE_M) * r.col_tiles;
+                c.rows += r.n1;
+                P.plan.push_back(r);
+                c.n++;
+                return r.row0;
+            };
+            for (; q < n_pairs && taken < cap; q++) {
+                const int a = pair_list[2 * q], b = pair_list[2 * q + 1];
+                const int64_t n1 = offs[a + 1] - offs[a], n2 = offs[b + 1] - offs[b];
+                const bool run = n1 > 0 && (!ratio || n2 > 0);       // the ratio filter keeps nothing without train rows
+                if (run) {
+                    const bool rev = ratio && cross;
+                    const int64_t rows = n1 + (rev ? n2 : 0);
+                    const int64_t cv = (stamp_q[a] == attempt ? 0 : n1) + (stamp_t[b] == attempt ? 0 : n2) +
+                                       (rev ? (stamp_q[b] == attempt || a == b ? 0 : n2) + (stamp_t[a] == attempt || a == b ? 0 : n1) : 0);
+                    if (taken > 0 && (c.rows + rows > L2B_MAX_ROWS || conv + cv > L2B_MAX_CONV_ROWS)) break;
+                    const int32_t row0 = gemm_pair(a, b, ob);
+                    const int32_t rrow0 = rev ? gemm_pair(b, a, 0) : 0;
+                    if (ratio) {
+                        P.rplan.push_back(L2RPair{ob, row0, rrow0, (int32_t)n1, (int32_t)n2, q, 0});
+                        c.rn++;
+                    }
+                    taken++;
+                }
+                ob += n1;
+            }
+            // candidate slots: the most segments any row pair is cut into (as in l2_dev_impl)
+            c.clusters = std::max(1, std::min(h->l2_max_clusters, c.items));
+            c.splits = 1;
+            for (int k = c.first; k < c.first + c.n; k++) {
+                const L2BPair &r = P.plan[k];
+                if (r.col_tiles == 0) continue;
+                for (int32_t x0 = r.item0; x0 < r.item0 + (r.n1 + 2 * TILE_M - 1) / (2 * TILE_M) * r.col_tiles; x0 += r.col_tiles) {
+                    const int64_t x1 = x0 + r.col_tiles - 1;
+                    const int k0 = (int)(((int64_t)(x0 + 1) * c.clusters - 1) / c.items), k1 = (int)(((x1 + 1) * c.clusters - 1) / c.items);
+                    c.splits = std::max(c.splits, k1 - k0 + 1);
+                }
+            }
+            if (taken > 1 && (int64_t)c.splits * c.rows * (CAND * 8 + EPI_GROUPS * 4) > L2B_MAX_CAND_BYTES) {
+                P.plan.resize(c.first); P.imgs.resize(c.img_first); P.rplan.resize(c.rfirst);
+                cap = taken / 2;
+                continue;
+            }
+            c.n_img = (int)P.imgs.size() - c.img_first;
+            P.bases.resize(P.bases.size() + 2 * (size_t)(c.n + 1) + (size_t)(c.n_img + 1) + (size_t)(c.rn + 1));
+            int32_t *ib = P.bases.data() + c.base_off, *rb = ib + c.n + 1, *gb = rb + c.n + 1, *fb = gb + c.n_img + 1;
+            for (int k = 0; k < c.n; k++) { ib[k] = P.plan[c.first + k].item0; rb[k] = P.plan[c.first + k].row0; }
+            ib[c.n] = c.items; rb[c.n] = c.rows;
+            int32_t g = 0;
+            for (int k = 0; k < c.n_img; k++) { gb[k] = g; g += P.imgs[c.img_first + k].n; }
+            gb[c.n_img] = g;
+            for (int k = 0; k < c.rn; k++) { fb[k] = c.fblocks; c.fblocks += (P.rplan[c.rfirst + k].n1 + L2F_THREADS - 1) / L2F_THREADS; }
+            fb[c.rn] = c.fblocks;
+            if (c.n > 0) P.chunks.push_back(c);
+            p = q;
+            out_base = ob;
+            break;
+        }
+    }
+}
+
+// Enqueues the chunks of a plan.  d_bj.. : knn2 results (the caller's arrays, or the per-chunk scratch with the ratio
+// filter, which then writes the triples).
+static int l2b_run(pgm_handle *h, const float *d_all, int32_t dim, int32_t n_pairs, const L2BPlan &P, bool ratio_mode,
+                   float ratio, bool cross, float max_sq_dist, int32_t *d_bj, float *d_bd, int32_t *d_sj, float *d_sd,
+                   int32_t *d_out_qi, int32_t *d_out_tj, float *d_out_dist, int64_t capacity, int32_t *out_counts) {
+    using namespace pgm_l2;
+    cudaStream_t s = h->stream;
+    const int dp = (dim + CHUNK_K - 1) / CHUNK_K * CHUNK_K, dpc = dp / CHUNK_K, kprime = dp + CHUNK_K;
+    int64_t max_rows = 1, max_a = 1, max_b = 1, max_cand = 1, max_fb = 1;
+    for (const L2BChunk &c : P.chunks) {
+        max_rows = std::max<int64_t>(max_rows, c.rows); max_a = std::max<int64_t>(max_a, c.a_rows);
+        max_b = std::max<int64_t>(max_b, c.b_rows); max_cand = std::max<int64_t>(max_cand, (int64_t)c.splits * c.rows);
+        max_fb = std::max<int64_t>(max_fb, c.fblocks);
+    }
+    // h->misc: plan | images | filter pairs | bases | counts || A' | B' | |q|^2 | cand_j | cand_d | cand_drop | flagged rows |
+    // fallback partials | knn2 scratch (ratio) | kept-row flags | block counts
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + std::max<size_t>(bytes, 1), 1024); return o; };
+    const size_t o_plan = take(sizeof(L2BPair) * P.plan.size()), o_img = take(sizeof(L2BImage) * P.imgs.size());
+    const size_t o_rplan = take(sizeof(L2RPair) * P.rplan.size()), o_bases = take(4 * P.bases.size());
+    const size_t o_counts = take(4 * (size_t)n_pairs), upload = o_counts;
+    const size_t o_a = take((size_t)max_a * kprime * 2), o_b = take((size_t)max_b * kprime * 2), o_qn = take((size_t)max_a * 4);
+    const size_t o_cj = take((size_t)max_cand * CAND * 4), o_cd = take((size_t)max_cand * CAND * 4);
+    const size_t o_drop = take((size_t)max_cand * EPI_GROUPS * 4), o_ovf = take((size_t)max_rows * 4);
+    const size_t o_part = take((size_t)max_rows * EX_MAX_SLICES_PER_ROW * 16);
+    const size_t o_knn = take(ratio_mode ? (size_t)max_rows * 16 : 0), o_keep = take(ratio_mode ? (size_t)max_rows * 4 : 0);
+    const size_t o_bcnt = take(ratio_mode ? (size_t)max_fb * 4 : 0);
+    int rc = ensure_dev(h, h->misc, off);
+    if (rc) return rc;
+    if ((rc = ensure_host(h, h->pin_in, upload + 4 * (size_t)n_pairs))) return rc;      // the plan, then the counts read-back
+    if (h->l2_state.cap < 16) {
+        if ((rc = ensure_dev(h, h->l2_state, 16))) return rc;
+        CU_CHECK(h, cudaMemsetAsync(h->l2_state.p, 0, h->l2_state.cap, s));
+    }
+    unsigned *hdr = (unsigned *)h->l2_state.p;
+    CU_CHECK(h, cudaStreamSynchronize(s));                 // the staging buffer may still feed an earlier call's copy
+    char *pin = (char *)h->pin_in.p, *dev = (char *)h->misc.p;
+    memcpy(pin + o_plan, P.plan.data(), sizeof(L2BPair) * P.plan.size());
+    memcpy(pin + o_img, P.imgs.data(), sizeof(L2BImage) * P.imgs.size());
+    memcpy(pin + o_rplan, P.rplan.data(), sizeof(L2RPair) * P.rplan.size());
+    memcpy(pin + o_bases, P.bases.data(), 4 * P.bases.size());
+    CU_CHECK(h, cudaMemcpyAsync(dev, pin, upload, cudaMemcpyHostToDevice, s));
+    CU_CHECK(h, cudaMemsetAsync(hdr + 3, 0, 4, s));       // flagged rows of this call, over all chunks
+    h->l2_hdr = hdr;
+    h->l2_fallback_word = 3;
+    if (ratio_mode) CU_CHECK(h, cudaMemsetAsync(dev + o_counts, 0, 4 * (size_t)n_pairs, s));
+    const L2BPair *d_plan = (const L2BPair *)(dev + o_plan);
+    const L2BImage *d_img = (const L2BImage *)(dev + o_img);
+    const L2RPair *d_rplan = (const L2RPair *)(dev + o_rplan);
+    const int32_t *d_bases = (const int32_t *)(dev + o_bases);
+    __half *a = (__half *)(dev + o_a), *b = (__half *)(dev + o_b);
+    float *qnorm = (float *)(dev + o_qn);
+    int32_t *cand_j = (int32_t *)(dev + o_cj), *ovf = (int32_t *)(dev + o_ovf);
+    float *cand_d = (float *)(dev + o_cd), *cand_drop = (float *)(dev + o_drop);
+    if (ratio_mode) {
+        d_bj = (int32_t *)(dev + o_knn); d_bd = (float *)(d_bj + max_rows);
+        d_sj = (int32_t *)(d_bd + max_rows); d_sd = (float *)(d_sj + max_rows);
+    }
+    // the band of l2_dev_impl's fp16 ranking
+    const float slack_rel = 0.00244140625f;
+    L2Params p{};
+    p.dpc = dpc; p.key_mask = 0x7FFFFFE0u;
+    p.band_rel = 0.5f * slack_rel;
+    p.band_abs_sqrt = 4.8828125e-7f * sqrtf((float)dp);
+    p.band_abs_const = 2.44140625e-4f;
+    p.absmax_bits = hdr; p.qnorm = qnorm; p.cand_j = cand_j; p.cand_d = cand_d; p.cand_drop = cand_drop;
+    cudaLaunchAttribute pdl{};
+    pdl.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    pdl.val.programmaticStreamSerializationAllowed = 1;
+    const float rr = ratio * ratio;                        // Lowe's ratio on Euclidean distances, on squared ones
+    for (const L2BChunk &c : P.chunks) {
+        const int32_t *ib = d_bases + c.base_off, *rb = ib + c.n + 1, *gb = rb + c.n + 1, *fb = gb + c.n_img + 1;
+        const L2BPair *cp = d_plan + c.first;
+        const size_t n_cand = (size_t)c.splits * c.rows;
+        int64_t conv_floats = 0;
+        for (int k = 0; k < c.n_img; k++) conv_floats += (int64_t)P.imgs[c.img_first + k].n * dim;
+        const int pb = (int)std::min<int64_t>((int64_t)h->num_sms * 8, (conv_floats + (int64_t)n_cand * CAND + 4095) / 4096 + 1);
+        l2b_prep_kernel<<<pb, 256, 0, s>>>(d_all, dim, d_img + c.img_first, c.n_img, hdr, cand_j, n_cand * CAND, cand_drop,
+                                           n_cand * EPI_GROUPS);
+        cudaLaunchConfig_t cfg{};
+        cfg.stream = s; cfg.attrs = &pdl; cfg.numAttrs = 1;
+        cfg.gridDim = dim3((unsigned)(((int64_t)(c.a_rows + c.b_rows) * 32 + 255) / 256)); cfg.blockDim = dim3(256);
+        CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2b_split16_kernel, d_all, (int)dim, dp, d_img + c.img_first, gb, c.n_img, a, b,
+                                       (const unsigned *)hdr, qnorm));
+        int launches = 4;
+        if (c.items > 0) {
+            CUtensorMap map_a, map_b;
+            if ((rc = make_operand_map(h, &map_a, a, std::max(c.a_rows, 1), kprime))) return rc;
+            if ((rc = make_operand_map(h, &map_b, b, std::max(c.b_rows, 1), kprime, B_ROWS2))) return rc;
+            p.items = c.items; p.bpairs = cp; p.item_base = ib; p.n_pairs = c.n; p.rows = c.rows;
+            cfg.gridDim = dim3(2 * (unsigned)c.clusters); cfg.blockDim = dim3(THREADS);
+            cfg.dynamicSmemBytes = l2_pair_smem_bytes();
+            CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2_topk_pair_kernel<false, true>, map_a, map_b, p));
+            launches++;
+        }
+        cfg.gridDim = dim3((unsigned)(((int64_t)c.rows * 32 + 255) / 256)); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = 0;
+        CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2b_refine_kernel, d_all, (int)dim, cp, rb, c.n, (int)c.rows, (const int32_t *)cand_j,
+                                       (const float *)cand_d, (const float *)cand_drop, (int)c.splits, d_bj, d_bd, d_sj, d_sd,
+                                       slack_rel, hdr, ovf));
+        cfg.gridDim = dim3((unsigned)h->num_sms * 4); cfg.blockDim = dim3(EX_THREADS);
+        CU_CHECK(h, cudaLaunchKernelEx(&cfg, l2b_exact_rows_kernel, d_all, (int)dim, cp, rb, c.n, (int)c.rows, hdr,
+                                       (const int32_t *)ovf, (float4 *)(dev + o_part), d_bj, d_bd, d_sj, d_sd));
+        if (ratio_mode && c.rn > 0) {
+            int32_t *keep = (int32_t *)(dev + o_keep), *bcnt = (int32_t *)(dev + o_bcnt);
+            l2b_filter_kernel<<<c.fblocks, L2F_THREADS, 0, s>>>(d_rplan + c.rfirst, fb, c.rn, c.rows, d_bj, d_bd, d_sd, ratio, rr,
+                                                                cross ? 1 : 0, max_sq_dist, keep, bcnt);
+            l2b_scatter_kernel<<<c.fblocks, L2F_THREADS, 0, s>>>(d_rplan + c.rfirst, fb, c.rn, keep, d_bj, d_bd, bcnt, capacity,
+                                                                 d_out_qi, d_out_tj, d_out_dist, (int32_t *)(dev + o_counts));
+            launches += 2;
+        }
+        CU_CHECK(h, cudaGetLastError());
+        h->stats.kernel_launches += launches;
+    }
+    h->stats.host_syncs += 1;
+    if (ratio_mode) {
+        CU_CHECK(h, cudaMemcpyAsync(pin + o_counts, dev + o_counts, 4 * (size_t)n_pairs, cudaMemcpyDeviceToHost, s));
+        CU_CHECK(h, cudaStreamSynchronize(s));
+        memcpy(out_counts, pin + o_counts, 4 * (size_t)n_pairs);
+        h->stats.host_syncs += 1;
+        for (int q = 0; q < n_pairs; q++) h->stats.matched += out_counts[q];
+    }
+    return PGM_OK;
+}
+
+// argument checks shared by both batch entry points; *evals = sum of n1 n2, *rows = sum of n1
+static int l2b_check(pgm_handle *h, const int64_t *image_offsets, int32_t n_images, const int32_t *pair_list, int32_t n_pairs,
+                     int32_t dim, int64_t *evals, int64_t *rows) {
+    if (dim < 1 || dim > 128) return fail(h, PGM_E_INVALID_ARG, "dim must be in 1..128");
+    *evals = 0; *rows = 0;
+    for (int p = 0; p < n_pairs; p++) {
+        const int a = pair_list[2 * p], b = pair_list[2 * p + 1];
+        if (a < 0 || a >= n_images || b < 0 || b >= n_images) return fail(h, PGM_E_INVALID_ARG, "pair index out of range");
+        const int64_t n1 = image_offsets[a + 1] - image_offsets[a], n2 = image_offsets[b + 1] - image_offsets[b];
+        if (n1 < 0 || n2 < 0 || n1 >= MAX_N || n2 >= MAX_N || image_offsets[a] < 0 || image_offsets[b] < 0)
+            return fail(h, PGM_E_INVALID_ARG, "bad image sizes");
+        *rows += n1;
+        *evals += n1 * n2;
+    }
+    return PGM_OK;
+}
+
+extern "C" int pgm_knn2_l2_pairs_batch_dev(pgm_handle *h, const float *d_all_desc, const int64_t *image_offsets, int32_t n_images,
+                                           const int32_t *pair_list, int32_t n_pairs, int32_t dim, int32_t *d_best_j,
+                                           float *d_best_d, int32_t *d_second_j, float *d_second_d, int64_t capacity) {
+    if (!h || n_pairs < 0 || n_images < 0 || (n_pairs > 0 && (!image_offsets || !pair_list))) return PGM_E_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    h->stats = pgm_stats{};
+    h->stats_pending = false;
+    int64_t evals, rows;
+    int rc = l2b_check(h, image_offsets, n_images, pair_list, n_pairs, dim, &evals, &rows);
+    if (rc) return rc;
+    if (capacity < rows) return fail(h, PGM_E_CAPACITY, "capacity < sum of query sizes");
+    if (n_pairs == 0 || rows == 0) return PGM_OK;
+    if (!d_all_desc || !d_best_j || !d_best_d || !d_second_j || !d_second_d) return fail(h, PGM_E_INVALID_ARG, "null pointer");
+    CU_CHECK(h, cudaSetDevice(h->device));
+    if ((rc = l2_setup(h))) return rc;
+    L2BPlan P;
+    l2b_plan(h, image_offsets, n_images, pair_list, n_pairs, false, false, P);
+    if ((rc = l2b_run(h, d_all_desc, dim, n_pairs, P, false, 0.f, false, -1.f, d_best_j, d_best_d, d_second_j, d_second_d,
+                      nullptr, nullptr, nullptr, capacity, nullptr)))
+        return rc;
+    h->stats.pairs = n_pairs;
+    h->stats.distance_evals = evals;
+    h->stats.evals_computed = evals;
+    return PGM_OK;
+}
+
+extern "C" int pgm_match_l2_ratio_crosscheck_pairs_batch_dev(pgm_handle *h, const float *d_all_desc, const int64_t *image_offsets,
+                                                             int32_t n_images, const int32_t *pair_list, int32_t n_pairs,
+                                                             int32_t dim, float ratio, int32_t cross_check, float max_sq_dist,
+                                                             int32_t *d_out_qi, int32_t *d_out_tj, float *d_out_dist,
+                                                             int64_t capacity, int32_t *out_counts) {
+    if (!h || !out_counts || n_pairs < 0 || n_images < 0 || (n_pairs > 0 && (!image_offsets || !pair_list))) return PGM_E_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    h->stats = pgm_stats{};
+    h->stats_pending = false;
+    int64_t evals, rows;
+    int rc = l2b_check(h, image_offsets, n_images, pair_list, n_pairs, dim, &evals, &rows);
+    if (rc) return rc;
+    if (capacity < rows) return fail(h, PGM_E_CAPACITY, "capacity < sum of query sizes");
+    if (n_pairs == 0) return PGM_OK;
+    if (!d_all_desc || !d_out_qi || !d_out_tj || !d_out_dist) return fail(h, PGM_E_INVALID_ARG, "null pointer");
+    CU_CHECK(h, cudaSetDevice(h->device));
+    if ((rc = l2_setup(h))) return rc;
+    const bool cross = cross_check != 0;
+    L2BPlan P;
+    l2b_plan(h, image_offsets, n_images, pair_list, n_pairs, true, cross, P);
+    if ((rc = l2b_run(h, d_all_desc, dim, n_pairs, P, true, ratio, cross, max_sq_dist, nullptr, nullptr, nullptr, nullptr,
+                      d_out_qi, d_out_tj, d_out_dist, capacity, out_counts)))
+        return rc;
+    h->stats.pairs = n_pairs;
+    h->stats.distance_evals = evals;
+    h->stats.evals_computed = cross ? 2 * evals : evals;    // the reversed pairs' top-2 pass gives the column best
     return PGM_OK;
 }
 

@@ -335,9 +335,61 @@ class Matcher:
                                           sj.ctypes.data, sd.ctypes.data))
         return bj[:n1], bd[:n1], sj[:n1], sd[:n1]
 
+    def knn2_l2_pairs_batch_dev(self, d_all_desc, image_offsets, pair_list):
+        """:meth:`knn2_l2` for many image pairs in one call.  ``d_all_desc``: torch float32 ``[rows, dim]`` on the GPU
+        (``dim <= 128``), image ``k`` = rows ``image_offsets[k]:image_offsets[k + 1]``.  Returns ``(best_j, best_d,
+        second_j, second_d, starts)``: tensors of ``sum of n1`` rows; pair ``p``'s query rows start at ``starts[p]``.
+        Per pair the result is bit-identical to :meth:`knn2_l2` on the CTA-pair path (``n1 > 128``)."""
+        import torch
+        offs = np.ascontiguousarray(image_offsets, dtype=np.int64)
+        pairs = np.ascontiguousarray(pair_list, dtype=np.int32).reshape(-1, 2)
+        starts = self._pair_starts(offs, pairs)
+        total = int(starts[-1])
+        dev = d_all_desc.device
+        bj = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+        sj = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+        bd = torch.empty(max(total, 1), dtype=torch.float32, device=dev)
+        sd = torch.empty(max(total, 1), dtype=torch.float32, device=dev)
+        with self.torch_ordered(dev):
+            self._check(self._lib.pgm_knn2_l2_pairs_batch_dev(
+                self._h, d_all_desc.data_ptr(), offs.ctypes.data, len(offs) - 1, pairs.ctypes.data, len(pairs),
+                int(d_all_desc.shape[1]), bj.data_ptr(), bd.data_ptr(), sj.data_ptr(), sd.data_ptr(), total))
+        return bj[:total], bd[:total], sj[:total], sd[:total], starts[:-1]
+
+    def match_l2_ratio_crosscheck_pairs_batch_dev(self, d_all_desc, image_offsets, pair_list, ratio: float = 0.8,
+                                                  cross_check: bool = True, max_sq_dist: float = -1.0):
+        """Float descriptors: nearest neighbour + Lowe's ratio test + cross-check for many image pairs in one call.
+        ``d_all_desc`` as in :meth:`knn2_l2_pairs_batch_dev`.  Keeps ``(i, j1, d1)`` iff ``n2 < 2 or ratio <= 0 or
+        d1 < ratio^2 d2`` (squared distances, fp32), ``j1``'s nearest query is ``i`` (with ``cross_check``) and
+        ``max_sq_dist < 0 or d1 <= max_sq_dist``.  Returns ``(qi int32, tj int32, dist float32, starts int64[n_pairs],
+        counts int32[n_pairs])``; pair ``p`` owns ``[starts[p], starts[p] + counts[p])`` in ascending ``qi``."""
+        import torch
+        offs = np.ascontiguousarray(image_offsets, dtype=np.int64)
+        pairs = np.ascontiguousarray(pair_list, dtype=np.int32).reshape(-1, 2)
+        starts = self._pair_starts(offs, pairs)
+        total = int(starts[-1])
+        dev = d_all_desc.device
+        qi = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+        tj = torch.empty(max(total, 1), dtype=torch.int32, device=dev)
+        dist = torch.empty(max(total, 1), dtype=torch.float32, device=dev)
+        counts = np.zeros(max(len(pairs), 1), dtype=np.int32)
+        with self.torch_ordered(dev):
+            self._check(self._lib.pgm_match_l2_ratio_crosscheck_pairs_batch_dev(
+                self._h, d_all_desc.data_ptr(), offs.ctypes.data, len(offs) - 1, pairs.ctypes.data, len(pairs),
+                int(d_all_desc.shape[1]), float(ratio), int(bool(cross_check)), float(max_sq_dist), qi.data_ptr(),
+                tj.data_ptr(), dist.data_ptr(), total, counts.ctypes.data))
+        return qi, tj, dist, starts[:-1], counts[:len(pairs)]
+
+    @staticmethod
+    def _pair_starts(offs, pairs):
+        sizes = np.diff(offs)
+        n1s = sizes[pairs[:, 0]] if len(pairs) else np.zeros(0, np.int64)
+        return np.concatenate([[0], np.cumsum(n1s)]).astype(np.int64)
+
     def l2_last_fallback_rows(self) -> int:
         """Queries of the last float call that were recomputed exhaustively (their candidate band could not be
-        certified from the kernel's top-8 lists); -1 if that call used the three-term bf16 ranking."""
+        certified from the kernel's top-8 lists; a batch call counts all its chunks and both directions); -1 if that
+        call used the three-term bf16 ranking."""
         return int(self._lib.pgm_l2_last_fallback_rows(self._h))
 
     # -- the producer of the matcher's inputs: FAST-12, BRIEF, NMS ----------

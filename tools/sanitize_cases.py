@@ -10,6 +10,9 @@
   5. 3 emulated train shards of a 700 x 650 pair (export / propose / stable commit kernels)
   6. ratio test + cross-check of 7 pairs of any size, empty and split ones included (fused distance pass with
      column splits, split-partial merge, block-parallel ordered compaction)
+  7. float L2 batch of 6 pairs: one large pair whose row pairs span several segments (split candidate slots), flagged
+     rows in two pairs (crowded band, identical train rows) taken by the batched fallback, then the ratio + cross-check
+     filter with its reversed pairs and ordered compaction
 Every result is checked against the oracle, so a sanitizer run is also a parity run."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -57,5 +60,33 @@ for ratio, cc, md in [(0.8, True, -1), (0.0, False, 60)]:
     for p, (a, b) in enumerate(pairs):
         assert (out[:, starts[p]:starts[p] + counts[p]].T == orc.match_ratio_crosscheck(imgs[a], imgs[b], ratio, cc, md)).all()
 print("case 6 ok", m.stats())
+rng = np.random.default_rng(9)
+big_q, big_t = rng.random((2600, 128), dtype=np.float32), rng.random((9000, 128), dtype=np.float32)
+crowd_q, crowd_t = rng.standard_normal((600, 128)).astype(np.float32), rng.standard_normal((3000, 128)).astype(np.float32)
+for k in range(12):
+    crowd_t[100 + k] = crowd_q[7] + np.float32(0.01 * (12 - k)) * np.eye(128, dtype=np.float32)[3]
+same_q, same_t = rng.standard_normal((300, 128)).astype(np.float32), np.tile(rng.standard_normal((1, 128)).astype(np.float32), (5000, 1))
+imgs = [big_q, big_t, crowd_q, crowd_t, same_q, same_t, rng.standard_normal((100, 128)).astype(np.float32)]
+offs = np.concatenate([[0], np.cumsum([len(x) for x in imgs])]).astype(np.int64)
+pairs = np.array([(0, 1), (2, 3), (4, 5), (6, 2), (3, 2), (1, 0)], dtype=np.int32)
+d_all = torch.from_numpy(np.concatenate(imgs)).cuda()
+res = [x.cpu().numpy() for x in m.knn2_l2_pairs_batch_dev(d_all, offs, pairs)[:4]]
+assert m.l2_last_fallback_rows() >= 301
+rev = [x.cpu().numpy() for x in m.knn2_l2_pairs_batch_dev(d_all, offs, pairs[:, ::-1].copy())[:4]]
+qi, tj, dist, starts, counts = (x.cpu().numpy() if hasattr(x, "cpu") else x
+                                for x in m.match_l2_ratio_crosscheck_pairs_batch_dev(d_all, offs, pairs, 0.8, True))
+o = ro = 0
+for p, (a, b) in enumerate(pairs):
+    n1, n2 = len(imgs[a]), len(imgs[b])
+    bj, bd, sj, sd = (x[o:o + n1] for x in res)
+    ej, ed, fj, fd = orc.l2_knn2(imgs[a], imgs[b])
+    for g_d, e_d in ((bd, ed), (sd, fd)):
+        assert (np.abs(g_d - e_d) <= 1e-4 * np.maximum(e_d, 1e-12) + 1e-6).all()
+    assert (bj != ej).mean() <= 0.01
+    keep = (bd < np.float32(np.float32(0.8) * np.float32(0.8)) * sd) & (rev[0][ro:ro + n2][bj] == np.arange(n1))
+    assert counts[p] == keep.sum() and (qi[starts[p]:starts[p] + counts[p]] == np.nonzero(keep)[0]).all()
+    assert (tj[starts[p]:starts[p] + counts[p]] == bj[keep]).all() and (dist[starts[p]:starts[p] + counts[p]] == bd[keep]).all()
+    o += n1; ro += n2
+print("case 7 ok", m.stats())
 m.close()
 print("ALL OK")
