@@ -348,6 +348,47 @@ int pgm_ransac_score(pgm_handle *h, const float *F, const uint8_t *valid, int32_
                      const int32_t *xy2, int32_t n, float threshold, int32_t *out_counts, int32_t *out_best,
                      uint8_t *out_best_mask);
 
+/* pgm_ransac_fundamental_pairs_batch_dev: GetFundamentalMatrix(list, n_samples, pairs_per_sample, threshold)
+ * (CameraPoseEstimation.cs:26-94, as the host mirror camera_pose_estimation.py restates it) for MANY match lists in one
+ * call, on the device, with no read-back (pgm_stats.host_syncs == 0).
+ *  - Inputs: d_all_xy device int32[rows][2] = (x, y) of every keypoint, image k at rows [image_offsets[k],
+ *    image_offsets[k + 1]) (host int64[n_images + 1]); pair_list host int32[n_pairs][2] = (image a, image b); pair p owns
+ *    the match slots [match_starts[p], match_starts[p] + match_counts[p]) (host arrays) of d_match_qi / d_match_tj
+ *    (device int32[capacity]): Keypoint1 = row image_offsets[a] + qi of d_all_xy, Keypoint2 = row image_offsets[b] + tj.
+ *    That is the output layout of the batch matchers (greedy tail triples included).  The indices must lie inside their
+ *    images (a precondition; the -DPGM_CHECKED build asserts it).
+ *  - Per pair, with P = pairs_per_sample (8..64) and S = n_samples (>= 1):
+ *    count < P: out_best = -2 (upstream throws, :29-32), inliers 0, F zeros, mask slots 0.
+ *    Hypothesis s draws P distinct indices in [0, count) with Floyd's algorithm, sorted ascending afterwards.  Draw t
+ *    (t = 0..P-1, j = count - P + t) is r = (u * (j + 1)) >> 32 with the 32-bit
+ *        u = splitmix64(key ^ ((uint64)s << 32 | t)) >> 32,   key = splitmix64(seed ^ splitmix64((uint64)(uint32)a << 32 | (uint32)b)),
+ *        splitmix64(z): z += 0x9E3779B97F4A7C15; z = (z ^ z >> 30) * 0xBF58476D1CE4E5B9; z = (z ^ z >> 27) * 0x94D049BB133111EB;
+ *                       return z ^ z >> 31;
+ *    Floyd: if r is already drawn, j is taken instead.  The key depends on the image pair, not on its position in the list.
+ *    Estimate: centroids in double rounded to float32, c = fl32(x - cx), rows of A = float32 (c1x c2x, c1x c2y, c1x,
+ *    c1y c2x, c1y c2y, c1y, c2x, c2y, 1); the null vector v of A in fp64 (Givens QR, one-sided Jacobi), its largest-
+ *    magnitude component positive (lowest index on exact ties; components equal up to rounding, as in the skew-symmetric
+ *    F of a pure translation, are ordered by the fp64 result); F0[i][j] = v[3 j + i]; F = T2^T F0 T1 in fp64, rounded once to
+ *    float32 (row-major).  With PGM_FLAG_RANSAC_RANK_TEST a hypothesis is skipped (count -1) unless #{sigma_k > 3
+ *    ulp_f32(sigma_0)} == 2, sigma the fp64 singular values of the float32 F (:46-51).  Scoring as pgm_ransac_score.
+ *    out_best = the first s with the largest positive count, else -1 (upstream throws, :87-88); out_inliers and
+ *    out_F (float32[n_pairs][9]) are the winner's (0 and zeros without one); d_out_mask = 1 at the winner's inlier slots,
+ *    0 at the pair's other slots.  No slot outside a pair's [start, start + count) is written.
+ *  - d_hyp_F (float[n_pairs][S][9]) and d_hyp_counts (int32[n_pairs][S]) are optional diagnostics (NULL in production):
+ *    every hypothesis' F and count (-1 if skipped); a pair with count < P leaves its rows unwritten.
+ *  - PGM_E_INVALID_ARG: P outside 8..64, S < 1, unknown flags, a bad pair or image index, a null pointer, a negative
+ *    count, start < 0, start + count > capacity, matches of an empty image. */
+#define PGM_FLAG_RANSAC_RANK_TEST 0x4u   /* apply upstream's rank gate (CameraPoseEstimation.cs:46-51) */
+int pgm_ransac_fundamental_pairs_batch_dev(pgm_handle *h,
+        const int32_t *d_all_xy, const int64_t *image_offsets, int32_t n_images,
+        const int32_t *pair_list, int32_t n_pairs,
+        const int32_t *d_match_qi, const int32_t *d_match_tj,
+        const int64_t *match_starts, const int32_t *match_counts,
+        int32_t n_samples, int32_t pairs_per_sample, float threshold, uint64_t seed, uint32_t flags,
+        int32_t *d_out_best, int32_t *d_out_inliers, float *d_out_F,
+        uint8_t *d_out_mask, int64_t capacity,
+        float *d_hyp_F, int32_t *d_hyp_counts);
+
 /* Nearest neighbour + ratio test + mutual cross-check (+ optional distance bound) for MANY small pairs in one launch --
  * the consecutive frames of a sequence (BASELINE configs[2]; per pair the same result as pgm_match_ratio_crosscheck, which
  * extends the nearest-neighbour-within-a-threshold use of python_src/scripts/match_keypoints.py:112-134).  Layout as for

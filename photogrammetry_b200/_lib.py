@@ -26,6 +26,7 @@ PGM_E_NOMEM = -6
 PGM_E_NO_DEVICE = -7
 PGM_FLAG_REFERENCE_COMPAT_TAIL = 0x1
 PGM_FLAG_PYTHON_GENERATION = 0x2
+PGM_FLAG_RANSAC_RANK_TEST = 0x4
 PGM_TAIL_DISTANCE = 2147483647
 
 # every symbol include/pgmatch.h declares (tests check the .so exports them all)
@@ -39,7 +40,7 @@ EXPORTED_SYMBOLS = (
     "pgm_match_keypoints_sorted", "pgm_match_keypoints_sorted_dev", "pgm_knn2_l2", "pgm_knn2_l2_dev", "pgm_l2_last_fallback_rows",
     "pgm_knn2_l2_pairs_batch_dev", "pgm_match_l2_ratio_crosscheck_pairs_batch_dev",
     "pgm_fast_detect", "pgm_brief_describe", "pgm_nms", "pgm_detect_describe_dev", "pgm_detect_describe_batch_dev",
-    "pgm_ransac_score",
+    "pgm_ransac_score", "pgm_ransac_fundamental_pairs_batch_dev",
     "pgm_shard_create", "pgm_shard_edge_capacity", "pgm_shard_round", "pgm_shard_commit", "pgm_shard_finish_round",
     "pgm_shard_finish", "pgm_shard_destroy",
     "pgm_multi_unique_id", "pgm_multi_create", "pgm_multi_destroy", "pgm_multi_match_train_sharded_dev",
@@ -161,6 +162,9 @@ def load() -> C.CDLL:
                                                       i32p]
         lib.pgm_ransac_score.argtypes = [C.c_void_p, vp, u8p, C.c_int32, i32p, i32p, C.c_int32, C.c_float, i32p,
                                          C.POINTER(C.c_int32), u8p]
+        lib.pgm_ransac_fundamental_pairs_batch_dev.argtypes = [C.c_void_p, i32p, i64p, C.c_int32, i32p, C.c_int32, i32p, i32p,
+                                                               i64p, i32p, C.c_int32, C.c_int32, C.c_float, C.c_uint64,
+                                                               C.c_uint32, i32p, i32p, vp, u8p, C.c_int64, vp, i32p]
         lib.pgm_shard_create.argtypes = [C.c_void_p, u8p, C.c_int32, u8p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                          C.c_int32, C.POINTER(C.c_void_p)]
         lib.pgm_shard_round.argtypes = [C.c_void_p, C.c_void_p, C.c_int32]

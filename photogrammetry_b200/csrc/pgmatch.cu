@@ -2430,6 +2430,105 @@ extern "C" int pgm_ransac_score(pgm_handle *h, const float *F, const uint8_t *va
     return PGM_OK;
 }
 
+// Many match lists in one call: the hypotheses of the pairs with count >= P form one flattened space g = k S + s
+// (k = the k-th such pair), cut into chunks of RB_CHUNK_HYPS whose F and rank flags reuse one scratch area.  The host
+// plans every chunk from host arrays and uploads the plan in one copy; nothing is read back.
+constexpr int64_t RB_CHUNK_HYPS = 1ll << 20;
+
+extern "C" int pgm_ransac_fundamental_pairs_batch_dev(pgm_handle *h, const int32_t *d_all_xy, const int64_t *image_offsets,
+        int32_t n_images, const int32_t *pair_list, int32_t n_pairs, const int32_t *d_match_qi, const int32_t *d_match_tj,
+        const int64_t *match_starts, const int32_t *match_counts, int32_t n_samples, int32_t pairs_per_sample,
+        float threshold, uint64_t seed, uint32_t flags, int32_t *d_out_best, int32_t *d_out_inliers, float *d_out_F,
+        uint8_t *d_out_mask, int64_t capacity, float *d_hyp_F, int32_t *d_hyp_counts) {
+    using namespace pgm_ransac;
+    if (!h) return PGM_E_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    h->stats = pgm_stats{};
+    h->stats_pending = false;
+    const int P = pairs_per_sample;
+    const int64_t S = n_samples;
+    if (P < 8 || P > RB_MAX_P || S < 1 || n_pairs < 0 || n_images < 0 || capacity < 0 || (flags & ~PGM_FLAG_RANSAC_RANK_TEST))
+        return fail(h, PGM_E_INVALID_ARG, "bad n_samples, pairs_per_sample, sizes or flags");
+    if (n_pairs == 0) return PGM_OK;
+    if (!image_offsets || !pair_list || !match_starts || !match_counts || !d_all_xy || !d_match_qi || !d_match_tj ||
+        !d_out_best || !d_out_inliers || !d_out_F || !d_out_mask)
+        return fail(h, PGM_E_INVALID_ARG, "null pointer");
+    std::vector<RbPair> plan(n_pairs);
+    std::vector<int32_t> act;
+    for (int p = 0; p < n_pairs; p++) {
+        const int a = pair_list[2 * p], b = pair_list[2 * p + 1];
+        if (a < 0 || a >= n_images || b < 0 || b >= n_images) return fail(h, PGM_E_INVALID_ARG, "pair index out of range");
+        const int64_t oa = image_offsets[a], ob = image_offsets[b];
+        const int64_t na = image_offsets[a + 1] - oa, nb = image_offsets[b + 1] - ob;
+        if (oa < 0 || ob < 0 || na < 0 || nb < 0 || na > INT32_MAX || nb > INT32_MAX) return fail(h, PGM_E_INVALID_ARG, "bad image offsets");
+        const int64_t st = match_starts[p];
+        const int32_t cnt = match_counts[p];
+        if (cnt < 0 || st < 0 || st + cnt > capacity) return fail(h, PGM_E_INVALID_ARG, "match slots outside [0, capacity)");
+        if (cnt > 0 && (na == 0 || nb == 0)) return fail(h, PGM_E_INVALID_ARG, "matches of an empty image");
+        plan[p] = RbPair{st, oa, ob, cnt, a, b, (int32_t)na, (int32_t)nb, 0};
+        if (cnt >= P) act.push_back(p);
+    }
+    // chunks of the flattened hypothesis space; item_base: per chunk, the score items' prefix over its pairs
+    struct Chunk { int64_t g0, g1, k0; int n_local, base_off, items; };
+    std::vector<Chunk> chunks;
+    std::vector<int32_t> bases;
+    const int64_t total = (int64_t)act.size() * S;
+    for (int64_t g0 = 0; g0 < total; g0 += RB_CHUNK_HYPS) {
+        const int64_t g1 = std::min(total, g0 + RB_CHUNK_HYPS);
+        Chunk c{g0, g1, g0 / S, 0, (int)bases.size(), 0};
+        for (int64_t k = c.k0; k * S < g1; k++) {
+            const int64_t len = std::min(g1, (k + 1) * S) - std::max(g0, k * S);
+            bases.push_back(c.items);
+            c.items += (int)((len + RB_SCORE_THREADS - 1) / RB_SCORE_THREADS);
+            c.n_local++;
+        }
+        bases.push_back(c.items);
+        chunks.push_back(c);
+    }
+    const int64_t hyps = std::min<int64_t>(std::max<int64_t>(total, 1), RB_CHUNK_HYPS);
+    // h->misc: plan | active pairs | item bases | keys | chunk F | chunk rank flags
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + std::max<size_t>(bytes, 1), 256); return o; };
+    const size_t o_plan = take(sizeof(RbPair) * plan.size()), o_act = take(4 * act.size()), o_bases = take(4 * bases.size());
+    const size_t upload = off;
+    const size_t o_keys = take(8 * (size_t)n_pairs), o_F = take((size_t)hyps * 36), o_v = take((size_t)hyps);
+    int rc = ensure_dev(h, h->misc, off);
+    if (rc) return rc;
+    CU_CHECK(h, cudaSetDevice(h->device));
+    cudaStream_t s = h->stream;
+    std::vector<char> host(upload);
+    memcpy(host.data() + o_plan, plan.data(), sizeof(RbPair) * plan.size());
+    if (!act.empty()) memcpy(host.data() + o_act, act.data(), 4 * act.size());
+    memcpy(host.data() + o_bases, bases.data(), 4 * bases.size());
+    char *dev = (char *)h->misc.p;
+    // pageable source: the runtime stages it before returning, so the vector may go; no stream synchronisation
+    CU_CHECK(h, cudaMemcpyAsync(dev, host.data(), upload, cudaMemcpyHostToDevice, s));
+    CU_CHECK(h, cudaMemsetAsync(dev + o_keys, 0, 8 * (size_t)n_pairs, s));
+    const RbPair *d_plan = (const RbPair *)(dev + o_plan);
+    const int32_t *d_act = (const int32_t *)(dev + o_act), *d_bases = (const int32_t *)(dev + o_bases);
+    unsigned long long *d_keys = (unsigned long long *)(dev + o_keys);
+    float *d_F = (float *)(dev + o_F);
+    uint8_t *d_v = (uint8_t *)(dev + o_v);
+    const int rank_test = (flags & PGM_FLAG_RANSAC_RANK_TEST) ? 1 : 0;
+    for (const Chunk &c : chunks) {
+        const unsigned grid = (unsigned)((c.g1 - c.g0 + RB_EST_THREADS - 1) / RB_EST_THREADS);
+        estimate_kernel<<<grid, RB_EST_THREADS, RB_EST_THREADS * RB_SM_DOUBLES * sizeof(double), s>>>(
+            d_plan, d_act, S, c.g0, c.g1, d_all_xy, d_match_qi, d_match_tj, P, seed, rank_test, d_F, d_v, d_hyp_F);
+        pairs_score_kernel<<<c.items, RB_SCORE_THREADS, 0, s>>>(d_plan, d_act, d_bases + c.base_off, c.n_local, c.k0, S,
+                                                                 c.g0, c.g1, d_F, d_v, d_all_xy, d_match_qi, d_match_tj,
+                                                                 threshold, d_keys, d_hyp_counts);
+        CU_CHECK(h, cudaGetLastError());
+        h->stats.kernel_launches += 2;
+    }
+    winner_kernel<<<n_pairs, RB_WIN_THREADS, 0, s>>>(d_plan, P, seed, d_keys, d_all_xy, d_match_qi, d_match_tj, threshold,
+                                                     d_out_best, d_out_inliers, d_out_F, d_out_mask);
+    CU_CHECK(h, cudaGetLastError());
+    h->stats.kernel_launches += 1;
+    h->stats.pairs = n_pairs;
+    h->stats.h2d_bytes = (int64_t)upload;
+    return PGM_OK;
+}
+
 // ---------------------------------------------------------------------------
 // train-sharded single pair (BASELINE configs[3]).  Two surfaces over the same kernels:
 //   pgm_shard_*   stepwise: the ONE exchange per round (element-wise min of X over the ranks) belongs to the caller

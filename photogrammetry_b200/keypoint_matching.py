@@ -519,6 +519,53 @@ class Matcher:
                                                float(threshold), counts.ctypes.data, C.byref(best), mask.ctypes.data))
         return counts[:len(F)], int(best.value), mask[:len(xy1)]
 
+    def ransac_fundamental_pairs_batch_dev(self, d_xy, image_offsets, pair_list, qi, tj, starts, counts,
+                                           n_samples: int = 2000, pairs_per_sample: int = 32, threshold: float = 0.001,
+                                           seed: int = 0, require_rank2: bool = True, hypotheses: bool = False):
+        """``GetFundamentalMatrix(list, n_samples, pairs_per_sample, threshold)`` (CameraPoseEstimation.cs:26-94) for
+        many match lists in one call, on the device and with no read-back.  The defaults are upstream's call
+        (Program.cs: 2000, 32, 0.001f) and the host mirror's rank gate.
+
+        ``d_xy``: torch int32 ``[rows, 2]`` keypoint coordinates, image ``k`` at rows ``image_offsets[k]:image_offsets[k+1]``;
+        ``qi``/``tj``: torch int32 match indices (e.g. rows 0 and 1 of what the batch matchers return) with ``starts`` /
+        ``counts`` as those methods return them.  Returns torch tensors ``(best int32[n_pairs], inliers int32[n_pairs],
+        F float32[n_pairs, 3, 3], mask uint8[capacity])`` -- ``best`` is the winning sample, -1 if no sample has an inlier,
+        -2 if the pair has fewer than ``pairs_per_sample`` matches -- plus ``(hyp_F float32[n_pairs, S, 3, 3],
+        hyp_counts int32[n_pairs, S])`` with ``hypotheses=True`` (rows of pairs below ``pairs_per_sample`` stay zero)."""
+        import torch
+        offs = np.ascontiguousarray(image_offsets, dtype=np.int64)
+        pairs = np.ascontiguousarray(pair_list, dtype=np.int32).reshape(-1, 2)
+        st = np.ascontiguousarray(starts, dtype=np.int64).reshape(-1)
+        cn = np.ascontiguousarray(counts, dtype=np.int32).reshape(-1)
+        n_pairs = len(pairs)
+        if len(st) != n_pairs or len(cn) != n_pairs:
+            raise ValueError("starts and counts need one entry per pair")
+        for name, t in (("d_xy", d_xy), ("qi", qi), ("tj", tj)):
+            if t.dtype != torch.int32 or not t.is_contiguous():
+                raise ValueError(f"{name} must be a contiguous int32 tensor")
+        capacity = min(int(qi.numel()), int(tj.numel()))
+        dev = d_xy.device
+        S = int(n_samples)
+        best = torch.empty(max(n_pairs, 1), dtype=torch.int32, device=dev)
+        inliers = torch.empty(max(n_pairs, 1), dtype=torch.int32, device=dev)
+        F = torch.empty((max(n_pairs, 1), 3, 3), dtype=torch.float32, device=dev)
+        mask = torch.zeros(max(capacity, 1), dtype=torch.uint8, device=dev)
+        hyp_F = hyp_c = None
+        if hypotheses:
+            hyp_F = torch.zeros((max(n_pairs, 1), max(S, 1), 3, 3), dtype=torch.float32, device=dev)
+            hyp_c = torch.zeros((max(n_pairs, 1), max(S, 1)), dtype=torch.int32, device=dev)
+        flags = _lib.PGM_FLAG_RANSAC_RANK_TEST if require_rank2 else 0
+        with self.torch_ordered(dev):
+            self._check(self._lib.pgm_ransac_fundamental_pairs_batch_dev(
+                self._h, d_xy.data_ptr(), offs.ctypes.data, len(offs) - 1, pairs.ctypes.data, n_pairs, qi.data_ptr(),
+                tj.data_ptr(), st.ctypes.data, cn.ctypes.data, S, int(pairs_per_sample), float(threshold),
+                int(seed) & 0xFFFFFFFFFFFFFFFF, flags, best.data_ptr(), inliers.data_ptr(), F.data_ptr(), mask.data_ptr(),
+                capacity, hyp_F.data_ptr() if hypotheses else None, hyp_c.data_ptr() if hypotheses else None))
+        out = (best[:n_pairs], inliers[:n_pairs], F[:n_pairs], mask[:capacity])
+        if hypotheses:
+            out += (hyp_F[:n_pairs], hyp_c[:n_pairs])
+        return out
+
     def set_profiling(self, enabled: bool) -> None:
         self._check(self._lib.pgm_set_profiling(self._h, int(bool(enabled))))
 

@@ -93,3 +93,45 @@ def config2_pair(n: int = 8192, dist: str = "U", desc_bits: int = 256):
         q = uniform_descriptors(1234, n, desc_bits)
         return q, noisy_copy_descriptors(42, q, desc_bits)
     raise ValueError(f"unknown distribution {dist!r}")
+
+
+def two_view_matches(seed: int, n_pairs: int, per_pair: int = 512, outlier_frac: float = 0.3, size: int = 4000):
+    """Match lists for the batched fundamental-matrix RANSAC: pair k = images (2k, 2k + 1), each with ``per_pair``
+    keypoints that are projections of one set of 3D points by two pinhole cameras (focal length ``size / 2``, principal
+    point at the image centre, second camera rotated by up to 0.1 rad and translated), rounded to pixels and clipped to
+    ``[0, size)``.  Match i joins keypoint i of image 2k with the same point's keypoint of image 2k + 1 (stored in a
+    permuted row order); a fraction ``outlier_frac`` of the matches points at a random keypoint instead.
+
+    Returns ``(xy int32[2 n_pairs per_pair, 2], image_offsets int64, pair_list int32[n_pairs, 2], qi int32, tj int32,
+    starts int64[n_pairs], counts int32[n_pairs])``: the layout the batch matchers produce."""
+    rng = np.random.default_rng(seed)
+    m = int(per_pair)
+    X = np.stack([rng.uniform(-1, 1, (n_pairs, m)), rng.uniform(-1, 1, (n_pairs, m)), rng.uniform(4, 8, (n_pairs, m))], -1)
+    ang = rng.uniform(-0.1, 0.1, (n_pairs, 3))
+    cx, sx = np.cos(ang[:, 0]), np.sin(ang[:, 0])
+    cy, sy = np.cos(ang[:, 1]), np.sin(ang[:, 1])
+    cz, sz = np.cos(ang[:, 2]), np.sin(ang[:, 2])
+    one, zero = np.ones(n_pairs), np.zeros(n_pairs)
+    Rx = np.stack([one, zero, zero, zero, cx, -sx, zero, sx, cx], -1).reshape(-1, 3, 3)
+    Ry = np.stack([cy, zero, sy, zero, one, zero, -sy, zero, cy], -1).reshape(-1, 3, 3)
+    Rz = np.stack([cz, -sz, zero, sz, cz, zero, zero, zero, one], -1).reshape(-1, 3, 3)
+    R = Rz @ Ry @ Rx
+    t = rng.uniform(-0.5, 0.5, (n_pairs, 1, 3))
+    f, c = size / 2.0, size / 2.0
+
+    def project(P):
+        return np.clip(np.rint(f * P[..., :2] / P[..., 2:3] + c), 0, size - 1).astype(np.int32)
+    x1 = project(X)
+    x2 = project(np.einsum("kij,kmj->kmi", R, X) + t)
+    perm = rng.permuted(np.tile(np.arange(m), (n_pairs, 1)), axis=1)          # row of point i in image 2k + 1
+    img2 = np.empty_like(x2)
+    np.put_along_axis(img2, perm[..., None], x2, axis=1)
+    tj = perm.copy()
+    out = rng.random((n_pairs, m)) < outlier_frac
+    tj[out] = rng.integers(0, m, size=int(out.sum()))
+    xy = np.stack([x1, img2], axis=1).reshape(-1, 2)
+    offs = np.arange(2 * n_pairs + 1, dtype=np.int64) * m
+    pairs = np.stack([np.arange(n_pairs) * 2, np.arange(n_pairs) * 2 + 1], -1).astype(np.int32)
+    qi = np.tile(np.arange(m, dtype=np.int32), n_pairs)
+    return (np.ascontiguousarray(xy), offs, pairs, qi, tj.reshape(-1).astype(np.int32),
+            np.arange(n_pairs, dtype=np.int64) * m, np.full(n_pairs, m, dtype=np.int32))

@@ -13,6 +13,8 @@
   7. float L2 batch of 6 pairs: one large pair whose row pairs span several segments (split candidate slots), flagged
      rows in two pairs (crowded band, identical train rows) taken by the batched fallback, then the ratio + cross-check
      filter with its reversed pairs and ordered compaction
+  8. batched fundamental-matrix RANSAC of 6 pairs: one below P, a degenerate one (every keypoint the same pixel), one of
+     20 000 matches (several shared-memory tiles per score CTA), S spread over two score items per pair
 Every result is checked against the oracle, so a sanitizer run is also a parity run."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -88,5 +90,26 @@ for p, (a, b) in enumerate(pairs):
     assert (tj[starts[p]:starts[p] + counts[p]] == bj[keep]).all() and (dist[starts[p]:starts[p] + counts[p]] == bd[keep]).all()
     o += n1; ro += n2
 print("case 7 ok", m.stats())
+from oracle import ransac_batch_np as R
+xy, offs, pl, qi, tj, st, cn = synthetic.two_view_matches(11, 4, 400)
+big = synthetic.two_view_matches(12, 1, 20000)
+n_img = len(offs) - 1
+xy = np.concatenate([xy, big[0], np.full((60, 2), (321, 654), np.int32)])
+offs = np.concatenate([offs, offs[-1] + big[1][1:], [offs[-1] + big[1][-1] + 60]]).astype(np.int64)
+pl = np.concatenate([pl, big[2] + n_img, [[n_img + 2, n_img + 2]]]).astype(np.int32)
+qi = np.concatenate([qi, big[3], np.arange(60, dtype=np.int32)])
+tj = np.concatenate([tj, big[4], np.arange(60, dtype=np.int32)])
+st = np.concatenate([st, [len(st) * 400], [len(st) * 400 + 20000]]).astype(np.int64)
+cn = np.concatenate([cn, [20000], [60]]).astype(np.int32)
+cn[1] = 31                                                  # below P
+d_xy, d_qi, d_tj = (torch.from_numpy(x).cuda() for x in (xy, qi, tj))
+best, inl, F, mask = (x.cpu().numpy() for x in m.ransac_fundamental_pairs_batch_dev(
+    d_xy, offs, pl, d_qi, d_tj, st, cn, n_samples=200, pairs_per_sample=32, threshold=0.001, seed=4, require_rank2=False))
+exp = R.get_fundamental_pairs(xy, offs, pl, qi, tj, st, cn, 200, 32, 0.001, 4, require_rank2=False)
+for p, (eb, ei, eF, em, _, _) in enumerate(exp):
+    assert best[p] == eb and inl[p] == ei and (mask[st[p]:st[p] + cn[p]] == em).all(), p
+    assert np.abs(F[p].astype(np.float64) - eF).max() <= 1e-6 * max(np.abs(eF).max(), 1e-30), p
+assert best[1] == -2 and np.isfinite(F).all()
+print("case 8 ok", m.stats())
 m.close()
 print("ALL OK")
