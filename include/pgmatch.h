@@ -329,11 +329,34 @@ int pgm_detect_describe_dev(pgm_handle *h, const float *d_gray, int32_t width, i
  * d_out_xy[n_images][capacity][2], d_out_score[n_images][capacity], d_out_desc[n_images][capacity][stride_bytes] --
  * and its keypoint count to d_out_counts[k] (device); a count above `capacity` means the list was truncated.
  * Nothing is read back between the images: the call enqueues six kernels for the whole batch.  out_counts
- * (host, int32[n_images]) may be NULL, in which case the call does not synchronise at all.  No NMS in this form. */
+ * (host, int32[n_images]) may be NULL, in which case the call does not synchronise at all.  No NMS in this form:
+ * pgm_detect_nms_describe_batch_dev below is the batched chain with it. */
 int pgm_detect_describe_batch_dev(pgm_handle *h, const float *d_gray, int32_t n_images, int32_t width, int32_t height,
                                   float threshold, const int32_t *pairs, int32_t n_pairs, int32_t stride_bytes,
                                   uint32_t flags, int32_t *d_out_xy, int32_t *d_out_score, uint8_t *d_out_desc,
                                   int32_t capacity, int32_t *d_out_counts, int32_t *out_counts);
+
+/* The batched form WITH non-maximum suppression: FAST-12 -> RedundantKeypointEliminator (radius nms_radius >= 0)
+ * -> BRIEF of the survivors, for n_images device-resident images of one size (the C# pipeline's per-frame chain,
+ * BuildKeypointDetectorPipeline, whose denoised keypoints TestService.cs:94-95 matches).  Arguments and output layout
+ * are those of pgm_detect_describe_batch_dev, plus nms_radius.
+ *  - For every image k and both generations the result equals pgm_detect_describe_dev(image k, threshold,
+ *    nms_radius, ...) bit for bit: survivors' (x, y), FastScore and descriptor bytes, in the reference's output
+ *    order (stable by FastScore descending).  NMS always runs over the image's full FAST list.
+ *  - d_out_counts[k] (device) = the number of survivors of image k.  A count above `capacity` means only the first
+ *    `capacity` survivors were written.  No slot at or beyond min(count, capacity) of an image is written.
+ *    out_counts (host, int32[n_images]) may be NULL.
+ *  - Synchronisation: one, the read-back of the per-image FAST totals that sizes the scratch (host_syncs = 1, 2 with
+ *    out_counts).  Every NMS round of every image runs on the device; the number of kernel launches depends neither
+ *    on the rounds nor on n_images.
+ *  - Refusals: PGM_E_INVALID_ARG for nms_radius < 0 (use pgm_detect_describe_batch_dev without NMS) and for every
+ *    argument pgm_detect_describe_batch_dev refuses; PGM_E_CAPACITY when the batch's FAST keypoints together exceed
+ *    2^31 - 1, after the read-back and before any later kernel runs.  n_images == 0 does nothing. */
+int pgm_detect_nms_describe_batch_dev(pgm_handle *h, const float *d_gray, int32_t n_images, int32_t width,
+                                      int32_t height, float threshold, int32_t nms_radius, const int32_t *pairs,
+                                      int32_t n_pairs, int32_t stride_bytes, uint32_t flags, int32_t *d_out_xy,
+                                      int32_t *d_out_score, uint8_t *d_out_desc, int32_t capacity,
+                                      int32_t *d_out_counts, int32_t *out_counts);
 
 /* ---- the consumer of the match list (SURVEY.md section 8, row f3) --------------------
  * pgm_ransac_score: the scoring loops of CameraPoseEstimation.GetFundamentalMatrix

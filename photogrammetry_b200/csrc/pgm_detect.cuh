@@ -14,6 +14,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "pgm_kernels.cuh"   // PGM_ASSERT, grid_barrier
+
 namespace pgm_det {
 
 // Ring tables as (dx, dy).  [0] = KeypointDetection.cs:15-19; entry 15 is upstream's typo ({-3, 1} twice), kept.
@@ -130,13 +132,15 @@ __global__ void emit_kernel(const uint8_t *__restrict__ score, int w, int h, con
 // (`descriptor <<= 1` per pair, first pair = MSB), stored little-endian in `stride` bytes.
 __global__ void brief_kernel(const float *__restrict__ img, int w, int h, const int32_t *__restrict__ xy, int n,
                              const int32_t *__restrict__ pairs /*[n_pairs][4]*/, int n_pairs, int stride_words,
-                             int lsb_first, uint32_t *__restrict__ desc, const int32_t *__restrict__ rowoff = nullptr) {
+                             int lsb_first, uint32_t *__restrict__ desc, const int32_t *__restrict__ rowoff = nullptr,
+                             const int32_t *__restrict__ counts = nullptr) {
     extern __shared__ uint32_t s_desc[];           // [warps][stride_words]
     const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int i = blockIdx.x * (blockDim.x >> 5) + wid;
-    if (rowoff) {                                  // batched form: blockIdx.y = image, n = capacity per image, and the
-        const int z = blockIdx.y;                  // image's keypoint count sits behind its row offsets on the device
-        const int found = __ldg(rowoff + (size_t)z * (h + 1) + h);
+    if (rowoff || counts) {                        // batched form: blockIdx.y = image, n = capacity per image, and the
+        const int z = blockIdx.y;                  // image's keypoint count sits on the device: behind its row offsets,
+                                                   // or in counts[z] (the survivors of the batched NMS)
+        const int found = counts ? __ldg(counts + z) : __ldg(rowoff + (size_t)z * (h + 1) + h);
         img += (size_t)z * w * h; xy += (size_t)z * n * 2; desc += (size_t)z * n * stride_words;
         n = min(n, found);
     }
@@ -325,6 +329,160 @@ __global__ void nms_emit_kernel(const int32_t *__restrict__ order, const uint8_t
         __syncthreads();
     }
     if (tid == 0) *n_kept = s_base;
+}
+
+// ---- batched NMS: many images, every round on the device (pgm_detect_nms_describe_batch_dev) ---------------
+// All images' FAST lists sit in one flat list, image z's at base[z] .. base[z + 1].  The rounds are those of
+// nms_round_binned_kernel, run for every image at once by one persistent kernel; nothing is read back per round.
+constexpr int NMS_BATCH_THREADS = 256;
+constexpr int NMS_EMIT_THREADS = 1024;
+constexpr int NMS_RANK_IMAGE_SHIFT = 40;   // rank key: image << 40 | (255 - score) << 32 | index within the image
+
+// Control words of the rounds kernel, zeroed before its launch.
+struct NmsBatchCtl {
+    int32_t undecided[3];   // round r counts into [r % 3]; see nms_rounds_batch_kernel
+    uint32_t grid_bar;      // grid_barrier counter
+    int32_t final_buf;      // which state buffer holds the final states (written at exit)
+};
+
+// Detect's row-major list of every image (one warp per row, ballot prefix, as emit_kernel) into the flat list at the
+// image's base, with each keypoint's rank key, its cell id (cells of side cs over [0, w) x [0, h), image-major) and
+// its own flat index (the values of the cell sort).
+__global__ void nms_batch_emit_kernel(const uint8_t *__restrict__ score, int w, int h, const int32_t *__restrict__ rowoff,
+                                      const int32_t *__restrict__ base, int cs, int ncx, int ncy,
+                                      int32_t *__restrict__ xy, int32_t *__restrict__ sc,
+                                      unsigned long long *__restrict__ rank_key, unsigned long long *__restrict__ cell,
+                                      int32_t *__restrict__ idx) {
+    const int y = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (y >= h) return;
+    const int z = blockIdx.y;
+    score += (size_t)z * w * h; rowoff += (size_t)z * (h + 1);
+    const int b0 = __ldg(base + z), n_img = __ldg(base + z + 1) - b0;
+    const unsigned long long row_cell = ((unsigned long long)z * ncy + y / cs) * ncx;
+    int local = rowoff[y];
+    for (int x0 = 0; x0 < w; x0 += 32) {
+        const int x = x0 + lane;
+        const uint8_t v = x < w ? score[(size_t)y * w + x] : 0;
+        const unsigned m = __ballot_sync(0xffffffffu, v != 0);
+        if (v) {
+            const int li = local + __popc(m & ((1u << lane) - 1u));
+            PGM_ASSERT(li >= 0 && li < n_img);
+            const int i = b0 + li;
+            xy[2 * (size_t)i] = x; xy[2 * (size_t)i + 1] = y; sc[i] = v;
+            rank_key[i] = ((unsigned long long)z << NMS_RANK_IMAGE_SHIFT) | ((unsigned long long)(255u - v) << 32) | (unsigned)li;
+            cell[i] = row_cell + (unsigned)(x / cs);
+            idx[i] = i;
+        }
+        local += __popc(m);
+    }
+}
+
+// order[r] = flat index of rank r, rank[order[r]] = r.  The key sorts by image first, so image z's ranks are exactly
+// base[z] .. base[z + 1] - 1, in LINQ's stable order by score descending.
+__global__ void nms_batch_order_kernel(const unsigned long long *__restrict__ sorted_key, int n, const int32_t *__restrict__ base,
+                                       int n_images, int32_t *__restrict__ order, int32_t *__restrict__ rank) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n) return;
+    const unsigned long long key = sorted_key[r];
+    const int z = (int)(key >> NMS_RANK_IMAGE_SHIFT), li = (int)(unsigned)key;
+    PGM_ASSERT(z >= 0 && z < n_images && li >= 0 && li < base[z + 1] - base[z]);
+    const int i = base[z] + li;
+    PGM_ASSERT(r >= base[z] && r < base[z + 1]);
+    order[r] = i; rank[i] = r;
+}
+
+// Every round of every image in one cooperative launch.  Round r applies nms_round_binned_kernel's rule to every
+// undecided keypoint (state: 0 undecided, 1 kept, 2 dropped; read from st[r & 1], written to st[(r + 1) & 1]) and
+// counts the keypoints it leaves undecided into ctl->undecided[r % 3].  Thread 0 zeroes the next round's counter
+// during round r; three counters, because with two the zeroing in round r + 1 would race with a late warp still
+// reading round r's count after the barrier.  Each round decides at least the best-ranked undecided keypoint of every
+// image that has one, so the rounds end after at most n of them.
+__global__ void __launch_bounds__(NMS_BATCH_THREADS) nms_rounds_batch_kernel(
+        const int32_t *__restrict__ xy, const int32_t *__restrict__ rank, int n, long long radius2, int cs, int ncx,
+        int ncy, const unsigned long long *__restrict__ cell, const unsigned long long *__restrict__ sorted_cell,
+        const int32_t *__restrict__ sorted_idx, uint8_t *st0, uint8_t *st1, NmsBatchCtl *ctl) {
+    const int gt = blockIdx.x * blockDim.x + threadIdx.x, gs = gridDim.x * blockDim.x;
+    unsigned epoch = 0;
+    for (int round = 0; round < n; round++) {      // (the bound is never reached, see above)
+        const uint8_t *st_in = (round & 1) ? st1 : st0;
+        uint8_t *st_out = (round & 1) ? st0 : st1;
+        int undecided = 0;
+        for (int i = gt; i < n; i += gs) {
+            const uint8_t st = __ldcg(st_in + i);
+            if (st != 0) { st_out[i] = st; continue; }
+            const int x = __ldg(xy + 2 * i), y = __ldg(xy + 2 * i + 1), r = __ldg(rank + i);
+            const int cx = x / cs, cy = y / cs;
+            const long long c = (long long)__ldg(cell + i);
+            bool any_kept = false, any_undecided = false;
+            for (int dy = -1; dy <= 1 && !any_kept; dy++) {
+                if (cy + dy < 0 || cy + dy >= ncy) continue;
+                // the three cells (cx-1 .. cx+1) of one cell row of this image are consecutive ids: one search, one run
+                const long long row = c - cx + (long long)dy * ncx;
+                const unsigned long long c0 = (unsigned long long)(row + max(cx - 1, 0));
+                const unsigned long long c1 = (unsigned long long)(row + min(cx + 1, ncx - 1));
+                for (int k = lower_bound_u64(sorted_cell, n, c0); k < n && __ldg(sorted_cell + k) <= c1; k++) {
+                    const int j = __ldg(sorted_idx + k);
+                    PGM_ASSERT(j >= 0 && j < n);
+                    if (__ldg(rank + j) >= r) continue;
+                    const uint8_t sj = __ldcg(st_in + j);
+                    if (sj == 2) continue;
+                    const long long ddx = (long long)__ldg(xy + 2 * j) - x, ddy = (long long)__ldg(xy + 2 * j + 1) - y;
+                    if (ddx * ddx + ddy * ddy > radius2) continue;       // IsAcceptableDistance: distance > radius survives
+                    if (sj == 1) { any_kept = true; break; }
+                    any_undecided = true;
+                }
+            }
+            const uint8_t ns = any_kept ? 2 : (any_undecided ? 0 : 1);
+            st_out[i] = ns;
+            undecided += ns == 0;
+        }
+        undecided = __reduce_add_sync(0xffffffffu, undecided);
+        if ((threadIdx.x & 31) == 0 && undecided) atomicAdd(&ctl->undecided[round % 3], undecided);
+        if (gt == 0) ctl->undecided[(round + 1) % 3] = 0;
+        pgm::grid_barrier(&ctl->grid_bar, gridDim.x, epoch);
+        if (__ldcg(&ctl->undecided[round % 3]) == 0) {                        // uniform over the grid
+            if (gt == 0) ctl->final_buf = (round + 1) & 1;
+            return;
+        }
+    }
+    PGM_ASSERT(false);
+}
+
+// One CTA per image: the kept keypoints of its rank-ordered run (ballot prefixes, as nms_emit_kernel) into the image's
+// `capacity` output slots, in the reference's output order; counts[z] = all survivors, also those beyond capacity.
+__global__ void __launch_bounds__(NMS_EMIT_THREADS) nms_batch_gather_kernel(
+        const int32_t *__restrict__ order, const int32_t *__restrict__ base, const uint8_t *__restrict__ st0,
+        const uint8_t *__restrict__ st1, const NmsBatchCtl *__restrict__ ctl, const int32_t *__restrict__ xy,
+        const int32_t *__restrict__ sc, int capacity, int32_t *__restrict__ out_xy, int32_t *__restrict__ out_sc,
+        int32_t *__restrict__ counts) {
+    __shared__ int s_w[NMS_EMIT_THREADS / 32];
+    __shared__ int s_base;
+    const int z = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const uint8_t *state = ctl->final_buf ? st1 : st0;
+    const int r0 = base[z], r1 = base[z + 1];
+    out_xy += (size_t)z * capacity * 2; out_sc += (size_t)z * capacity;
+    if (tid == 0) s_base = 0;
+    __syncthreads();
+    for (int rb = r0; rb < r1; rb += NMS_EMIT_THREADS) {
+        const int r = rb + tid;
+        const int i = r < r1 ? order[r] : 0;
+        PGM_ASSERT(r >= r1 || (i >= r0 && i < r1));
+        const bool hit = r < r1 && state[i] == 1;
+        const unsigned m = __ballot_sync(0xffffffffu, hit);
+        if (lane == 0) s_w[wid] = __popc(m);
+        __syncthreads();
+        int off = s_base;
+        for (int k = 0; k < wid; k++) off += s_w[k];
+        const int pos = off + __popc(m & ((1u << lane) - 1u));
+        if (hit && pos < capacity) {
+            out_xy[2 * (size_t)pos] = xy[2 * (size_t)i]; out_xy[2 * (size_t)pos + 1] = xy[2 * (size_t)i + 1];
+            out_sc[pos] = sc[i];
+        }
+        __syncthreads();
+        if (tid == 0) { int t = 0; for (int k = 0; k < NMS_EMIT_THREADS / 32; k++) t += s_w[k]; s_base += t; }
+        __syncthreads();
+    }
+    if (tid == 0) counts[z] = s_base;
 }
 
 }  // namespace pgm_det

@@ -2320,7 +2320,7 @@ extern "C" int pgm_detect_describe_dev(pgm_handle *h, const float *d_gray, int32
 // Many equally sized images in one call, nothing read back in between: FAST-12 -> ordered keypoint list -> BRIEF for
 // image k into its own `capacity` output slots; the counts stay on the device (d_out_counts) and are copied to
 // `out_counts` at the end if the caller wants them (one synchronisation for the whole batch, none if NULL).  A count
-// above `capacity` means the image's list was truncated.  No NMS in this form.
+// above `capacity` means the image's list was truncated.  No NMS in this form (pgm_detect_nms_describe_batch_dev has it).
 __global__ void batch_counts_kernel(const int32_t *__restrict__ rowoff, int h, int n_images, int32_t *__restrict__ counts) {
     const int z = blockIdx.x * blockDim.x + threadIdx.x;
     if (z < n_images) counts[z] = rowoff[(size_t)z * (h + 1) + h];
@@ -2372,6 +2372,142 @@ extern "C" int pgm_detect_describe_batch_dev(pgm_handle *h, const float *d_gray,
     CU_CHECK(h, cudaGetLastError());
     if (out_counts) {
         if ((rc = ensure_host(h, h->pin_out, (size_t)n_images * 4))) return rc;
+        CU_CHECK(h, cudaMemcpyAsync(h->pin_out.p, d_out_counts, (size_t)n_images * 4, cudaMemcpyDeviceToHost, s));
+        CU_CHECK(h, cudaStreamSynchronize(s));
+        memcpy(out_counts, h->pin_out.p, (size_t)n_images * 4);
+        h->stats.host_syncs++; h->stats.d2h_bytes += (int64_t)n_images * 4;
+    }
+    return PGM_OK;
+}
+
+// The batched chain with NMS: FAST-12 -> RedundantKeypointEliminator -> BRIEF for every image, equal per image to
+// pgm_detect_describe_dev(nms_radius).  One read-back (the per-image FAST totals, which size the flat keypoint list);
+// the NMS rounds of all images run in one cooperative kernel that decides by itself when they are over.
+extern "C" int pgm_detect_nms_describe_batch_dev(pgm_handle *h, const float *d_gray, int32_t n_images, int32_t width,
+                                                 int32_t height, float threshold, int32_t nms_radius, const int32_t *pairs,
+                                                 int32_t n_pairs, int32_t stride_bytes, uint32_t flags, int32_t *d_out_xy,
+                                                 int32_t *d_out_score, uint8_t *d_out_desc, int32_t capacity,
+                                                 int32_t *d_out_counts, int32_t *out_counts) {
+    using namespace pgm_det;
+    if (!h) return PGM_E_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    int rc = check_format(h, n_pairs, stride_bytes);       // desc_bits == NumGaussianPairs
+    if (rc) return rc;
+    if (!d_gray || n_images < 0 || n_images > 65535 || width < 1 || height < 1 || width > 65535 || height > 65535 ||
+        nms_radius < 0 || !pairs || capacity < 1 || !d_out_xy || !d_out_score || !d_out_desc || !d_out_counts)
+        return fail(h, PGM_E_INVALID_ARG, "bad arguments");
+    h->stats = pgm_stats{};
+    h->stats_pending = false;
+    if (n_images == 0) return PGM_OK;
+    CU_CHECK(h, cudaSetDevice(h->device));
+    cudaStream_t s = h->stream;
+    const bool py = (flags & PGM_FLAG_PYTHON_GENERATION) != 0;
+
+    // 1. FAST-12 of every image, per-image totals read back once
+    const size_t npx = (size_t)width * height;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
+    const size_t o_sc = take(npx * n_images), o_cnt = take((size_t)height * n_images * 4);
+    const size_t o_off = take((size_t)(height + 1) * n_images * 4), o_tot = take((size_t)n_images * 4);
+    const size_t o_base = take((size_t)(n_images + 1) * 4), o_pairs = take((size_t)n_pairs * 16);
+    if ((rc = ensure_dev(h, h->misc, off))) return rc;
+    if ((rc = ensure_host(h, h->pin_out, (size_t)n_images * 4))) return rc;
+    char *mb = (char *)h->misc.p;
+    uint8_t *d_sc = (uint8_t *)(mb + o_sc);
+    int32_t *d_cnt = (int32_t *)(mb + o_cnt), *d_off = (int32_t *)(mb + o_off), *d_tot = (int32_t *)(mb + o_tot);
+    int32_t *d_base = (int32_t *)(mb + o_base), *d_pairs = (int32_t *)(mb + o_pairs);
+    dim3 blk(32, 8), grd((width + 31) / 32, (height + 7) / 8, n_images);
+    if (py) fast_score_kernel<1><<<grd, blk, 0, s>>>(d_gray, width, height, threshold, d_sc);
+    else fast_score_kernel<0><<<grd, blk, 0, s>>>(d_gray, width, height, threshold, d_sc);
+    row_count_kernel<<<dim3(height, n_images), 128, 0, s>>>(d_sc, width, d_cnt);
+    scan_kernel<<<n_images, 1024, 0, s>>>(d_cnt, height, d_off);
+    batch_counts_kernel<<<(n_images + 255) / 256, 256, 0, s>>>(d_off, height, n_images, d_tot);
+    CU_CHECK(h, cudaMemcpyAsync(h->pin_out.p, d_tot, (size_t)n_images * 4, cudaMemcpyDeviceToHost, s));
+    CU_CHECK(h, cudaStreamSynchronize(s));
+    h->stats.kernel_launches += 4; h->stats.host_syncs++; h->stats.d2h_bytes += (int64_t)n_images * 4;
+
+    // image bases of the flat keypoint list and the pair table, staged together (the sync above freed pin_in);
+    // every index below is an int32
+    const int32_t *h_tot = (const int32_t *)h->pin_out.p;
+    int64_t total = 0;
+    for (int z = 0; z < n_images; z++) total += h_tot[z];
+    if (total > INT32_MAX) return fail(h, PGM_E_CAPACITY, "the batch has more than 2^31 - 1 FAST keypoints: split it");
+    const int32_t n = (int32_t)total;
+    const size_t base_bytes = (size_t)(n_images + 1) * 4;
+    if ((rc = ensure_host(h, h->pin_in, base_bytes + (size_t)n_pairs * 16))) return rc;
+    int32_t *h_base = (int32_t *)h->pin_in.p;
+    h_base[0] = 0;
+    for (int z = 0; z < n_images; z++) h_base[z + 1] = h_base[z] + h_tot[z];
+    memcpy((char *)h->pin_in.p + base_bytes, pairs, (size_t)n_pairs * 16);
+    CU_CHECK(h, cudaMemcpyAsync(d_base, h->pin_in.p, base_bytes, cudaMemcpyHostToDevice, s));
+    CU_CHECK(h, cudaMemcpyAsync(d_pairs, (char *)h->pin_in.p + base_bytes, (size_t)n_pairs * 16, cudaMemcpyHostToDevice, s));
+    h->stats.h2d_bytes += (int64_t)base_bytes + (int64_t)n_pairs * 16;
+    if (n == 0) {
+        CU_CHECK(h, cudaMemsetAsync(d_out_counts, 0, (size_t)n_images * 4, s));
+    } else {
+        // scratch of the flat list: h->out; radix-sort temporaries: h->out2
+        const int cs = std::max(nms_radius, 1);
+        const int ncx = (width - 1) / cs + 1, ncy = (height - 1) / cs + 1;
+        const long long r2 = (long long)nms_radius * nms_radius;
+        size_t o2 = 0;
+        auto take2 = [&](size_t bytes) { size_t o = o2; o2 = align_up(o2 + bytes, 256); return o; };
+        const size_t o_xy = take2((size_t)n * 8), o_s = take2((size_t)n * 4), o_rk = take2((size_t)n * 4), o_or = take2((size_t)n * 4);
+        const size_t o_k0 = take2((size_t)n * 8), o_k1 = take2((size_t)n * 8), o_c0 = take2((size_t)n * 8), o_c1 = take2((size_t)n * 8);
+        const size_t o_v0 = take2((size_t)n * 4), o_v1 = take2((size_t)n * 4), o_st0 = take2(n), o_st1 = take2(n);
+        const size_t o_ctl = take2(sizeof(NmsBatchCtl));
+        if ((rc = ensure_dev(h, h->out, o2))) return rc;
+        char *ob = (char *)h->out.p;
+        int32_t *d_xy = (int32_t *)(ob + o_xy), *d_s = (int32_t *)(ob + o_s), *d_rk = (int32_t *)(ob + o_rk);
+        int32_t *d_or = (int32_t *)(ob + o_or), *d_v0 = (int32_t *)(ob + o_v0), *d_v1 = (int32_t *)(ob + o_v1);
+        unsigned long long *d_k0 = (unsigned long long *)(ob + o_k0), *d_k1 = (unsigned long long *)(ob + o_k1);
+        unsigned long long *d_c0 = (unsigned long long *)(ob + o_c0), *d_c1 = (unsigned long long *)(ob + o_c1);
+        uint8_t *d_st0 = (uint8_t *)(ob + o_st0), *d_st1 = (uint8_t *)(ob + o_st1);
+        NmsBatchCtl *d_ctl = (NmsBatchCtl *)(ob + o_ctl);
+        int img_bits = 0, cell_bits = 1;
+        while ((n_images - 1) >> img_bits) img_bits++;
+        const unsigned long long n_cells = (unsigned long long)n_images * ncy * ncx;
+        while (cell_bits < 64 && (n_cells - 1) >> cell_bits) cell_bits++;
+        const int rank_bits = NMS_RANK_IMAGE_SHIFT + img_bits;
+        size_t tmp_bytes = 0, tmp2 = 0;
+        CU_CHECK(h, cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, d_k0, d_k1, n, 0, rank_bits, s));
+        CU_CHECK(h, cub::DeviceRadixSort::SortPairs(nullptr, tmp2, d_c0, d_c1, d_v0, d_v1, n, 0, cell_bits, s));
+        tmp_bytes = std::max(tmp_bytes, tmp2);
+        if ((rc = ensure_dev(h, h->out2, tmp_bytes))) return rc;
+        int nb = 0;
+        CU_CHECK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, nms_rounds_batch_kernel, NMS_BATCH_THREADS, 0));
+        const int rounds_grid = (int)std::min<int64_t>((int64_t)std::max(nb, 1) * h->num_sms,
+                                                       ((int64_t)n + NMS_BATCH_THREADS - 1) / NMS_BATCH_THREADS);
+
+        // 2. flat list with rank keys and cell ids; 3. rank order; 4. cell order
+        nms_batch_emit_kernel<<<dim3((height + 3) / 4, n_images), 128, 0, s>>>(d_sc, width, height, d_off, d_base, cs, ncx,
+                                                                              ncy, d_xy, d_s, d_k0, d_c0, d_v0);
+        CU_CHECK(h, cub::DeviceRadixSort::SortKeys(h->out2.p, tmp_bytes, d_k0, d_k1, n, 0, rank_bits, s));
+        nms_batch_order_kernel<<<(n + 255) / 256, 256, 0, s>>>(d_k1, n, d_base, n_images, d_or, d_rk);
+        CU_CHECK(h, cub::DeviceRadixSort::SortPairs(h->out2.p, tmp_bytes, d_c0, d_c1, d_v0, d_v1, n, 0, cell_bits, s));
+        // 5. every round of every image; 6. survivors in output order into the caller's slots
+        CU_CHECK(h, cudaMemsetAsync(d_st0, 0, n, s));
+        CU_CHECK(h, cudaMemsetAsync(d_ctl, 0, sizeof(NmsBatchCtl), s));
+        int n_arg = n, cs_arg = cs, ncx_arg = ncx, ncy_arg = ncy;
+        long long r2_arg = r2;
+        const int32_t *a_xy = d_xy, *a_rk = d_rk, *a_v1 = d_v1;
+        const unsigned long long *a_c0 = d_c0, *a_c1 = d_c1;
+        void *args[] = {&a_xy, &a_rk, &n_arg, &r2_arg, &cs_arg, &ncx_arg, &ncy_arg, &a_c0, &a_c1, &a_v1, &d_st0, &d_st1, &d_ctl};
+        CU_CHECK(h, cudaLaunchCooperativeKernel((void *)nms_rounds_batch_kernel, dim3(rounds_grid), dim3(NMS_BATCH_THREADS),
+                                                args, 0, s));
+        nms_batch_gather_kernel<<<n_images, NMS_EMIT_THREADS, 0, s>>>(d_or, d_base, d_st0, d_st1, d_ctl, d_xy, d_s,
+                                                                      capacity, d_out_xy, d_out_score, d_out_counts);
+        h->stats.kernel_launches += 6;     // emit, rank sort, order, cell sort, rounds, gather (a radix sort counts once)
+    }
+    // 7. BRIEF of the survivors
+    if (n > 0) {
+        const int warps = 4, sw = stride_bytes / 4;
+        brief_kernel<<<dim3((capacity + warps - 1) / warps, n_images), warps * 32, warps * sw * 4, s>>>(
+            d_gray, width, height, d_out_xy, capacity, d_pairs, n_pairs, sw, py ? 1 : 0, (uint32_t *)d_out_desc, nullptr,
+            d_out_counts);
+        h->stats.kernel_launches += 1;
+    }
+    CU_CHECK(h, cudaGetLastError());
+    if (out_counts) {
         CU_CHECK(h, cudaMemcpyAsync(h->pin_out.p, d_out_counts, (size_t)n_images * 4, cudaMemcpyDeviceToHost, s));
         CU_CHECK(h, cudaStreamSynchronize(s));
         memcpy(out_counts, h->pin_out.p, (size_t)n_images * 4);

@@ -460,11 +460,16 @@ class Matcher:
             return xy[:n], sc[:n], desc[:n]
 
     def detect_describe_batch_dev(self, d_gray, threshold: float, pairs: np.ndarray, capacity: int = 4096,
-                                  stride: Optional[int] = None, python_generation: bool = False, read_counts: bool = True):
+                                  stride: Optional[int] = None, python_generation: bool = False, read_counts: bool = True,
+                                  nms_radius: int = -1):
         """FAST-12 -> BRIEF for a stack of device-resident images (torch float32 ``[K, H, W]``), one call, nothing read
         back between the images.  Returns ``(xy int32[K, capacity, 2], score int32[K, capacity], desc uint8[K, capacity,
         stride], counts)`` where ``counts`` is a numpy int32[K] (one synchronisation) or, with ``read_counts=False``,
-        a device tensor (no synchronisation at all).  A count above ``capacity`` means that image's list was truncated."""
+        a device tensor (no synchronisation at all).  A count above ``capacity`` means that image's list was truncated.
+
+        With ``nms_radius >= 0`` the chain includes the reference's NMS (RedundantKeypointEliminator) on every image's
+        full FAST list, as :meth:`detect_describe_dev` does per image: the counts are then the survivors, in the
+        reference's output order, and the call synchronises once more, to size its scratch from the FAST totals."""
         import torch
         pairs = np.ascontiguousarray(pairs, dtype=np.int32).reshape(-1, 4)
         k, hgt, wid = (int(x) for x in d_gray.shape)
@@ -479,10 +484,17 @@ class Matcher:
         d_cnt = torch.zeros(max(k, 1), dtype=torch.int32, device=d_gray.device)
         h_cnt = np.zeros(max(k, 1), dtype=np.int32)
         with self.torch_ordered(d_gray.device):
-            self._check(self._lib.pgm_detect_describe_batch_dev(
-                self._h, d_gray.data_ptr(), k, wid, hgt, float(threshold), pairs.ctypes.data, n_pairs, stride, flags,
-                xy.data_ptr(), sc.data_ptr(), desc.data_ptr(), cap, d_cnt.data_ptr(),
-                h_cnt.ctypes.data if read_counts else None))
+            if nms_radius >= 0:
+                rc = self._lib.pgm_detect_nms_describe_batch_dev(
+                    self._h, d_gray.data_ptr(), k, wid, hgt, float(threshold), int(nms_radius), pairs.ctypes.data, n_pairs,
+                    stride, flags, xy.data_ptr(), sc.data_ptr(), desc.data_ptr(), cap, d_cnt.data_ptr(),
+                    h_cnt.ctypes.data if read_counts else None)
+            else:
+                rc = self._lib.pgm_detect_describe_batch_dev(
+                    self._h, d_gray.data_ptr(), k, wid, hgt, float(threshold), pairs.ctypes.data, n_pairs, stride, flags,
+                    xy.data_ptr(), sc.data_ptr(), desc.data_ptr(), cap, d_cnt.data_ptr(),
+                    h_cnt.ctypes.data if read_counts else None)
+            self._check(rc)
         return xy, sc, desc, (h_cnt[:k] if read_counts else d_cnt[:k])
 
     def nms(self, xy: np.ndarray, score: np.ndarray, radius: int) -> np.ndarray:

@@ -6,7 +6,8 @@ shifted right by a growing offset, columns shifted out of the frame dropped, vac
 K = 32 frames at 5 k px.  The pipeline is the reference's own chain (TestService.cs:80-96 per pair; FAST-12 + BRIEF of
 the Python generation, which the reference tree can execute): detector -> descriptors -> matcher, all on the GPU:
 
-    frames (one H2D) -> pgm_detect_describe_batch_dev (6 kernels for all frames, one read-back of K counts)
+    frames (one H2D) -> pgm_detect_describe_batch_dev (6 kernels for all frames, one read-back of K counts), or with
+                        NMS pgm_detect_nms_describe_batch_dev (every NMS round on the device, one more read-back)
                      -> pgm_match_pairs_batch_dev over the K - 1 consecutive pairs (greedy, the reference's MatchKeypoints)
                      -> pgm_match_ratio_crosscheck_batch_dev: nearest / second nearest + ratio test + cross-check of every
                         consecutive pair in one launch (the north_star extension)
@@ -68,15 +69,17 @@ class SequenceResult:
 
 def match_sequence_dev(matcher, d_frames, threshold: float, pairs: np.ndarray, ratio: float = 0.8,
                        cross_check: bool = True, capacity: int = 4096, python_generation: bool = True,
-                       desc_bits: int = 256, timings: dict | None = None) -> SequenceResult:
-    """``d_frames``: torch float32 ``[K, H, W]`` on the matcher's GPU (grey values on the generation's scale)."""
+                       desc_bits: int = 256, timings: dict | None = None, nms_radius: int = -1) -> SequenceResult:
+    """``d_frames``: torch float32 ``[K, H, W]`` on the matcher's GPU (grey values on the generation's scale).
+    ``nms_radius >= 0`` matches the keypoints that survive the reference's NMS (RedundantKeypointEliminator) of that
+    radius, as the C# pipeline does (BuildKeypointDetectorPipeline, TestService.cs:94-95)."""
     import torch
 
     from .sharding import consecutive_pairs
     table = pairs_table(pairs)
     t0 = time.perf_counter()
     xy, _sc, desc, counts = matcher.detect_describe_batch_dev(d_frames, threshold, table, capacity=capacity,
-                                                              python_generation=python_generation)
+                                                              python_generation=python_generation, nms_radius=nms_radius)
     if (counts > capacity).any():
         raise ValueError(f"a frame has {int(counts.max())} keypoints, more than capacity={capacity}")
     t1 = time.perf_counter()

@@ -135,3 +135,34 @@ def two_view_matches(seed: int, n_pairs: int, per_pair: int = 512, outlier_frac:
     qi = np.tile(np.arange(m, dtype=np.int32), n_pairs)
     return (np.ascontiguousarray(xy), offs, pairs, qi, tj.reshape(-1).astype(np.int32),
             np.arange(n_pairs, dtype=np.int64) * m, np.full(n_pairs, m, dtype=np.int32))
+
+
+# ---- images for the keypoint producer -----------------------------------------------------------------------------
+def rectangles_image(h: int = 3000, w: int = 4000, seed: int = 7, shift: int = 0) -> np.ndarray:
+    """float32[h, w] on the Grayscale.K scale: 1500 random overlapping rectangles on 0.5 and 8000 random 3 x 3 blobs
+    (tools/detect_one.py's image; 4000 x 3000 is the size of the reference's lego photographs), shifted right by
+    ``shift`` px with the vacated columns black, as scripts/image_editing.py:8-15 shifts its frames."""
+    rng = np.random.default_rng(seed)
+    img = np.full((h, w), 0.5, dtype=np.float32)
+    for _ in range(1500):
+        x0, y0 = int(rng.integers(0, w - 40)), int(rng.integers(0, h - 40))
+        rw, rh = int(rng.integers(20, 400)), int(rng.integers(20, 400))
+        img[y0:y0 + rh, x0:x0 + rw] = np.float32(rng.random())
+    for _ in range(8000):                      # small blobs: every ring pixel differs from the centre
+        x0, y0 = int(rng.integers(5, w - 8)), int(rng.integers(5, h - 8))
+        img[y0:y0 + 3, x0:x0 + 3] = np.float32(rng.random())
+    if shift:
+        out = np.zeros_like(img)
+        out[:, shift:] = img[:, :w - shift]
+        img = out
+    return img
+
+
+def dotted_row_image(h: int = 40, w: int = 2000, value: float = 1.0) -> np.ndarray:
+    """float32[h, w], black but for a dot of ``value`` every 4 px on row 20 (x = 8, 12, ..., 1988 at the default
+    size): 496 FAST keypoints of score 16 at threshold 0.1 (``value`` 255 and threshold 50 for the Python generation).
+    At NMS radius 4 each dot suppresses its right neighbour only once it is itself kept, so the parallel rounds form a
+    chain of 496 and every other dot survives (248)."""
+    img = np.zeros((h, w), dtype=np.float32)
+    img[20, 8:w - 8:4] = np.float32(value)
+    return img

@@ -15,6 +15,8 @@
      filter with its reversed pairs and ordered compaction
   8. batched fundamental-matrix RANSAC of 6 pairs: one below P, a degenerate one (every keypoint the same pixel), one of
      20 000 matches (several shared-memory tiles per score CTA), S spread over two score items per pair
+  9. batched detect -> NMS -> BRIEF of 4 frames: the dotted-row chain (496 device-side rounds in the cooperative kernel),
+     a blank frame (empty run) and two random frames, against the oracle chain
 Every result is checked against the oracle, so a sanitizer run is also a parity run."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -111,5 +113,21 @@ for p, (eb, ei, eF, em, _, _) in enumerate(exp):
     assert np.abs(F[p].astype(np.float64) - eF).max() <= 1e-6 * max(np.abs(eF).max(), 1e-30), p
 assert best[1] == -2 and np.isfinite(F).all()
 print("case 8 ok", m.stats())
+from oracle import detect_np as D
+from photogrammetry_b200.descriptors import pack_descriptors
+rng = np.random.default_rng(12)
+frames = np.stack([synthetic.dotted_row_image(), np.zeros((40, 2000), np.float32),
+                   rng.random((40, 2000), dtype=np.float32), rng.random((40, 2000), dtype=np.float32)])
+dpairs = D.gaussian_pairs(11, 256, 50)
+xy, sc, desc, counts = m.detect_describe_batch_dev(torch.from_numpy(frames).cuda(), 0.1, dpairs.reshape(-1, 4),
+                                                   capacity=4096, nms_radius=4)
+for k in range(4):
+    exy, esc = D.detect_vectorised(frames[k], 0.1)
+    kept = D.eliminate_redundant_vectorised(exy, esc, 4)
+    n = len(kept)
+    assert counts[k] == n and (xy[k, :n].cpu().numpy() == exy[kept]).all() and (sc[k, :n].cpu().numpy() == esc[kept]).all()
+    assert (desc[k, :n].cpu().numpy() == pack_descriptors(D.brief_descriptors(frames[k], exy[kept], dpairs), 256)).all()
+assert counts[0] == 248 and counts[1] == 0
+print("case 9 ok", m.stats())
 m.close()
 print("ALL OK")
