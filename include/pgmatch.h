@@ -358,6 +358,32 @@ int pgm_detect_nms_describe_batch_dev(pgm_handle *h, const float *d_gray, int32_
                                       int32_t *d_out_score, uint8_t *d_out_desc, int32_t capacity,
                                       int32_t *d_out_counts, int32_t *out_counts);
 
+/* The batched chain for images of ANY sizes, with or without NMS: a photogrammetry capture is an unordered set of
+ * photos (portrait next to landscape, mixed cameras and crops), and upstream detects each at its own size
+ * (KeypointDetection.Detect takes a Matrix<Grayscale> of any dimensions).  Image k is row-major widths[k] x
+ * heights[k] at d_gray + pixel_offsets[k] (device memory); pixel_offsets (int64[n_images + 1], the delimiter
+ * convention of the matchers' image_offsets), widths and heights (int32[n_images]) are host memory.  Only the declared
+ * pixels are read: gaps between the images may hold anything.  nms_radius < 0 skips NMS.
+ *  - Output layout, flags (both generations) and counts are those of pgm_detect_describe_batch_dev (nms_radius < 0)
+ *    and pgm_detect_nms_describe_batch_dev (nms_radius >= 0): image k owns `capacity` slots, d_out_counts[k] (device)
+ *    can be above `capacity`, and no slot at or beyond min(count, capacity) of an image is written.
+ *  - For every image k the result equals pgm_detect_describe_dev(image k, widths[k], heights[k], threshold,
+ *    nms_radius, ...) bit for bit: (x, y), FastScore, descriptor bytes and order.  Images below 7 pixels on a side
+ *    have no FAST interior and count 0.
+ *  - Synchronisation and launches are those of the uniform forms, whatever n_images and the mix of sizes:
+ *    host_syncs 0 without NMS and 1 with it, plus 1 with out_counts; 6 kernel launches without NMS, 11 with it.
+ *  - Refusals: PGM_E_INVALID_ARG for a null pointer, n_images outside 0..65535, a width or height outside
+ *    1..65535, pixel_offsets[0] < 0, pixel_offsets[k + 1] < pixel_offsets[k] + widths[k] * heights[k],
+ *    capacity < 1 and every descriptor format pgm_detect_describe_batch_dev refuses; PGM_E_CAPACITY when the set's
+ *    FAST keypoints together exceed 2^31 - 1 (NMS only; after the read-back and before any later kernel runs).
+ *    n_images == 0 does nothing. */
+int pgm_detect_describe_images_batch_dev(pgm_handle *h, const float *d_gray, const int64_t *pixel_offsets,
+                                         const int32_t *widths, const int32_t *heights, int32_t n_images,
+                                         float threshold, int32_t nms_radius, const int32_t *pairs, int32_t n_pairs,
+                                         int32_t stride_bytes, uint32_t flags, int32_t *d_out_xy, int32_t *d_out_score,
+                                         uint8_t *d_out_desc, int32_t capacity, int32_t *d_out_counts,
+                                         int32_t *out_counts);
+
 /* ---- the consumer of the match list (SURVEY.md section 8, row f3) --------------------
  * pgm_ransac_score: the scoring loops of CameraPoseEstimation.GetFundamentalMatrix
  * (ImageProcessing/CameraPoseEstimation.cs:41-88).  F: n_hyp row-major 3x3 float matrices (the estimates of the

@@ -40,7 +40,7 @@ EXPORTED_SYMBOLS = (
     "pgm_match_keypoints_sorted", "pgm_match_keypoints_sorted_dev", "pgm_knn2_l2", "pgm_knn2_l2_dev", "pgm_l2_last_fallback_rows",
     "pgm_knn2_l2_pairs_batch_dev", "pgm_match_l2_ratio_crosscheck_pairs_batch_dev",
     "pgm_fast_detect", "pgm_brief_describe", "pgm_nms", "pgm_detect_describe_dev", "pgm_detect_describe_batch_dev",
-    "pgm_detect_nms_describe_batch_dev",
+    "pgm_detect_nms_describe_batch_dev", "pgm_detect_describe_images_batch_dev",
     "pgm_ransac_score", "pgm_ransac_fundamental_pairs_batch_dev",
     "pgm_shard_create", "pgm_shard_edge_capacity", "pgm_shard_round", "pgm_shard_commit", "pgm_shard_finish_round",
     "pgm_shard_finish", "pgm_shard_destroy",
@@ -164,6 +164,9 @@ def load() -> C.CDLL:
         lib.pgm_detect_nms_describe_batch_dev.argtypes = [C.c_void_p, vp, C.c_int32, C.c_int32, C.c_int32, C.c_float,
                                                           C.c_int32, i32p, C.c_int32, C.c_int32, C.c_uint32, i32p, i32p,
                                                           u8p, C.c_int32, i32p, i32p]
+        lib.pgm_detect_describe_images_batch_dev.argtypes = [C.c_void_p, vp, i64p, i32p, i32p, C.c_int32, C.c_float,
+                                                             C.c_int32, i32p, C.c_int32, C.c_int32, C.c_uint32, i32p,
+                                                             i32p, u8p, C.c_int32, i32p, i32p]
         lib.pgm_ransac_score.argtypes = [C.c_void_p, vp, u8p, C.c_int32, i32p, i32p, C.c_int32, C.c_float, i32p,
                                          C.POINTER(C.c_int32), u8p]
         lib.pgm_ransac_fundamental_pairs_batch_dev.argtypes = [C.c_void_p, i32p, i64p, C.c_int32, i32p, C.c_int32, i32p, i32p,

@@ -27,13 +27,47 @@ __constant__ int c_ring[2][16][2] = {
     {{0, -3}, {1, -3}, {2, -2}, {3, -1}, {3, 0}, {3, 1}, {2, 2}, {1, 3},
      {0, 3}, {-1, 3}, {-2, 2}, {-3, 1}, {-3, 0}, {-3, -1}, {-2, -2}, {-1, -3}}};
 
-// score map: 0 = no keypoint, else the longest circular run (12..16) = Keypoint.FastScore
+// ---- batch geometry ------------------------------------------------------------------------------------------------
+// Image k of a batch, as the batch kernels see it.  Every image owns a run of each flat index space, at a prefix of
+// the sizes of the images before it; the table has n_images + 1 entries, the last holding the totals.  Work items are
+// flat over all images (FAST tiles, rows) unless every image has one size (see fast_score_kernel).
+constexpr int FAST_TILE_W = 32, FAST_TILE_H = 8;   // fast_score_kernel's block
+struct ImageGeom {
+    long long px;     // first pixel in the caller's image buffer
+    long long sc;     // first byte of the score map (sum of w * h)
+    long long row;    // first of h + 1 row slots: row counts, row offsets (slot h = the image's total), row work items
+    long long tile;   // first FAST tile (FAST_TILE_W x FAST_TILE_H pixels)
+    long long cell;   // first NMS cell id (cells of side max(radius, 1) over [0, w) x [0, h)); 0 without NMS
+    int w, h;
+    int ncx, ncy;     // NMS cells per row / column; 0 without NMS
+};
+
+// The flat kernels run a resident grid (FLAT_CTAS_PER_SM_* CTAs per SM) in which every CTA (or warp) takes one
+// contiguous, balanced range of the work items: the image lookup, a dependent chain of table loads, is paid once per
+// range.  Paid once per short-lived CTA it adds its latency to every FAST tile and row (about 10 % on 4000 x 3000 frames).
+constexpr int FLAT_CTAS_PER_SM_256 = 8, FLAT_CTAS_PER_SM_128 = 16;   // full occupancy at <= 32 registers
+
+// [*b, *e): the items of work unit u out of n_units
+__device__ __forceinline__ void unit_range(long long n_items, long long u, long long n_units, long long *b, long long *e) {
+    const long long per = (n_items + n_units - 1) / n_units;
+    *b = min(u * per, n_items); *e = min(*b + per, n_items);
+}
+
+// image owning flat item t of the index space F (the last k with geo[k].*F <= t; every image owns at least one item)
+template <long long ImageGeom::*F>
+__device__ __forceinline__ int image_of(const ImageGeom *__restrict__ geo, int n_images, long long t) {
+    int lo = 0, hi = n_images - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (geo[mid].*F <= t) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// score of pixel (x, y): 0 = no keypoint, else the longest circular run (12..16) = Keypoint.FastScore
 template <int RING>
-__global__ void fast_score_kernel(const float *__restrict__ img, int w, int h, float threshold,
-                                  uint8_t *__restrict__ score) {
-    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
-    if (x >= w || y >= h) return;
-    img += (size_t)blockIdx.z * w * h; score += (size_t)blockIdx.z * w * h;      // batched form: blockIdx.z = image
+__device__ __forceinline__ uint8_t fast_score_at(const float *__restrict__ img, int w, int h, int x, int y,
+                                                 float threshold) {
     uint8_t out = 0;
     if (x >= 3 && x < w - 3 && y >= 3 && y < h - 3) {                 // Detect's loop bounds, :45-47
         const float *p = img + (size_t)y * w + x;
@@ -71,28 +105,113 @@ __global__ void fast_score_kernel(const float *__restrict__ img, int w, int h, f
             }
         }
     }
-    score[(size_t)y * w + x] = out;
+    return out;
+}
+
+// score map of one image, block (FAST_TILE_W, FAST_TILE_H)
+template <int RING>
+__global__ void fast_score_kernel(const float *__restrict__ img, int w, int h, float threshold,
+                                  uint8_t *__restrict__ score) {
+    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
+    if (x >= w || y >= h) return;
+    score[(size_t)y * w + x] = fast_score_at<RING>(img, w, h, x, y, threshold);
+}
+
+// batched form, image k's map at score + geo[k].sc.  A set of one size uw x uh packed back to back (uw > 0) runs on the
+// grid (tiles x, tiles y, images) and reads no table: these CTAs are short and latency-bound, and a table read before
+// the pixel loads would add its latency to each.  Any other set: one contiguous range of the flat FAST tile space
+// (geo[].tile) per CTA.
+template <int RING>
+__global__ void __launch_bounds__(FAST_TILE_W * FAST_TILE_H, FLAT_CTAS_PER_SM_256) fast_score_kernel(
+        const float *__restrict__ img, const ImageGeom *__restrict__ geo, int n_images, int uw, int uh,
+        float threshold, uint8_t *__restrict__ score) {
+    if (uw) {
+        const int x = blockIdx.x * FAST_TILE_W + threadIdx.x, y = blockIdx.y * FAST_TILE_H + threadIdx.y;
+        if (x >= uw || y >= uh) return;
+        const long long off = (long long)blockIdx.z * uw * uh;
+        score[off + (long long)y * uw + x] = fast_score_at<RING>(img + off, uw, uh, x, y, threshold);
+        return;
+    }
+    long long t0, t1;
+    unit_range(geo[n_images].tile, blockIdx.x, gridDim.x, &t0, &t1);
+    if (t0 >= t1) return;
+    // the image's pointers and sizes and the tile's coordinates stay in registers while the range is inside the image
+    int z = image_of<&ImageGeom::tile>(geo, n_images, t0), w = 0, h = 0, ntx = 1, left = 0;
+    const float *im = nullptr;
+    uint8_t *sm = nullptr;
+    auto enter = [&]() {
+        im = img + geo[z].px; sm = score + geo[z].sc; w = geo[z].w; h = geo[z].h;
+        ntx = (w + FAST_TILE_W - 1) / FAST_TILE_W; left = (int)(geo[z + 1].tile - geo[z].tile);   // < 2^24 tiles
+    };
+    enter();
+    const int lt = (int)(t0 - geo[z].tile);
+    int ty = lt / ntx, tx = lt - ty * ntx;
+    left -= lt;
+    for (int n = (int)(t1 - t0); n > 0; n--) {                           // per <= 2^31 tiles
+        if (left == 0) { z++; enter(); tx = ty = 0; }                      // every image owns a tile: none is skipped
+        PGM_ASSERT(z < n_images && left > 0);
+        const int x = tx * FAST_TILE_W + threadIdx.x, y = ty * FAST_TILE_H + threadIdx.y;
+        if (x < w && y < h) sm[(long long)y * w + x] = fast_score_at<RING>(im, w, h, x, y, threshold);
+        if (++tx == ntx) { tx = 0; ty++; }
+        left--;
+    }
+}
+
+// keypoints in one row of a score map, summed over the block (every thread gets the sum; safe to call in a loop)
+__device__ __forceinline__ int row_count_block(const uint8_t *__restrict__ row, int w) {
+    __shared__ int s;
+    int c = 0;
+    for (int x = threadIdx.x; x < w; x += blockDim.x) c += row[x] != 0;
+    c = __reduce_add_sync(0xffffffffu, c);
+    if (threadIdx.x == 0) s = 0;
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0 && c) atomicAdd(&s, c);
+    __syncthreads();
+    const int total = s;
+    __syncthreads();
+    return total;
 }
 
 // per-row keypoint counts (one block per row)
 __global__ void row_count_kernel(const uint8_t *__restrict__ score, int w, int32_t *__restrict__ rowcnt) {
     const int y = blockIdx.x;
-    score += (size_t)blockIdx.y * w * gridDim.x; rowcnt += (size_t)blockIdx.y * gridDim.x;   // batched form: blockIdx.y = image
-    int c = 0;
-    for (int x = threadIdx.x; x < w; x += blockDim.x) c += score[(size_t)y * w + x] != 0;
-    __shared__ int s;
-    if (threadIdx.x == 0) s = 0;
-    __syncthreads();
-    for (int o = 16; o; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-    if ((threadIdx.x & 31) == 0) atomicAdd(&s, c);
-    __syncthreads();
-    if (threadIdx.x == 0) rowcnt[y] = s;
+    const int c = row_count_block(score + (size_t)y * w, w);
+    if (threadIdx.x == 0) rowcnt[y] = c;
 }
 
-// exclusive scan of n <= 65536 ints by one block of 1024 threads; total written to out[n]
-__global__ void scan_kernel(const int32_t *__restrict__ in, int n, int32_t *__restrict__ out) {
+// batched form; rowcnt has the row slots' layout.  One size uw x uh (uw > 0): grid (rows, images), no table read.  Any
+// other set: one contiguous range of the flat row-slot space (geo[].row) per block.
+__global__ void __launch_bounds__(128, FLAT_CTAS_PER_SM_128) row_count_kernel(
+        const uint8_t *__restrict__ score, const ImageGeom *__restrict__ geo, int n_images, int uw, int uh,
+        int32_t *__restrict__ rowcnt) {
+    if (uw) {
+        const int y = blockIdx.x, z = blockIdx.y;
+        const int c = row_count_block(score + ((long long)z * uh + y) * uw, uw);
+        if (threadIdx.x == 0) rowcnt[(long long)z * (uh + 1) + y] = c;
+        return;
+    }
+    long long g0, g1;
+    unit_range(geo[n_images].row, blockIdx.x, gridDim.x, &g0, &g1);
+    if (g0 >= g1) return;
+    int z = image_of<&ImageGeom::row>(geo, n_images, g0);
+    long long row0 = geo[z].row;
+    int w = geo[z].w, h = geo[z].h;
+    for (long long g = g0; g < g1; g++) {
+        if (g > row0 + h) { z++; row0 = geo[z].row; w = geo[z].w; h = geo[z].h; }   // past the total's slot
+        const int y = (int)(g - row0);
+        PGM_ASSERT(z < n_images && y >= 0 && y <= h);
+        if (y == h) continue;                                               // the total's slot
+        const int c = row_count_block(score + geo[z].sc + (long long)y * w, w);
+        if (threadIdx.x == 0) rowcnt[g] = c;
+    }
+}
+
+// exclusive scan of n <= 65536 ints by one block of 1024 threads; total written to out[n].  Batched form (geo given):
+// blockIdx.x = image, n = its height, in / out at its row slots.
+__global__ void scan_kernel(const int32_t *__restrict__ in, int n, int32_t *__restrict__ out,
+                            const ImageGeom *__restrict__ geo = nullptr) {
     __shared__ int s_w[32];
-    in += (size_t)blockIdx.x * n; out += (size_t)blockIdx.x * (n + 1);          // batched form: blockIdx.x = image
+    if (geo) { n = geo[blockIdx.x].h; in += geo[blockIdx.x].row; out += geo[blockIdx.x].row; }
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const int per = (n + 1023) / 1024, p0 = min(tid * per, n), p1 = min(p0 + per, n);
     int sum = 0;
@@ -107,18 +226,14 @@ __global__ void scan_kernel(const int32_t *__restrict__ in, int n, int32_t *__re
     if (tid == 0) out[n] = tot;
 }
 
-// ordered emission of one row (one warp per row, ballot prefix): Detect's row-major list order
-__global__ void emit_kernel(const uint8_t *__restrict__ score, int w, int h, const int32_t *__restrict__ rowoff,
-                            int capacity, int32_t *__restrict__ xy, int32_t *__restrict__ sc) {
-    const int y = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (y >= h) return;
-    // batched form: blockIdx.y = image; every image owns `capacity` output slots
-    score += (size_t)blockIdx.y * w * h; rowoff += (size_t)blockIdx.y * (h + 1);
-    xy += (size_t)blockIdx.y * capacity * 2; sc += (size_t)blockIdx.y * capacity;
-    int base = rowoff[y];
+// ordered emission of row y of one score map by one warp (ballot prefix): Detect's row-major list order, from list
+// position `base`, into slots below `capacity`
+__device__ __forceinline__ void emit_row(const uint8_t *__restrict__ row, int w, int y, int base, int capacity,
+                                         int32_t *__restrict__ xy, int32_t *__restrict__ sc) {
+    const int lane = threadIdx.x & 31;
     for (int x0 = 0; x0 < w; x0 += 32) {
         const int x = x0 + lane;
-        const uint8_t v = x < w ? score[(size_t)y * w + x] : 0;
+        const uint8_t v = x < w ? row[x] : 0;
         const unsigned m = __ballot_sync(0xffffffffu, v != 0);
         if (v) {
             const int pos = base + __popc(m & ((1u << lane) - 1u));
@@ -128,21 +243,57 @@ __global__ void emit_kernel(const uint8_t *__restrict__ score, int w, int h, con
     }
 }
 
+// one warp per row
+__global__ void emit_kernel(const uint8_t *__restrict__ score, int w, int h, const int32_t *__restrict__ rowoff,
+                            int capacity, int32_t *__restrict__ xy, int32_t *__restrict__ sc) {
+    const int y = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (y >= h) return;
+    emit_row(score + (size_t)y * w, w, y, rowoff[y], capacity, xy, sc);
+}
+
+// batched form; every image owns `capacity` output slots.  One size uw x uh (uw > 0): grid (rows / 4, images), one warp
+// per row, no table read.  Any other set: one contiguous range of the flat row-slot space per warp.
+__global__ void __launch_bounds__(128, FLAT_CTAS_PER_SM_128) emit_kernel(
+        const uint8_t *__restrict__ score, const ImageGeom *__restrict__ geo, int n_images, int uw, int uh,
+        const int32_t *__restrict__ rowoff, int capacity, int32_t *__restrict__ xy, int32_t *__restrict__ sc) {
+    if (uw) {
+        const int y = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), z = blockIdx.y;
+        if (y >= uh) return;
+        emit_row(score + ((long long)z * uh + y) * uw, uw, y, rowoff[(long long)z * (uh + 1) + y], capacity,
+                 xy + (size_t)z * capacity * 2, sc + (size_t)z * capacity);
+        return;
+    }
+    long long g0, g1;
+    unit_range(geo[n_images].row, (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5),
+               (long long)gridDim.x * (blockDim.x >> 5), &g0, &g1);
+    if (g0 >= g1) return;
+    int z = image_of<&ImageGeom::row>(geo, n_images, g0);
+    long long row0 = geo[z].row;
+    int h = geo[z].h;
+    for (long long g = g0; g < g1; g++) {
+        if (g > row0 + h) { z++; row0 = geo[z].row; h = geo[z].h; }
+        const int w = geo[z].w, y = (int)(g - row0);
+        PGM_ASSERT(z < n_images && y >= 0 && y <= h);
+        if (y == h) continue;
+        emit_row(score + geo[z].sc + (long long)y * w, w, y, rowoff[g], capacity, xy + (size_t)z * capacity * 2,
+                 sc + (size_t)z * capacity);
+    }
+}
+
 // BRIEF: one warp per keypoint.  pair p sets bit (n_pairs - 1 - p) of the descriptor integer
 // (`descriptor <<= 1` per pair, first pair = MSB), stored little-endian in `stride` bytes.
 __global__ void brief_kernel(const float *__restrict__ img, int w, int h, const int32_t *__restrict__ xy, int n,
                              const int32_t *__restrict__ pairs /*[n_pairs][4]*/, int n_pairs, int stride_words,
-                             int lsb_first, uint32_t *__restrict__ desc, const int32_t *__restrict__ rowoff = nullptr,
+                             int lsb_first, uint32_t *__restrict__ desc, const ImageGeom *__restrict__ geo = nullptr,
                              const int32_t *__restrict__ counts = nullptr) {
     extern __shared__ uint32_t s_desc[];           // [warps][stride_words]
     const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int i = blockIdx.x * (blockDim.x >> 5) + wid;
-    if (rowoff || counts) {                        // batched form: blockIdx.y = image, n = capacity per image, and the
-        const int z = blockIdx.y;                  // image's keypoint count sits on the device: behind its row offsets,
-                                                   // or in counts[z] (the survivors of the batched NMS)
-        const int found = counts ? __ldg(counts + z) : __ldg(rowoff + (size_t)z * (h + 1) + h);
-        img += (size_t)z * w * h; xy += (size_t)z * n * 2; desc += (size_t)z * n * stride_words;
-        n = min(n, found);
+    if (geo) {                                     // batched form: blockIdx.y = image, its geometry in geo, n = capacity
+        const int z = blockIdx.y;                  // per image, and the image's keypoint count in counts[z] on the device
+        w = geo[z].w; h = geo[z].h;
+        img += geo[z].px; xy += (size_t)z * n * 2; desc += (size_t)z * n * stride_words;
+        n = min(n, __ldg(counts + z));
     }
     uint32_t *mine = s_desc + wid * stride_words;
     for (int k = lane; k < stride_words; k += 32) mine[k] = 0u;
@@ -345,35 +496,63 @@ struct NmsBatchCtl {
     int32_t final_buf;      // which state buffer holds the final states (written at exit)
 };
 
-// Detect's row-major list of every image (one warp per row, ballot prefix, as emit_kernel) into the flat list at the
-// image's base, with each keypoint's rank key, its cell id (cells of side cs over [0, w) x [0, h), image-major) and
-// its own flat index (the values of the cell sort).
-__global__ void nms_batch_emit_kernel(const uint8_t *__restrict__ score, int w, int h, const int32_t *__restrict__ rowoff,
-                                      const int32_t *__restrict__ base, int cs, int ncx, int ncy,
-                                      int32_t *__restrict__ xy, int32_t *__restrict__ sc,
-                                      unsigned long long *__restrict__ rank_key, unsigned long long *__restrict__ cell,
-                                      int32_t *__restrict__ idx) {
-    const int y = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (y >= h) return;
-    const int z = blockIdx.y;
-    score += (size_t)z * w * h; rowoff += (size_t)z * (h + 1);
-    const int b0 = __ldg(base + z), n_img = __ldg(base + z + 1) - b0;
-    const unsigned long long row_cell = ((unsigned long long)z * ncy + y / cs) * ncx;
-    int local = rowoff[y];
-    for (int x0 = 0; x0 < w; x0 += 32) {
-        const int x = x0 + lane;
-        const uint8_t v = x < w ? score[(size_t)y * w + x] : 0;
-        const unsigned m = __ballot_sync(0xffffffffu, v != 0);
-        if (v) {
-            const int li = local + __popc(m & ((1u << lane) - 1u));
-            PGM_ASSERT(li >= 0 && li < n_img);
-            const int i = b0 + li;
-            xy[2 * (size_t)i] = x; xy[2 * (size_t)i + 1] = y; sc[i] = v;
-            rank_key[i] = ((unsigned long long)z << NMS_RANK_IMAGE_SHIFT) | ((unsigned long long)(255u - v) << 32) | (unsigned)li;
-            cell[i] = row_cell + (unsigned)(x / cs);
-            idx[i] = i;
+// Detect's row-major list of every image (one warp per row slot, ballot prefix, as emit_kernel) into the flat list at
+// the image's base, with each keypoint's rank key, its cell id (geo[z].cell + cy * ncx + cx, cells of side cs over
+// [0, w) x [0, h)) and its own flat index (the values of the cell sort).
+// One size uw x uh (uw > 0): grid (rows / 4, images), no table read; any other set: a range of row slots per warp
+// (as emit_kernel).
+__global__ void __launch_bounds__(128, FLAT_CTAS_PER_SM_128) nms_batch_emit_kernel(
+        const uint8_t *__restrict__ score, const ImageGeom *__restrict__ geo, int n_images, int uw, int uh,
+        const int32_t *__restrict__ rowoff, const int32_t *__restrict__ base, int cs, int32_t *__restrict__ xy,
+        int32_t *__restrict__ sc, unsigned long long *__restrict__ rank_key, unsigned long long *__restrict__ cell,
+        int32_t *__restrict__ idx) {
+    const int lane = threadIdx.x & 31;
+    long long g0, g1;
+    int z = 0;
+    if (uw) {
+        const int y = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+        if (y >= uh) return;
+        z = blockIdx.y; g0 = (long long)z * (uh + 1) + y; g1 = g0 + 1;
+    } else {                                                               // one range of row slots per warp
+        unit_range(geo[n_images].row, (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5),
+                   (long long)gridDim.x * (blockDim.x >> 5), &g0, &g1);
+        if (g0 >= g1) return;
+        z = image_of<&ImageGeom::row>(geo, n_images, g0);
+    }
+    for (long long g = g0; g < g1; g++) {
+        int w, h, y, ncx;
+        long long sc0, cell0;
+        if (uw) {
+            w = uw; h = uh; y = (int)(g - (long long)z * (uh + 1));
+            ncx = (uw - 1) / cs + 1;
+            sc0 = (long long)z * uw * uh; cell0 = (long long)z * ncx * ((uh - 1) / cs + 1);
+        } else {
+            if (g > geo[z].row + geo[z].h) z++;
+            w = geo[z].w; h = geo[z].h; y = (int)(g - geo[z].row); ncx = geo[z].ncx;
+            sc0 = geo[z].sc; cell0 = geo[z].cell;
         }
-        local += __popc(m);
+        PGM_ASSERT(z < n_images && y >= 0 && y <= h);
+        if (y == h) continue;
+        const uint8_t *row = score + sc0 + (long long)y * w;
+        const int b0 = __ldg(base + z), n_img = __ldg(base + z + 1) - b0;
+        const unsigned long long row_cell = (unsigned long long)cell0 + (unsigned long long)(y / cs) * ncx;
+        PGM_ASSERT(row_cell + ncx <= (unsigned long long)geo[n_images].cell);
+        int local = rowoff[g];
+        for (int x0 = 0; x0 < w; x0 += 32) {
+            const int x = x0 + lane;
+            const uint8_t v = x < w ? row[x] : 0;
+            const unsigned m = __ballot_sync(0xffffffffu, v != 0);
+            if (v) {
+                const int li = local + __popc(m & ((1u << lane) - 1u));
+                PGM_ASSERT(li >= 0 && li < n_img);
+                const int i = b0 + li;
+                xy[2 * (size_t)i] = x; xy[2 * (size_t)i + 1] = y; sc[i] = v;
+                rank_key[i] = ((unsigned long long)z << NMS_RANK_IMAGE_SHIFT) | ((unsigned long long)(255u - v) << 32) | (unsigned)li;
+                cell[i] = row_cell + (unsigned)(x / cs);
+                idx[i] = i;
+            }
+            local += __popc(m);
+        }
     }
 }
 
@@ -398,8 +577,9 @@ __global__ void nms_batch_order_kernel(const unsigned long long *__restrict__ so
 // reading round r's count after the barrier.  Each round decides at least the best-ranked undecided keypoint of every
 // image that has one, so the rounds end after at most n of them.
 __global__ void __launch_bounds__(NMS_BATCH_THREADS) nms_rounds_batch_kernel(
-        const int32_t *__restrict__ xy, const int32_t *__restrict__ rank, int n, long long radius2, int cs, int ncx,
-        int ncy, const unsigned long long *__restrict__ cell, const unsigned long long *__restrict__ sorted_cell,
+        const int32_t *__restrict__ xy, const int32_t *__restrict__ rank, int n, long long radius2, int cs,
+        const ImageGeom *__restrict__ geo, int n_images, const unsigned long long *__restrict__ rank_key,
+        const unsigned long long *__restrict__ cell, const unsigned long long *__restrict__ sorted_cell,
         const int32_t *__restrict__ sorted_idx, uint8_t *st0, uint8_t *st1, NmsBatchCtl *ctl) {
     const int gt = blockIdx.x * blockDim.x + threadIdx.x, gs = gridDim.x * blockDim.x;
     unsigned epoch = 0;
@@ -411,8 +591,11 @@ __global__ void __launch_bounds__(NMS_BATCH_THREADS) nms_rounds_batch_kernel(
             const uint8_t st = __ldcg(st_in + i);
             if (st != 0) { st_out[i] = st; continue; }
             const int x = __ldg(xy + 2 * i), y = __ldg(xy + 2 * i + 1), r = __ldg(rank + i);
-            const int cx = x / cs, cy = y / cs;
+            const int z = (int)(__ldg(rank_key + i) >> NMS_RANK_IMAGE_SHIFT);   // the image's cell grid
+            PGM_ASSERT(z >= 0 && z < n_images);
+            const int ncx = geo[z].ncx, ncy = geo[z].ncy, cx = x / cs, cy = y / cs;
             const long long c = (long long)__ldg(cell + i);
+            PGM_ASSERT(cx < ncx && cy < ncy && c == geo[z].cell + (long long)cy * ncx + cx);
             bool any_kept = false, any_undecided = false;
             for (int dy = -1; dy <= 1 && !any_kept; dy++) {
                 if (cy + dy < 0 || cy + dy >= ncy) continue;

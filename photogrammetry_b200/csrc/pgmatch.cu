@@ -2317,21 +2317,206 @@ extern "C" int pgm_detect_describe_dev(pgm_handle *h, const float *d_gray, int32
     return PGM_OK;
 }
 
-// Many equally sized images in one call, nothing read back in between: FAST-12 -> ordered keypoint list -> BRIEF for
-// image k into its own `capacity` output slots; the counts stay on the device (d_out_counts) and are copied to
-// `out_counts` at the end if the caller wants them (one synchronisation for the whole batch, none if NULL).  A count
-// above `capacity` means the image's list was truncated.  No NMS in this form (pgm_detect_nms_describe_batch_dev has it).
-__global__ void batch_counts_kernel(const int32_t *__restrict__ rowoff, int h, int n_images, int32_t *__restrict__ counts) {
+// Batched detection: many images in one call, every image at its own size (pgm_detect.cuh's ImageGeom table).
+// counts[z] = the FAST total behind image z's row offsets (slot h of its rows)
+__global__ void batch_counts_kernel(const int32_t *__restrict__ rowoff, const pgm_det::ImageGeom *__restrict__ geo,
+                                    int n_images, int32_t *__restrict__ counts) {
     const int z = blockIdx.x * blockDim.x + threadIdx.x;
-    if (z < n_images) counts[z] = rowoff[(size_t)z * (h + 1) + h];
+    if (z < n_images) counts[z] = rowoff[geo[z].row + geo[z].h];
 }
 
+// resident grid of a flat kernel (pgm_detect.cuh): `ctas_per_sm` per SM, at most one CTA per `per_cta` items
+static unsigned flat_grid(const pgm_handle *h, long long items, int ctas_per_sm, int per_cta) {
+    return (unsigned)std::max<long long>(std::min<long long>((long long)h->num_sms * ctas_per_sm, (items + per_cta - 1) / per_cta), 1);
+}
+
+// The three batch entry points' common body.  Image k is widths[k] x heights[k] at d_gray + pixel_offsets[k]; the
+// caller holds h->mu, has checked every argument and reset the statistics, and n_images >= 1.
+//   no NMS (nms_radius < 0): FAST-12 -> ordered keypoint list -> BRIEF for image k into its own `capacity` output
+//     slots; the counts stay on the device (d_out_counts), nothing is read back.  6 kernel launches.
+//   NMS: FAST-12 -> RedundantKeypointEliminator -> BRIEF, equal per image to pgm_detect_describe_dev(nms_radius).  One
+//     read-back (the per-image FAST totals, which size the flat keypoint list); the NMS rounds of all images run in one
+//     cooperative kernel that decides by itself when they are over.  11 kernel launches.
+// Either way the counts are copied to `out_counts` at the end if the caller wants them (one more synchronisation).
+static int detect_batch(pgm_handle *h, const float *d_gray, const int64_t *pixel_offsets, const int32_t *widths,
+                        const int32_t *heights, int32_t n_images, float threshold, int32_t nms_radius,
+                        const int32_t *pairs, int32_t n_pairs, int32_t stride_bytes, uint32_t flags, int32_t *d_out_xy,
+                        int32_t *d_out_score, uint8_t *d_out_desc, int32_t capacity, int32_t *d_out_counts,
+                        int32_t *out_counts) {
+    using namespace pgm_det;
+    CU_CHECK(h, cudaSetDevice(h->device));
+    cudaStream_t s = h->stream;
+    const bool py = (flags & PGM_FLAG_PYTHON_GENERATION) != 0, nms = nms_radius >= 0;
+    const int cs = std::max(nms_radius, 1);
+
+    // the geometry table and the pair table, staged together
+    const size_t geo_bytes = align_up((size_t)(n_images + 1) * sizeof(ImageGeom), 256), pair_bytes = (size_t)n_pairs * 16;
+    int rc = ensure_host(h, h->pin_in, geo_bytes + pair_bytes);
+    if (rc) return rc;
+    CU_CHECK(h, cudaStreamSynchronize(s));                 // the staging buffer may still feed an earlier call's copy
+    ImageGeom *hg = (ImageGeom *)h->pin_in.p, acc{};
+    for (int z = 0; z < n_images; z++) {
+        const int w = widths[z], hh = heights[z];
+        acc.px = pixel_offsets[z]; acc.w = w; acc.h = hh;
+        acc.ncx = nms ? (w - 1) / cs + 1 : 0; acc.ncy = nms ? (hh - 1) / cs + 1 : 0;
+        hg[z] = acc;
+        acc.sc += (long long)w * hh; acc.row += hh + 1;
+        acc.tile += (long long)((w + FAST_TILE_W - 1) / FAST_TILE_W) * ((hh + FAST_TILE_H - 1) / FAST_TILE_H);
+        acc.cell += (long long)acc.ncx * acc.ncy;
+    }
+    acc.px = 0; acc.w = acc.h = acc.ncx = acc.ncy = 0;
+    hg[n_images] = acc;                                    // totals
+    memcpy((char *)h->pin_in.p + geo_bytes, pairs, pair_bytes);
+
+    size_t off = 0;
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
+    const size_t o_geo = take(geo_bytes + pair_bytes), o_sc = take((size_t)acc.sc), o_cnt = take((size_t)acc.row * 4);
+    const size_t o_off = take((size_t)acc.row * 4), o_tot = take((size_t)n_images * 4), o_base = take((size_t)(n_images + 1) * 4);
+    if ((rc = ensure_dev(h, h->misc, off))) return rc;
+    if ((rc = ensure_host(h, h->pin_out, (size_t)n_images * 4))) return rc;
+    char *mb = (char *)h->misc.p;
+    const ImageGeom *d_geo = (const ImageGeom *)(mb + o_geo);
+    const int32_t *d_pairs = (const int32_t *)(mb + o_geo + geo_bytes);
+    uint8_t *d_sc = (uint8_t *)(mb + o_sc);
+    int32_t *d_cnt = (int32_t *)(mb + o_cnt), *d_off = (int32_t *)(mb + o_off), *d_tot = (int32_t *)(mb + o_tot);
+    int32_t *d_base = (int32_t *)(mb + o_base);
+    CU_CHECK(h, cudaMemcpyAsync(mb + o_geo, h->pin_in.p, geo_bytes + pair_bytes, cudaMemcpyHostToDevice, s));
+    h->stats.h2d_bytes += (int64_t)(geo_bytes + pair_bytes);
+
+    // 1. FAST-12 of every image: score maps, row counts, row offsets (slot h = the image's total)
+    const dim3 tile(FAST_TILE_W, FAST_TILE_H);
+    // one size packed back to back: the kernels' table-free grids (pgm_detect.cuh); else flat work over all images
+    bool one_size = true;
+    for (int z = 1; z < n_images && one_size; z++)
+        one_size = widths[z] == widths[0] && heights[z] == heights[0] &&
+                   pixel_offsets[z] == pixel_offsets[0] + (int64_t)z * widths[0] * heights[0];
+    const int uw = one_size ? widths[0] : 0, uh = one_size ? heights[0] : 0;
+    const float *d_img = one_size ? d_gray + pixel_offsets[0] : d_gray;
+    const dim3 fast_grid = one_size ? dim3((uw + FAST_TILE_W - 1) / FAST_TILE_W, (uh + FAST_TILE_H - 1) / FAST_TILE_H, n_images)
+                                    : dim3(flat_grid(h, acc.tile, FLAT_CTAS_PER_SM_256, 1));
+    const dim3 row_grid = one_size ? dim3(uh, n_images) : dim3(flat_grid(h, acc.row, FLAT_CTAS_PER_SM_128, 1));
+    const dim3 warp_grid = one_size ? dim3((uh + 3) / 4, n_images) : dim3(flat_grid(h, acc.row, FLAT_CTAS_PER_SM_128, 4));
+    if (py) fast_score_kernel<1><<<fast_grid, tile, 0, s>>>(d_img, d_geo, n_images, uw, uh, threshold, d_sc);
+    else fast_score_kernel<0><<<fast_grid, tile, 0, s>>>(d_img, d_geo, n_images, uw, uh, threshold, d_sc);
+    row_count_kernel<<<row_grid, 128, 0, s>>>(d_sc, d_geo, n_images, uw, uh, d_cnt);
+    scan_kernel<<<n_images, 1024, 0, s>>>(d_cnt, 0, d_off, d_geo);
+    const int warps = 4, sw = stride_bytes / 4;
+    if (!nms) {
+        batch_counts_kernel<<<(n_images + 255) / 256, 256, 0, s>>>(d_off, d_geo, n_images, d_out_counts);
+        emit_kernel<<<warp_grid, 128, 0, s>>>(d_sc, d_geo, n_images, uw, uh, d_off, capacity, d_out_xy, d_out_score);
+        brief_kernel<<<dim3((capacity + warps - 1) / warps, n_images), warps * 32, warps * sw * 4, s>>>(
+            d_gray, 0, 0, d_out_xy, capacity, d_pairs, n_pairs, sw, py ? 1 : 0, (uint32_t *)d_out_desc, d_geo, d_out_counts);
+        h->stats.kernel_launches += 6;
+    } else {
+        batch_counts_kernel<<<(n_images + 255) / 256, 256, 0, s>>>(d_off, d_geo, n_images, d_tot);
+        CU_CHECK(h, cudaMemcpyAsync(h->pin_out.p, d_tot, (size_t)n_images * 4, cudaMemcpyDeviceToHost, s));
+        CU_CHECK(h, cudaStreamSynchronize(s));
+        h->stats.kernel_launches += 4; h->stats.host_syncs++; h->stats.d2h_bytes += (int64_t)n_images * 4;
+
+        // image bases of the flat keypoint list (the sync above freed pin_in); every index below is an int32
+        const int32_t *h_tot = (const int32_t *)h->pin_out.p;
+        int64_t total = 0;
+        for (int z = 0; z < n_images; z++) total += h_tot[z];
+        if (total > INT32_MAX) return fail(h, PGM_E_CAPACITY, "the batch has more than 2^31 - 1 FAST keypoints: split it");
+        const int32_t n = (int32_t)total;
+        const size_t base_bytes = (size_t)(n_images + 1) * 4;
+        if ((rc = ensure_host(h, h->pin_in, base_bytes))) return rc;
+        int32_t *h_base = (int32_t *)h->pin_in.p;
+        h_base[0] = 0;
+        for (int z = 0; z < n_images; z++) h_base[z + 1] = h_base[z] + h_tot[z];
+        CU_CHECK(h, cudaMemcpyAsync(d_base, h->pin_in.p, base_bytes, cudaMemcpyHostToDevice, s));
+        h->stats.h2d_bytes += (int64_t)base_bytes;
+        if (n == 0) {
+            CU_CHECK(h, cudaMemsetAsync(d_out_counts, 0, (size_t)n_images * 4, s));
+        } else {
+            // scratch of the flat list: h->out; radix-sort temporaries: h->out2
+            const long long r2 = (long long)nms_radius * nms_radius;
+            size_t o2 = 0;
+            auto take2 = [&](size_t bytes) { size_t o = o2; o2 = align_up(o2 + bytes, 256); return o; };
+            const size_t o_xy = take2((size_t)n * 8), o_s = take2((size_t)n * 4), o_rk = take2((size_t)n * 4), o_or = take2((size_t)n * 4);
+            const size_t o_k0 = take2((size_t)n * 8), o_k1 = take2((size_t)n * 8), o_c0 = take2((size_t)n * 8), o_c1 = take2((size_t)n * 8);
+            const size_t o_v0 = take2((size_t)n * 4), o_v1 = take2((size_t)n * 4), o_st0 = take2(n), o_st1 = take2(n);
+            const size_t o_ctl = take2(sizeof(NmsBatchCtl));
+            if ((rc = ensure_dev(h, h->out, o2))) return rc;
+            char *ob = (char *)h->out.p;
+            int32_t *d_xy = (int32_t *)(ob + o_xy), *d_s = (int32_t *)(ob + o_s), *d_rk = (int32_t *)(ob + o_rk);
+            int32_t *d_or = (int32_t *)(ob + o_or), *d_v0 = (int32_t *)(ob + o_v0), *d_v1 = (int32_t *)(ob + o_v1);
+            unsigned long long *d_k0 = (unsigned long long *)(ob + o_k0), *d_k1 = (unsigned long long *)(ob + o_k1);
+            unsigned long long *d_c0 = (unsigned long long *)(ob + o_c0), *d_c1 = (unsigned long long *)(ob + o_c1);
+            uint8_t *d_st0 = (uint8_t *)(ob + o_st0), *d_st1 = (uint8_t *)(ob + o_st1);
+            NmsBatchCtl *d_ctl = (NmsBatchCtl *)(ob + o_ctl);
+            int img_bits = 0, cell_bits = 1;
+            while ((n_images - 1) >> img_bits) img_bits++;
+            const unsigned long long n_cells = (unsigned long long)acc.cell;      // sum over the images of ncx * ncy
+            while (cell_bits < 64 && (n_cells - 1) >> cell_bits) cell_bits++;
+            const int rank_bits = NMS_RANK_IMAGE_SHIFT + img_bits;
+            size_t tmp_bytes = 0, tmp2 = 0;
+            CU_CHECK(h, cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, d_k0, d_k1, n, 0, rank_bits, s));
+            CU_CHECK(h, cub::DeviceRadixSort::SortPairs(nullptr, tmp2, d_c0, d_c1, d_v0, d_v1, n, 0, cell_bits, s));
+            tmp_bytes = std::max(tmp_bytes, tmp2);
+            if ((rc = ensure_dev(h, h->out2, tmp_bytes))) return rc;
+            int nb = 0;
+            CU_CHECK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, nms_rounds_batch_kernel, NMS_BATCH_THREADS, 0));
+            const int rounds_grid = (int)std::min<int64_t>((int64_t)std::max(nb, 1) * h->num_sms,
+                                                           ((int64_t)n + NMS_BATCH_THREADS - 1) / NMS_BATCH_THREADS);
+
+            // 2. flat list with rank keys and cell ids; 3. rank order; 4. cell order
+            nms_batch_emit_kernel<<<warp_grid, 128, 0, s>>>(d_sc, d_geo, n_images, uw, uh, d_off, d_base, cs, d_xy,
+                                                                         d_s, d_k0, d_c0, d_v0);
+            CU_CHECK(h, cub::DeviceRadixSort::SortKeys(h->out2.p, tmp_bytes, d_k0, d_k1, n, 0, rank_bits, s));
+            nms_batch_order_kernel<<<(n + 255) / 256, 256, 0, s>>>(d_k1, n, d_base, n_images, d_or, d_rk);
+            CU_CHECK(h, cub::DeviceRadixSort::SortPairs(h->out2.p, tmp_bytes, d_c0, d_c1, d_v0, d_v1, n, 0, cell_bits, s));
+            // 5. every round of every image; 6. survivors in output order into the caller's slots
+            CU_CHECK(h, cudaMemsetAsync(d_st0, 0, n, s));
+            CU_CHECK(h, cudaMemsetAsync(d_ctl, 0, sizeof(NmsBatchCtl), s));
+            int n_arg = n, cs_arg = cs, ni_arg = n_images;
+            long long r2_arg = r2;
+            const int32_t *a_xy = d_xy, *a_rk = d_rk, *a_v1 = d_v1;
+            const unsigned long long *a_k0 = d_k0, *a_c0 = d_c0, *a_c1 = d_c1;
+            void *args[] = {&a_xy, &a_rk, &n_arg, &r2_arg, &cs_arg, &d_geo, &ni_arg, &a_k0, &a_c0, &a_c1, &a_v1,
+                            &d_st0, &d_st1, &d_ctl};
+            CU_CHECK(h, cudaLaunchCooperativeKernel((void *)nms_rounds_batch_kernel, dim3(rounds_grid),
+                                                    dim3(NMS_BATCH_THREADS), args, 0, s));
+            nms_batch_gather_kernel<<<n_images, NMS_EMIT_THREADS, 0, s>>>(d_or, d_base, d_st0, d_st1, d_ctl, d_xy, d_s,
+                                                                          capacity, d_out_xy, d_out_score, d_out_counts);
+            // 7. BRIEF of the survivors
+            brief_kernel<<<dim3((capacity + warps - 1) / warps, n_images), warps * 32, warps * sw * 4, s>>>(
+                d_gray, 0, 0, d_out_xy, capacity, d_pairs, n_pairs, sw, py ? 1 : 0, (uint32_t *)d_out_desc, d_geo,
+                d_out_counts);
+            // emit, rank sort, order, cell sort, rounds, gather, BRIEF (a radix sort counts once)
+            h->stats.kernel_launches += 7;
+        }
+    }
+    CU_CHECK(h, cudaGetLastError());
+    if (out_counts) {
+        CU_CHECK(h, cudaMemcpyAsync(h->pin_out.p, d_out_counts, (size_t)n_images * 4, cudaMemcpyDeviceToHost, s));
+        CU_CHECK(h, cudaStreamSynchronize(s));
+        memcpy(out_counts, h->pin_out.p, (size_t)n_images * 4);
+        h->stats.host_syncs++; h->stats.d2h_bytes += (int64_t)n_images * 4;
+    }
+    return PGM_OK;
+}
+
+// the uniform forms: image k at d_gray + k * width * height
+static int detect_batch_uniform(pgm_handle *h, const float *d_gray, int32_t n_images, int32_t width, int32_t height,
+                                float threshold, int32_t nms_radius, const int32_t *pairs, int32_t n_pairs,
+                                int32_t stride_bytes, uint32_t flags, int32_t *d_out_xy, int32_t *d_out_score,
+                                uint8_t *d_out_desc, int32_t capacity, int32_t *d_out_counts, int32_t *out_counts) {
+    std::vector<int64_t> offsets(n_images);
+    for (int z = 0; z < n_images; z++) offsets[z] = (int64_t)z * width * height;
+    const std::vector<int32_t> widths(n_images, width), heights(n_images, height);
+    return detect_batch(h, d_gray, offsets.data(), widths.data(), heights.data(), n_images, threshold, nms_radius, pairs,
+                        n_pairs, stride_bytes, flags, d_out_xy, d_out_score, d_out_desc, capacity, d_out_counts,
+                        out_counts);
+}
+
+// Many equally sized images in one call, nothing read back in between.  A count above `capacity` means the image's
+// list was truncated.  No NMS in this form (pgm_detect_nms_describe_batch_dev has it).
 extern "C" int pgm_detect_describe_batch_dev(pgm_handle *h, const float *d_gray, int32_t n_images, int32_t width,
                                              int32_t height, float threshold, const int32_t *pairs, int32_t n_pairs,
                                              int32_t stride_bytes, uint32_t flags, int32_t *d_out_xy,
                                              int32_t *d_out_score, uint8_t *d_out_desc, int32_t capacity,
                                              int32_t *d_out_counts, int32_t *out_counts) {
-    using namespace pgm_det;
     if (!h) return PGM_E_INVALID_ARG;
     std::lock_guard<std::mutex> lk(h->mu);
     int rc = check_format(h, n_pairs, stride_bytes);       // desc_bits == NumGaussianPairs
@@ -2342,53 +2527,16 @@ extern "C" int pgm_detect_describe_batch_dev(pgm_handle *h, const float *d_gray,
     h->stats = pgm_stats{};
     h->stats_pending = false;
     if (n_images == 0) return PGM_OK;
-    CU_CHECK(h, cudaSetDevice(h->device));
-    cudaStream_t s = h->stream;
-    const size_t npx = (size_t)width * height;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-    const size_t o_sc = take(npx * n_images), o_cnt = take((size_t)height * n_images * 4);
-    const size_t o_off = take((size_t)(height + 1) * n_images * 4), o_pairs = take((size_t)n_pairs * 16);
-    if ((rc = ensure_dev(h, h->misc, off))) return rc;
-    if ((rc = ensure_host(h, h->pin_in, (size_t)n_pairs * 16))) return rc;
-    char *base = (char *)h->misc.p;
-    uint8_t *d_sc = (uint8_t *)(base + o_sc);
-    int32_t *d_cnt = (int32_t *)(base + o_cnt), *d_off = (int32_t *)(base + o_off), *d_pairs = (int32_t *)(base + o_pairs);
-    CU_CHECK(h, cudaStreamSynchronize(s));                 // the staging buffer may still feed an earlier call's copy
-    memcpy(h->pin_in.p, pairs, (size_t)n_pairs * 16);
-    CU_CHECK(h, cudaMemcpyAsync(d_pairs, h->pin_in.p, (size_t)n_pairs * 16, cudaMemcpyHostToDevice, s));
-    dim3 blk(32, 8), grd((width + 31) / 32, (height + 7) / 8, n_images);
-    if (flags & PGM_FLAG_PYTHON_GENERATION) fast_score_kernel<1><<<grd, blk, 0, s>>>(d_gray, width, height, threshold, d_sc);
-    else fast_score_kernel<0><<<grd, blk, 0, s>>>(d_gray, width, height, threshold, d_sc);
-    row_count_kernel<<<dim3(height, n_images), 128, 0, s>>>(d_sc, width, d_cnt);
-    scan_kernel<<<n_images, 1024, 0, s>>>(d_cnt, height, d_off);
-    emit_kernel<<<dim3((height + 3) / 4, n_images), 128, 0, s>>>(d_sc, width, height, d_off, capacity, d_out_xy, d_out_score);
-    const int warps = 4, sw = stride_bytes / 4;
-    brief_kernel<<<dim3((capacity + warps - 1) / warps, n_images), warps * 32, warps * sw * 4, s>>>(
-        d_gray, width, height, d_out_xy, capacity, d_pairs, n_pairs, sw, (flags & PGM_FLAG_PYTHON_GENERATION) ? 1 : 0,
-        (uint32_t *)d_out_desc, d_off);
-    batch_counts_kernel<<<(n_images + 255) / 256, 256, 0, s>>>(d_off, height, n_images, d_out_counts);
-    h->stats.kernel_launches += 6;
-    CU_CHECK(h, cudaGetLastError());
-    if (out_counts) {
-        if ((rc = ensure_host(h, h->pin_out, (size_t)n_images * 4))) return rc;
-        CU_CHECK(h, cudaMemcpyAsync(h->pin_out.p, d_out_counts, (size_t)n_images * 4, cudaMemcpyDeviceToHost, s));
-        CU_CHECK(h, cudaStreamSynchronize(s));
-        memcpy(out_counts, h->pin_out.p, (size_t)n_images * 4);
-        h->stats.host_syncs++; h->stats.d2h_bytes += (int64_t)n_images * 4;
-    }
-    return PGM_OK;
+    return detect_batch_uniform(h, d_gray, n_images, width, height, threshold, -1, pairs, n_pairs, stride_bytes, flags,
+                                d_out_xy, d_out_score, d_out_desc, capacity, d_out_counts, out_counts);
 }
 
-// The batched chain with NMS: FAST-12 -> RedundantKeypointEliminator -> BRIEF for every image, equal per image to
-// pgm_detect_describe_dev(nms_radius).  One read-back (the per-image FAST totals, which size the flat keypoint list);
-// the NMS rounds of all images run in one cooperative kernel that decides by itself when they are over.
+// The batched chain with NMS, equal per image to pgm_detect_describe_dev(nms_radius).
 extern "C" int pgm_detect_nms_describe_batch_dev(pgm_handle *h, const float *d_gray, int32_t n_images, int32_t width,
                                                  int32_t height, float threshold, int32_t nms_radius, const int32_t *pairs,
                                                  int32_t n_pairs, int32_t stride_bytes, uint32_t flags, int32_t *d_out_xy,
                                                  int32_t *d_out_score, uint8_t *d_out_desc, int32_t capacity,
                                                  int32_t *d_out_counts, int32_t *out_counts) {
-    using namespace pgm_det;
     if (!h) return PGM_E_INVALID_ARG;
     std::lock_guard<std::mutex> lk(h->mu);
     int rc = check_format(h, n_pairs, stride_bytes);       // desc_bits == NumGaussianPairs
@@ -2399,121 +2547,36 @@ extern "C" int pgm_detect_nms_describe_batch_dev(pgm_handle *h, const float *d_g
     h->stats = pgm_stats{};
     h->stats_pending = false;
     if (n_images == 0) return PGM_OK;
-    CU_CHECK(h, cudaSetDevice(h->device));
-    cudaStream_t s = h->stream;
-    const bool py = (flags & PGM_FLAG_PYTHON_GENERATION) != 0;
+    return detect_batch_uniform(h, d_gray, n_images, width, height, threshold, nms_radius, pairs, n_pairs, stride_bytes,
+                                flags, d_out_xy, d_out_score, d_out_desc, capacity, d_out_counts, out_counts);
+}
 
-    // 1. FAST-12 of every image, per-image totals read back once
-    const size_t npx = (size_t)width * height;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-    const size_t o_sc = take(npx * n_images), o_cnt = take((size_t)height * n_images * 4);
-    const size_t o_off = take((size_t)(height + 1) * n_images * 4), o_tot = take((size_t)n_images * 4);
-    const size_t o_base = take((size_t)(n_images + 1) * 4), o_pairs = take((size_t)n_pairs * 16);
-    if ((rc = ensure_dev(h, h->misc, off))) return rc;
-    if ((rc = ensure_host(h, h->pin_out, (size_t)n_images * 4))) return rc;
-    char *mb = (char *)h->misc.p;
-    uint8_t *d_sc = (uint8_t *)(mb + o_sc);
-    int32_t *d_cnt = (int32_t *)(mb + o_cnt), *d_off = (int32_t *)(mb + o_off), *d_tot = (int32_t *)(mb + o_tot);
-    int32_t *d_base = (int32_t *)(mb + o_base), *d_pairs = (int32_t *)(mb + o_pairs);
-    dim3 blk(32, 8), grd((width + 31) / 32, (height + 7) / 8, n_images);
-    if (py) fast_score_kernel<1><<<grd, blk, 0, s>>>(d_gray, width, height, threshold, d_sc);
-    else fast_score_kernel<0><<<grd, blk, 0, s>>>(d_gray, width, height, threshold, d_sc);
-    row_count_kernel<<<dim3(height, n_images), 128, 0, s>>>(d_sc, width, d_cnt);
-    scan_kernel<<<n_images, 1024, 0, s>>>(d_cnt, height, d_off);
-    batch_counts_kernel<<<(n_images + 255) / 256, 256, 0, s>>>(d_off, height, n_images, d_tot);
-    CU_CHECK(h, cudaMemcpyAsync(h->pin_out.p, d_tot, (size_t)n_images * 4, cudaMemcpyDeviceToHost, s));
-    CU_CHECK(h, cudaStreamSynchronize(s));
-    h->stats.kernel_launches += 4; h->stats.host_syncs++; h->stats.d2h_bytes += (int64_t)n_images * 4;
-
-    // image bases of the flat keypoint list and the pair table, staged together (the sync above freed pin_in);
-    // every index below is an int32
-    const int32_t *h_tot = (const int32_t *)h->pin_out.p;
-    int64_t total = 0;
-    for (int z = 0; z < n_images; z++) total += h_tot[z];
-    if (total > INT32_MAX) return fail(h, PGM_E_CAPACITY, "the batch has more than 2^31 - 1 FAST keypoints: split it");
-    const int32_t n = (int32_t)total;
-    const size_t base_bytes = (size_t)(n_images + 1) * 4;
-    if ((rc = ensure_host(h, h->pin_in, base_bytes + (size_t)n_pairs * 16))) return rc;
-    int32_t *h_base = (int32_t *)h->pin_in.p;
-    h_base[0] = 0;
-    for (int z = 0; z < n_images; z++) h_base[z + 1] = h_base[z] + h_tot[z];
-    memcpy((char *)h->pin_in.p + base_bytes, pairs, (size_t)n_pairs * 16);
-    CU_CHECK(h, cudaMemcpyAsync(d_base, h->pin_in.p, base_bytes, cudaMemcpyHostToDevice, s));
-    CU_CHECK(h, cudaMemcpyAsync(d_pairs, (char *)h->pin_in.p + base_bytes, (size_t)n_pairs * 16, cudaMemcpyHostToDevice, s));
-    h->stats.h2d_bytes += (int64_t)base_bytes + (int64_t)n_pairs * 16;
-    if (n == 0) {
-        CU_CHECK(h, cudaMemsetAsync(d_out_counts, 0, (size_t)n_images * 4, s));
-    } else {
-        // scratch of the flat list: h->out; radix-sort temporaries: h->out2
-        const int cs = std::max(nms_radius, 1);
-        const int ncx = (width - 1) / cs + 1, ncy = (height - 1) / cs + 1;
-        const long long r2 = (long long)nms_radius * nms_radius;
-        size_t o2 = 0;
-        auto take2 = [&](size_t bytes) { size_t o = o2; o2 = align_up(o2 + bytes, 256); return o; };
-        const size_t o_xy = take2((size_t)n * 8), o_s = take2((size_t)n * 4), o_rk = take2((size_t)n * 4), o_or = take2((size_t)n * 4);
-        const size_t o_k0 = take2((size_t)n * 8), o_k1 = take2((size_t)n * 8), o_c0 = take2((size_t)n * 8), o_c1 = take2((size_t)n * 8);
-        const size_t o_v0 = take2((size_t)n * 4), o_v1 = take2((size_t)n * 4), o_st0 = take2(n), o_st1 = take2(n);
-        const size_t o_ctl = take2(sizeof(NmsBatchCtl));
-        if ((rc = ensure_dev(h, h->out, o2))) return rc;
-        char *ob = (char *)h->out.p;
-        int32_t *d_xy = (int32_t *)(ob + o_xy), *d_s = (int32_t *)(ob + o_s), *d_rk = (int32_t *)(ob + o_rk);
-        int32_t *d_or = (int32_t *)(ob + o_or), *d_v0 = (int32_t *)(ob + o_v0), *d_v1 = (int32_t *)(ob + o_v1);
-        unsigned long long *d_k0 = (unsigned long long *)(ob + o_k0), *d_k1 = (unsigned long long *)(ob + o_k1);
-        unsigned long long *d_c0 = (unsigned long long *)(ob + o_c0), *d_c1 = (unsigned long long *)(ob + o_c1);
-        uint8_t *d_st0 = (uint8_t *)(ob + o_st0), *d_st1 = (uint8_t *)(ob + o_st1);
-        NmsBatchCtl *d_ctl = (NmsBatchCtl *)(ob + o_ctl);
-        int img_bits = 0, cell_bits = 1;
-        while ((n_images - 1) >> img_bits) img_bits++;
-        const unsigned long long n_cells = (unsigned long long)n_images * ncy * ncx;
-        while (cell_bits < 64 && (n_cells - 1) >> cell_bits) cell_bits++;
-        const int rank_bits = NMS_RANK_IMAGE_SHIFT + img_bits;
-        size_t tmp_bytes = 0, tmp2 = 0;
-        CU_CHECK(h, cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, d_k0, d_k1, n, 0, rank_bits, s));
-        CU_CHECK(h, cub::DeviceRadixSort::SortPairs(nullptr, tmp2, d_c0, d_c1, d_v0, d_v1, n, 0, cell_bits, s));
-        tmp_bytes = std::max(tmp_bytes, tmp2);
-        if ((rc = ensure_dev(h, h->out2, tmp_bytes))) return rc;
-        int nb = 0;
-        CU_CHECK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, nms_rounds_batch_kernel, NMS_BATCH_THREADS, 0));
-        const int rounds_grid = (int)std::min<int64_t>((int64_t)std::max(nb, 1) * h->num_sms,
-                                                       ((int64_t)n + NMS_BATCH_THREADS - 1) / NMS_BATCH_THREADS);
-
-        // 2. flat list with rank keys and cell ids; 3. rank order; 4. cell order
-        nms_batch_emit_kernel<<<dim3((height + 3) / 4, n_images), 128, 0, s>>>(d_sc, width, height, d_off, d_base, cs, ncx,
-                                                                              ncy, d_xy, d_s, d_k0, d_c0, d_v0);
-        CU_CHECK(h, cub::DeviceRadixSort::SortKeys(h->out2.p, tmp_bytes, d_k0, d_k1, n, 0, rank_bits, s));
-        nms_batch_order_kernel<<<(n + 255) / 256, 256, 0, s>>>(d_k1, n, d_base, n_images, d_or, d_rk);
-        CU_CHECK(h, cub::DeviceRadixSort::SortPairs(h->out2.p, tmp_bytes, d_c0, d_c1, d_v0, d_v1, n, 0, cell_bits, s));
-        // 5. every round of every image; 6. survivors in output order into the caller's slots
-        CU_CHECK(h, cudaMemsetAsync(d_st0, 0, n, s));
-        CU_CHECK(h, cudaMemsetAsync(d_ctl, 0, sizeof(NmsBatchCtl), s));
-        int n_arg = n, cs_arg = cs, ncx_arg = ncx, ncy_arg = ncy;
-        long long r2_arg = r2;
-        const int32_t *a_xy = d_xy, *a_rk = d_rk, *a_v1 = d_v1;
-        const unsigned long long *a_c0 = d_c0, *a_c1 = d_c1;
-        void *args[] = {&a_xy, &a_rk, &n_arg, &r2_arg, &cs_arg, &ncx_arg, &ncy_arg, &a_c0, &a_c1, &a_v1, &d_st0, &d_st1, &d_ctl};
-        CU_CHECK(h, cudaLaunchCooperativeKernel((void *)nms_rounds_batch_kernel, dim3(rounds_grid), dim3(NMS_BATCH_THREADS),
-                                                args, 0, s));
-        nms_batch_gather_kernel<<<n_images, NMS_EMIT_THREADS, 0, s>>>(d_or, d_base, d_st0, d_st1, d_ctl, d_xy, d_s,
-                                                                      capacity, d_out_xy, d_out_score, d_out_counts);
-        h->stats.kernel_launches += 6;     // emit, rank sort, order, cell sort, rounds, gather (a radix sort counts once)
+// Images of any sizes in one call: image k is widths[k] x heights[k] at d_gray + pixel_offsets[k].
+extern "C" int pgm_detect_describe_images_batch_dev(pgm_handle *h, const float *d_gray, const int64_t *pixel_offsets,
+                                                    const int32_t *widths, const int32_t *heights, int32_t n_images,
+                                                    float threshold, int32_t nms_radius, const int32_t *pairs,
+                                                    int32_t n_pairs, int32_t stride_bytes, uint32_t flags,
+                                                    int32_t *d_out_xy, int32_t *d_out_score, uint8_t *d_out_desc,
+                                                    int32_t capacity, int32_t *d_out_counts, int32_t *out_counts) {
+    if (!h) return PGM_E_INVALID_ARG;
+    std::lock_guard<std::mutex> lk(h->mu);
+    int rc = check_format(h, n_pairs, stride_bytes);       // desc_bits == NumGaussianPairs
+    if (rc) return rc;
+    if (!d_gray || !pixel_offsets || !widths || !heights || n_images < 0 || n_images > 65535 || !pairs ||
+        capacity < 1 || !d_out_xy || !d_out_score || !d_out_desc || !d_out_counts)
+        return fail(h, PGM_E_INVALID_ARG, "bad arguments");
+    if (pixel_offsets[0] < 0) return fail(h, PGM_E_INVALID_ARG, "pixel_offsets[0] < 0");
+    for (int z = 0; z < n_images; z++) {
+        if (widths[z] < 1 || heights[z] < 1 || widths[z] > 65535 || heights[z] > 65535)
+            return fail(h, PGM_E_INVALID_ARG, "an image size is outside 1..65535");   // MatrixDimensions are ushort upstream
+        if (pixel_offsets[z + 1] < pixel_offsets[z] + (int64_t)widths[z] * heights[z])
+            return fail(h, PGM_E_INVALID_ARG, "pixel_offsets[k + 1] < pixel_offsets[k] + widths[k] * heights[k]");
     }
-    // 7. BRIEF of the survivors
-    if (n > 0) {
-        const int warps = 4, sw = stride_bytes / 4;
-        brief_kernel<<<dim3((capacity + warps - 1) / warps, n_images), warps * 32, warps * sw * 4, s>>>(
-            d_gray, width, height, d_out_xy, capacity, d_pairs, n_pairs, sw, py ? 1 : 0, (uint32_t *)d_out_desc, nullptr,
-            d_out_counts);
-        h->stats.kernel_launches += 1;
-    }
-    CU_CHECK(h, cudaGetLastError());
-    if (out_counts) {
-        CU_CHECK(h, cudaMemcpyAsync(h->pin_out.p, d_out_counts, (size_t)n_images * 4, cudaMemcpyDeviceToHost, s));
-        CU_CHECK(h, cudaStreamSynchronize(s));
-        memcpy(out_counts, h->pin_out.p, (size_t)n_images * 4);
-        h->stats.host_syncs++; h->stats.d2h_bytes += (int64_t)n_images * 4;
-    }
-    return PGM_OK;
+    h->stats = pgm_stats{};
+    h->stats_pending = false;
+    if (n_images == 0) return PGM_OK;
+    return detect_batch(h, d_gray, pixel_offsets, widths, heights, n_images, threshold, nms_radius, pairs, n_pairs,
+                        stride_bytes, flags, d_out_xy, d_out_score, d_out_desc, capacity, d_out_counts, out_counts);
 }
 
 // ---------------------------------------------------------------------------

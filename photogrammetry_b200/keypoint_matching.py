@@ -497,6 +497,40 @@ class Matcher:
             self._check(rc)
         return xy, sc, desc, (h_cnt[:k] if read_counts else d_cnt[:k])
 
+    def detect_describe_images_batch_dev(self, images, threshold: float, pairs: np.ndarray, capacity: int = 4096,
+                                         stride: Optional[int] = None, python_generation: bool = False,
+                                         read_counts: bool = True, nms_radius: int = -1):
+        """:meth:`detect_describe_batch_dev` for images of any sizes: ``images`` is a list of 2-D torch float32 tensors on
+        this matcher's GPU, each detected at its own size (portrait next to landscape, mixed cameras and crops), in one
+        call.  They are packed into one flat device buffer.  Arguments, return value and synchronisation are those of
+        :meth:`detect_describe_batch_dev`; per image the result equals :meth:`detect_describe_dev` on that image."""
+        import torch
+        pairs = np.ascontiguousarray(pairs, dtype=np.int32).reshape(-1, 4)
+        k = len(images)
+        if any(im.dim() != 2 or im.dtype != torch.float32 for im in images):
+            raise ValueError("images must be 2-D float32 tensors")
+        heights = np.array([int(im.shape[0]) for im in images], dtype=np.int32)
+        widths = np.array([int(im.shape[1]) for im in images], dtype=np.int32)
+        offs = np.zeros(k + 1, dtype=np.int64)
+        offs[1:] = np.cumsum(widths.astype(np.int64) * heights)
+        n_pairs = len(pairs)
+        stride = stride or ((n_pairs + 127) // 128) * 16
+        flags = PGM_FLAG_PYTHON_GENERATION if python_generation else 0
+        dev = images[0].device if k else torch.device("cuda", self.device)
+        cap = max(int(capacity), 1)
+        with self.torch_ordered(dev):
+            d_gray = torch.cat([im.reshape(-1) for im in images]) if k else torch.empty(1, dtype=torch.float32, device=dev)
+            xy = torch.empty((k, cap, 2), dtype=torch.int32, device=dev)
+            sc = torch.empty((k, cap), dtype=torch.int32, device=dev)
+            desc = torch.zeros((k, cap, stride), dtype=torch.uint8, device=dev)
+            d_cnt = torch.zeros(max(k, 1), dtype=torch.int32, device=dev)
+            h_cnt = np.zeros(max(k, 1), dtype=np.int32)
+            self._check(self._lib.pgm_detect_describe_images_batch_dev(
+                self._h, d_gray.data_ptr(), offs.ctypes.data, widths.ctypes.data, heights.ctypes.data, k, float(threshold),
+                int(nms_radius), pairs.ctypes.data, n_pairs, stride, flags, xy.data_ptr(), sc.data_ptr(), desc.data_ptr(),
+                cap, d_cnt.data_ptr(), h_cnt.ctypes.data if read_counts else None))
+        return xy, sc, desc, (h_cnt[:k] if read_counts else d_cnt[:k])
+
     def nms(self, xy: np.ndarray, score: np.ndarray, radius: int) -> np.ndarray:
         """``RedundantKeypointEliminator.EliminateRedundantKeypoints`` (RedundantKeypointEliminator.cs:16-39):
         indices of the surviving keypoints in the reference's output order."""

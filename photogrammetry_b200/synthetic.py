@@ -166,3 +166,19 @@ def dotted_row_image(h: int = 40, w: int = 2000, value: float = 1.0) -> np.ndarr
     img = np.zeros((h, w), dtype=np.float32)
     img[20, 8:w - 8:4] = np.float32(value)
     return img
+
+
+def scene_crops(seed: int, boxes):
+    """Crops of one seeded scene (a :func:`rectangles_image` just large enough to hold every box): ``boxes`` is a list of
+    ``(x0, y0, w, h)`` in scene pixels, so a set can mix sizes and portrait / landscape orientations.  Returns
+    ``(crops, offsets)``: float32[h, w] copies and int64[len(boxes), 2] = (x0, y0).  A scene point at (x, y) in crop a
+    is at (x + x0_a - x0_b, y + y0_a - y0_b) in crop b: overlapping crops are a pure translation apart, which gives
+    their correspondences a known ground truth."""
+    boxes = np.asarray(boxes, dtype=np.int64).reshape(-1, 4)
+    if (boxes[:, :2] < 0).any() or (boxes[:, 2:] < 1).any():
+        raise ValueError("boxes need x0, y0 >= 0 and w, h >= 1")
+    w = max(int((boxes[:, 0] + boxes[:, 2]).max()), 64)
+    h = max(int((boxes[:, 1] + boxes[:, 3]).max()), 64)
+    scene = rectangles_image(h, w, seed)
+    crops = [np.ascontiguousarray(scene[y0:y0 + bh, x0:x0 + bw]) for x0, y0, bw, bh in boxes.tolist()]
+    return crops, np.ascontiguousarray(boxes[:, :2])

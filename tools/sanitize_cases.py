@@ -17,6 +17,9 @@
      20 000 matches (several shared-memory tiles per score CTA), S spread over two score items per pair
   9. batched detect -> NMS -> BRIEF of 4 frames: the dotted-row chain (496 device-side rounds in the cooperative kernel),
      a blank frame (empty run) and two random frames, against the oracle chain
+ 10. detect -> NMS -> BRIEF of a set of images of different sizes in one call (flat FAST tiles and row slots,
+     per-image NMS cells): landscape and portrait frames, odd widths, a 5 x 9 image with no FAST interior and the
+     dotted-row chain, with gaps between the images, against single-image calls
 Every result is checked against the oracle, so a sanitizer run is also a parity run."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -129,5 +132,21 @@ for k in range(4):
     assert (desc[k, :n].cpu().numpy() == pack_descriptors(D.brief_descriptors(frames[k], exy[kept], dpairs), 256)).all()
 assert counts[0] == 248 and counts[1] == 0
 print("case 9 ok", m.stats())
+ims = [rng.random((61, 83), dtype=np.float32), rng.random((83, 61), dtype=np.float32), rng.random((9, 5), dtype=np.float32),
+       synthetic.dotted_row_image(), rng.random((33, 257), dtype=np.float32)]
+buf, offs = [], [0]
+for im in ims:                                               # 13 NaN pixels after every image
+    buf += [im.ravel(), np.full(13, np.nan, np.float32)]
+    offs.append(offs[-1] + im.size + 13)
+d_buf = torch.from_numpy(np.concatenate(buf)).cuda()
+views = [d_buf[offs[k]:offs[k] + im.size].view(im.shape) for k, im in enumerate(ims)]
+xy, sc, desc, counts = m.detect_describe_images_batch_dev(views, 0.1, dpairs.reshape(-1, 4), capacity=4096, nms_radius=4)
+for k, v in enumerate(views):
+    exy, esc, edesc = (x.cpu().numpy() for x in m.detect_describe_dev(v.contiguous(), 0.1, dpairs.reshape(-1, 4), nms_radius=4))
+    n = len(exy)
+    assert counts[k] == n and (xy[k, :n].cpu().numpy() == exy).all() and (sc[k, :n].cpu().numpy() == esc).all(), k
+    assert (desc[k, :n].cpu().numpy() == edesc).all(), k
+assert counts[2] == 0 and counts[3] == 248
+print("case 10 ok", m.stats())
 m.close()
 print("ALL OK")
